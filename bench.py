@@ -49,6 +49,38 @@ def _emit(line):
     out.flush()
 
 
+DUMP_BYTES = 62_000_000   # payload of --dump-outputs: with the .npy headers the files stay under 64 MB
+
+
+def registration_outputs(out, binding):
+    """Host copies of what one dev_register_scene_shot call left in `out`, cut to the valid rows.  Correspondences
+    are (index_query, index_match, distance) rows in float64, which holds both int32 and float32 exactly."""
+    def corr_rows(t, n):
+        c = t[:n].cpu().numpy().view(binding.CORR_DTYPE).reshape(-1)
+        return np.stack([c["index_query"], c["index_match"], c["distance"]], axis=1).astype(np.float64)
+
+    m = min(int(out["n_inst"].item()), PARAMS["max_instances"])
+    off = out["inst_offsets"][:m + 1].cpu().numpy()
+    return {"corrs": corr_rows(out["corrs"], int(out["n_corrs"].item())),
+            "transforms": out["transforms"][:m * 16].cpu().numpy().reshape(m, 4, 4),
+            "inst_offsets": off.astype(np.float64),
+            "inst_counts": out["inst_counts"][:m].cpu().numpy().astype(np.float64),
+            "inst_corrs": corr_rows(out["inst_corrs"], min(int(off[-1]), out["corr_cap"]))}
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes name -> array as out_dir/<name>.npy.  Above DUMP_BYTES in all, every array keeps the same fraction of
+    its rows, picked with a fixed seed, so that two builds with equally long outputs write the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    frac = min(1.0, DUMP_BYTES / total) if total else 1.0
+    for name, a in arrays.items():
+        if frac < 1.0 and len(a) > 1:
+            keep = max(1, int(len(a) * frac))
+            a = a[np.sort(np.random.Generator(np.random.PCG64(0)).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload(scene_id, scene_points, model_points):
     synth = importlib.import_module(PKG).synth
     model = synth.make_model("y", model_points)
@@ -277,7 +309,6 @@ def run_b200(args, rank, world, local_rank):
     B = L * max(1, args.scenes_per_lane)   # scene registrations per step and rank
     if fixed_total:
         B = max(1, fixed_total // world)   # this rank's share of the batch (every rank the same: one gather per scene)
-        args.steps = 1
     streams = [torch.cuda.Stream(device=dev) for _ in range(L)]
     ctxs = [binding.Context(local_rank, stream=st.cuda_stream) for st in streams]
     if blocking:
@@ -387,6 +418,12 @@ def run_b200(args, rank, world, local_rank):
     total_ms = max(ev_start.elapsed_time(e) for e in ev_ends)
     launches = sum(c.launches for c in ctxs) - launches0
     desc_done = float(sum(Kss[s % P] for s in range(n_scene_steps)))
+    if args.dump_outputs and rank == 0:
+        # lane l ran scenes l, l + L, ... of the timed pass and its buffers hold the last of them; the lanes whose last
+        # scene belongs to the last step (all of them when B >= L) hold the last registrations of that step
+        last = [l for l in range(L) if l < n_scene_steps and l + L * ((n_scene_steps - 1 - l) // L) >= n_scene_steps - B]
+        dump_outputs(args.dump_outputs, {"lane%d_%s" % (l, k): v for l in last
+                                         for k, v in registration_outputs(outs[l], binding).items()})
 
     ms = total_ms / args.steps
     t = torch.tensor([ms, desc_done, single_ms], dtype=torch.float64, device=dev)
@@ -826,7 +863,13 @@ def main():
                          "scaling), e.g. --total-scenes 256 --scene-points 500000 --pool 8")
     ap.add_argument("--other-configs", type=int, default=1,
                     help="also measure BASELINE configs 1, 2 and 4 (small) and report them under other_configs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the registrations of the last step returned as "
+                         "DIR/lane<l>_<name>.npy (float32/float64, at most 64 MB), to compare two builds on the same "
+                         "inputs")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "batch"):
+        ap.error("--dump-outputs applies to --impl b200 --mode batch")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     # stdout carries exactly one JSON line: anything a library prints there (NCCL's version banner)
     # goes to stderr instead
