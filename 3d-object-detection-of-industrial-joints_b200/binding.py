@@ -42,6 +42,8 @@ EXPORTS = [
     "b200_board_params_default",
     "b200_ctx_srand",
     "b200_board_lrf",
+    "b200_model_create_shot_hough", "b200_model_download_frames", "b200_register_scene_shot_hough",
+    "b200_dev_register_scene_shot_hough", "b200_register_scene_batch_shot_hough",
     "b200_hv_params_default", "b200_hv_create", "b200_hv_destroy", "b200_hv_set_params", "b200_hv_set_scene",
     "b200_hv_add_models", "b200_hv_verify", "b200_hv_last_size", "b200_hv_last_copy", "b200_hv_optimize",
 ]
@@ -79,6 +81,17 @@ def board_params(find_holes=True, tangent_radius=0.0, margin_thresh=0.85, check_
     """PCL's constructor defaults, with find_holes as the reference sets it (SHOT.cpp:442)."""
     return BoardParams(int(find_holes), float(tangent_radius), float(margin_thresh), int(check_margin_array_size),
                        float(hole_size_prob_thresh), float(steep_thresh))
+
+
+class HoughParams(C.Structure):
+    """b200_hough_params: BOARD frames + Hough3DGrouping of the resident Hough branch."""
+    _fields_ = [("rf_radius", C.c_double), ("board", BoardParams), ("bin_size", C.c_double), ("threshold", C.c_double)]
+
+
+def hough_params(rf_radius=0.02, bin_size=0.02, threshold=2.0, **board):
+    """The reference's Hough branch (SHOT_scenes.cpp:54-55: rf_rad_ / cg_size_ 0.02, cg_thresh_ 2); keyword
+    arguments go to board_params (find_holes on)."""
+    return HoughParams(float(rf_radius), board_params(**board), float(bin_size), float(threshold))
 
 
 class HvParams(C.Structure):
@@ -181,6 +194,17 @@ def lib():
             "b200_board_params_default": [C.POINTER(BoardParams)],
             "b200_ctx_srand": [vp, C.c_uint],
             "b200_board_lrf": [vp, vp, fp, fp, i, i, d, C.POINTER(BoardParams), fp],
+            "b200_model_create_shot_hough": [vp, fp, i, i, fp, i, i, C.POINTER(ShotParams), C.POINTER(HoughParams),
+                                             C.POINTER(vp)],
+            "b200_model_download_frames": [vp, vp, fp],
+            "b200_register_scene_shot_hough": [vp, vp, fp, i, i, fp, i, i, C.POINTER(ShotParams), C.POINTER(HoughParams),
+                                               fp, ip, C.POINTER(Corr), i, ip, C.POINTER(Corr), ip, fp],
+            "b200_dev_register_scene_shot_hough": [vp, vp, vp, i, i, vp, i, i, C.POINTER(ShotParams),
+                                                   C.POINTER(HoughParams), vp, vp, vp, vp, i, vp, vp, vp, vp, vp, vp],
+            "b200_register_scene_batch_shot_hough": [i, vp, i, C.POINTER(fp), ip, i, C.POINTER(fp), ip, i,
+                                                     C.POINTER(ShotParams), C.POINTER(HoughParams), i, C.POINTER(fp),
+                                                     C.POINTER(ip), C.POINTER(C.POINTER(Corr)), ip, ip,
+                                                     C.POINTER(C.POINTER(Corr)), ip, ip],
             "b200_remove_nan": [vp, fp, i, i, fp, ip, ip],
             "b200_transform_points": [vp, fp, i, i, fp, fp],
             "b200_icp_align": [vp, fp, i, i, vp, i, d, d, d, fp, fp, fp, C.POINTER(d), ip, ip],
@@ -314,6 +338,12 @@ class Model:
         kp = np.zeros((K, 3), dtype=np.float32)
         self.ctx._chk(lib().b200_model_download(self.ctx.h, self.h, _f(desc), _f(kp)))
         return desc, kp
+
+    def download_frames(self):
+        """K x 9 BOARD frames of a model from Context.model_create_shot_hough (b200_model_download_frames)."""
+        rf = np.zeros((max(self.size, 1), 9), dtype=np.float32)
+        self.ctx._chk(lib().b200_model_download_frames(self.ctx.h, self.h, _f(rf)))
+        return rf[:self.size]
 
     def close(self):
         if self.h and self.ctx.h:
@@ -841,6 +871,47 @@ class Context:
         return {"transforms": T[:m].reshape(m, 4, 4), "instances": InstanceList(ic, off, m),
                 "n_instances": n_inst.value, "corrs": corrs[:n_corr.value], "truncated": rc == ERR_CAPACITY}
 
+    # ---- resident Hough branch (BOARD frames + Hough3DGrouping) ------------------------------------
+    def model_create_shot_hough(self, xyz, kp, params, hough):
+        """b200_model_create_shot_hough: the SHOT model plus its BOARD frames (drawn from this context's rand()
+        stream) and Hough votes."""
+        xyz, kp = _pts(xyz), _pts(kp)
+        h = C.c_void_p()
+        self._chk(lib().b200_model_create_shot_hough(self.h, _f(xyz), len(xyz), xyz.shape[1], _f(kp), len(kp),
+                                                     kp.shape[1], C.byref(params), C.byref(hough), C.byref(h)))
+        return Model(self, h)
+
+    def register_scene_shot_hough(self, model, scene_xyz, scene_kp, params, hough):
+        """Host buffers in, host results out (b200_register_scene_shot_hough).  As register_scene_shot, plus the scene
+        frames ("rf", Ks x 9) and the return code ("status": 0, or ERR_CAPACITY when the instances were truncated or
+        the Hough space would exceed 2^27 bins)."""
+        scene_xyz, scene_kp = _pts(scene_xyz), _pts(scene_kp)
+        mi, Ks = params.max_instances, len(scene_kp)
+        T = np.empty((mi, 16), dtype=np.float32)
+        off = np.zeros(mi + 1, dtype=np.int32)
+        ic = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
+        corrs = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
+        rf = np.empty((max(Ks, 1), 9), dtype=np.float32)
+        n_inst, n_corr = C.c_int(), C.c_int()
+        rc = lib().b200_register_scene_shot_hough(self.h, model.h, _f(scene_xyz), len(scene_xyz), scene_xyz.shape[1],
+                                                  _f(scene_kp), Ks, scene_kp.shape[1], C.byref(params), C.byref(hough),
+                                                  _f(T), _i(off), _c(ic), max(Ks, 1), C.byref(n_inst), _c(corrs),
+                                                  C.byref(n_corr), _f(rf))
+        if rc not in (OK, ERR_CAPACITY):
+            self._chk(rc)
+        m = min(n_inst.value, mi)
+        return {"transforms": T[:m].reshape(m, 4, 4), "instances": InstanceList(ic, off, m),
+                "n_instances": n_inst.value, "corrs": corrs[:n_corr.value], "rf": rf[:Ks], "status": rc}
+
+    def dev_register_scene_shot_hough(self, model, d_xyz, n, stride, d_kp, Ks, kstride, params, hough, out):
+        """All buffers resident (torch CUDA tensors in `out`, as dev_register_scene_shot, plus the device int
+        out["status"] and optionally out["rf"]), asynchronous (b200_dev_register_scene_shot_hough)."""
+        self._chk(lib().b200_dev_register_scene_shot_hough(
+            self.h, model.h, _dptr(d_xyz), int(n), int(stride), _dptr(d_kp), int(Ks), int(kstride), C.byref(params),
+            C.byref(hough), _dptr(out["transforms"]), _dptr(out["inst_offsets"]), _dptr(out["inst_counts"]),
+            _dptr(out["inst_corrs"]), int(out["corr_cap"]), _dptr(out["n_inst"]), _dptr(out["corrs"]),
+            _dptr(out["n_corrs"]), _dptr(out.get("desc")), _dptr(out.get("rf")), _dptr(out["status"])))
+
     # ---- resident FPFH pipeline (FPFH_demo.cpp:405-538) -------------------------------------------
     def model_create_fpfh(self, kp, params):
         kp = _pts(kp)
@@ -940,10 +1011,11 @@ def comm_unique_id():
     return bytes(buf)
 
 
-def register_scene_batch(model, scenes, keypoints, params, lanes=4, device=0):
+def register_scene_batch(model, scenes, keypoints, params, lanes=4, device=0, hough=None):
     """b200_register_scene_batch_shot: a batch of scenes against one resident model, `lanes` scenes in flight on
     `device` (contexts and host threads live inside the library).  Returns one result dict per scene, like
-    Context.register_scene_shot."""
+    Context.register_scene_shot.  With `hough` (HoughParams), b200_register_scene_batch_shot_hough: the Hough branch
+    against a model from Context.model_create_shot_hough."""
     n = len(scenes)
     scenes = [_pts(x) for x in scenes]
     keypoints = [_pts(k) for k in keypoints]
@@ -962,11 +1034,15 @@ def register_scene_batch(model, scenes, keypoints, params, lanes=4, device=0):
     n_inst = np.zeros(max(n, 1), dtype=np.int32)
     n_corr = np.zeros(max(n, 1), dtype=np.int32)
     status = np.zeros(max(n, 1), dtype=np.int32)
-    rc = lib().b200_register_scene_batch_shot(
-        int(device), model.h, n, (fp * n)(*[_f(x) for x in scenes]), _i(npts), stride,
-        (fp * n)(*[_f(k) for k in keypoints]), _i(nkp), kstride, C.byref(params), int(lanes),
-        (fp * n)(*[_f(t) for t in T]), (ip * n)(*[_i(o) for o in off]), (cp * n)(*[_c(a) for a in ic]), _i(cap),
-        _i(n_inst), (cp * n)(*[_c(a) for a in co]), _i(n_corr), _i(status))
+    inputs = (int(device), model.h, n, (fp * n)(*[_f(x) for x in scenes]), _i(npts), stride,
+              (fp * n)(*[_f(k) for k in keypoints]), _i(nkp), kstride, C.byref(params))
+    outputs = (int(lanes), (fp * n)(*[_f(t) for t in T]), (ip * n)(*[_i(o) for o in off]),
+               (cp * n)(*[_c(a) for a in ic]), _i(cap), _i(n_inst), (cp * n)(*[_c(a) for a in co]), _i(n_corr),
+               _i(status))
+    if hough is None:
+        rc = lib().b200_register_scene_batch_shot(*inputs, *outputs)
+    else:
+        rc = lib().b200_register_scene_batch_shot_hough(*inputs, C.byref(hough), *outputs)
     if rc != OK:
         raise B200Error(rc, lib().b200_last_error(None).decode())
     out = []

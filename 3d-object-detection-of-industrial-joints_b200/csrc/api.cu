@@ -1,6 +1,7 @@
 // api.cu — the C ABI of libb200reg.so (include/b200reg.h): argument checking, host<->device staging
 // and the resident SHOT registration pipeline.  No torch types, no exceptions across the boundary.
 #include <algorithm>
+#include <functional>
 #include <mutex>
 #include <thread>
 #include <array>
@@ -121,27 +122,55 @@ int check_params(b200_ctx *ctx, const b200_shot_params *p) {
   return B200_OK;
 }
 
-// scene side of the pipeline on resident buffers
-int scene_pipeline(b200_ctx *ctx, const b200_model *model, b200_cloud *scene, const float4 *d_kp, int Ks,
-                   const b200_shot_params *p, float *d_T, int *d_inst_offsets, int *d_inst_counts,
-                   b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst, b200_corr *d_corrs, int *d_n_corrs,
-                   float *d_desc_out) {
-  DevBuf<float> normals, desc_tmp;
-  B200_TRY(normals.alloc(ctx, (size_t)std::max(scene->n, 1) * 4));
-  WideSection wide;  // this scene's turn for the GPU-wide stages; dev_gc ends it before the grouping kernel
+int check_hough_params(b200_ctx *ctx, const b200_hough_params *h) {
+  if (!h) return ctx->fail(B200_ERR_INVALID, "null Hough params");
+  if (!(h->rf_radius > 0.0)) return ctx->fail(B200_ERR_INVALID, "hough params: rf_radius must be > 0");
+  if (!(h->bin_size > 0.0)) return ctx->fail(B200_ERR_INVALID, "hough params: bin_size must be > 0");
+  return B200_OK;
+}
+
+// normals -> SHOT352 -> correspondence search: the part of the scene pipeline both grouping branches share.  It is
+// the start of this scene's turn for the GPU-wide stages (`wide`), which the grouping stage ends.
+int scene_match(b200_ctx *ctx, const b200_model *model, b200_cloud *scene, const float4 *d_kp, int Ks,
+                const b200_shot_params *p, WideSection &wide, float *d_normals, DevBuf<float> &desc_tmp,
+                float *d_desc_out, b200_corr *d_corrs, int *d_n_corrs) {
   B200_TRY(wide.enter(ctx));
-  B200_TRY(dev_normals(ctx, scene, scene->raw.p, scene->n, true, p->normal_k, p->normal_radius, nullptr, normals.p));
+  B200_TRY(dev_normals(ctx, scene, scene->raw.p, scene->n, true, p->normal_k, p->normal_radius, nullptr, d_normals));
   float *d_desc = d_desc_out;
   if (!d_desc) {
     B200_TRY(desc_tmp.alloc(ctx, (size_t)std::max(Ks, 1) * 352));
     d_desc = desc_tmp.p;
   }
-  B200_TRY(dev_shot(ctx, scene, normals.p, d_kp, Ks, p->descr_radius, d_desc, nullptr, false));
-  B200_TRY(dev_match(ctx, model->desc.p, model->K, d_desc, Ks, 352, p->match_mode, p->match_thr, d_corrs, d_n_corrs,
-                     &model->tc));
-  B200_TRY(dev_gc(ctx, model->kp.p, d_kp, d_corrs, d_n_corrs, Ks, p->gc_size, p->gc_threshold, d_T, p->max_instances,
-                  d_inst_offsets, d_inst_counts, d_inst_corrs, corr_cap, d_n_inst));
-  return B200_OK;
+  B200_TRY(dev_shot(ctx, scene, d_normals, d_kp, Ks, p->descr_radius, d_desc, nullptr, false));
+  return dev_match(ctx, model->desc.p, model->K, d_desc, Ks, 352, p->match_mode, p->match_thr, d_corrs, d_n_corrs,
+                   &model->tc);
+}
+
+// scene side of the pipeline on resident buffers: geometric-consistency grouping (h == nullptr) or the Hough branch
+// (BOARD frames of the scene keypoints -> Hough3DGrouping; d_rf_out nullable, d_status: see dev_hough3d)
+int scene_pipeline(b200_ctx *ctx, const b200_model *model, b200_cloud *scene, const float4 *d_kp, int Ks,
+                   const b200_shot_params *p, float *d_T, int *d_inst_offsets, int *d_inst_counts,
+                   b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst, b200_corr *d_corrs, int *d_n_corrs,
+                   float *d_desc_out, const b200_hough_params *h = nullptr, float *d_rf_out = nullptr,
+                   int *d_status = nullptr) {
+  DevBuf<float> normals, desc_tmp;
+  B200_TRY(normals.alloc(ctx, (size_t)std::max(scene->n, 1) * 4));
+  WideSection wide;  // this scene's turn for the GPU-wide stages; dev_gc / dev_hough3d end it before the latency-bound part
+  B200_TRY(scene_match(ctx, model, scene, d_kp, Ks, p, wide, normals.p, desc_tmp, d_desc_out, d_corrs, d_n_corrs));
+  if (!h)
+    return dev_gc(ctx, model->kp.p, d_kp, d_corrs, d_n_corrs, Ks, p->gc_size, p->gc_threshold, d_T, p->max_instances,
+                  d_inst_offsets, d_inst_counts, d_inst_corrs, corr_cap, d_n_inst);
+  DevBuf<float> rf_tmp;
+  float *d_rf = d_rf_out;
+  if (!d_rf) {
+    B200_TRY(rf_tmp.alloc(ctx, (size_t)std::max(Ks, 1) * 9));
+    d_rf = rf_tmp.p;
+  }
+  uint32_t stream_state[31];  // every scene starts from the model's recorded rand() state
+  memcpy(stream_state, model->rand_state, sizeof(stream_state));
+  B200_TRY(dev_board_lrf_from(ctx, scene, normals.p, d_kp, Ks, h->rf_radius, &h->board, stream_state, d_rf));
+  return dev_hough3d(ctx, model->kp.p, model->votes.p, d_kp, d_rf, d_corrs, d_n_corrs, Ks, h->bin_size, h->threshold,
+                     d_T, p->max_instances, d_inst_offsets, d_inst_counts, d_inst_corrs, corr_cap, d_n_inst, d_status);
 }
 
 __global__ void unpack_points_kernel(const float4 *__restrict__ in, int n, float *__restrict__ out) {
@@ -257,6 +286,7 @@ int b200_ctx_destroy(b200_ctx *ctx) {
   ctx->arena_destroy();
   if (ctx->mt_state) cudaFree(ctx->mt_state);
   if (ctx->mailbox_host) cudaFreeHost(ctx->mailbox_host);
+  if (ctx->board_draws) cudaFreeHost(ctx->board_draws);
   if (ctx->sync_ev) cudaEventDestroy(ctx->sync_ev);
   if (ctx->own_stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
@@ -313,7 +343,7 @@ int b200_ctx_stage_count(void) { return ST_COUNT; }
 const char *b200_ctx_stage_name(int stage) {
   static const char *names[ST_COUNT] = {"grid_build", "normals", "neighbor_count", "shot", "fpfh",
                                         "match",      "gc_sort", "gc_adjacency",   "gc_group", "gc_ransac",
-                                        "match_filter"};
+                                        "match_filter", "board", "hough"};
   return (stage >= 0 && stage < ST_COUNT) ? names[stage] : "";
 }
 
@@ -707,22 +737,30 @@ int b200_hough3d_recognize(b200_ctx *ctx, const float *model_kp, const float *mo
     if (corrs[i].index_query < 0 || corrs[i].index_query >= Km || corrs[i].index_match < 0 ||
         corrs[i].index_match >= Ks)
       return ctx->fail(B200_ERR_INVALID, "hough3d_recognize: correspondence index out of range");
+  if (!(bin_size > 0.0)) return ctx->fail(B200_ERR_INVALID, "hough3d: bin size must be > 0");
   DevBuf<float4> dm, ds;
-  DevBuf<float> dmrf, dsrf, dT;
+  DevBuf<float> dmrf, dsrf, dvotes, dT;
   B200_TRY(upload_points(ctx, model_kp, Km, mstride, dm));
   B200_TRY(upload_points(ctx, scene_kp, Ks, sstride, ds));
   B200_TRY(upload(ctx, dmrf, model_rf, (size_t)Km * 9));
   B200_TRY(upload(ctx, dsrf, scene_rf, (size_t)Ks * 9));
+  B200_TRY(dvotes.alloc(ctx, (size_t)std::max(Km, 1) * 3));
+  B200_TRY(dev_hough_model_votes(ctx, dm.p, dmrf.p, Km, dvotes.p));
   DevBuf<b200_corr> dc, dic;
-  DevBuf<int> doffs, dcnts, dn;
+  DevBuf<int> dC, doffs, dcnts, dn, dstatus;
   B200_TRY(upload(ctx, dc, corrs, (size_t)C));
+  B200_TRY(upload(ctx, dC, &C, 1));
   B200_TRY(dic.alloc(ctx, (size_t)C));
   B200_TRY(doffs.alloc(ctx, (size_t)max_inst + 1));
   B200_TRY(dcnts.alloc(ctx, (size_t)max_inst));
   B200_TRY(dn.alloc(ctx, 1));
+  B200_TRY(dstatus.alloc(ctx, 1));
   B200_TRY(dT.alloc(ctx, (size_t)max_inst * 16));
-  B200_TRY(dev_hough3d(ctx, dm.p, dmrf.p, Km, ds.p, dsrf.p, dc.p, C, bin_size, threshold, dT.p, max_inst, doffs.p, dcnts.p,
-                       dic.p, C, dn.p));
+  B200_TRY(dev_hough3d(ctx, dm.p, dvotes.p, ds.p, dsrf.p, dc.p, dC.p, C, bin_size, threshold, dT.p, max_inst, doffs.p,
+                       dcnts.p, dic.p, C, dn.p, dstatus.p));
+  int status = B200_OK;
+  B200_TRY(readback_small(ctx, dstatus.p, &status, sizeof(int)));
+  if (status == B200_ERR_CAPACITY) return ctx->fail(B200_ERR_CAPACITY, "hough3d: more than 2^27 bins (bin size too small)");
   return download_instances(ctx, dT.p, doffs.p, dcnts.p, dic.p, dn.p, max_inst, C, transforms, inst_offsets,
                             inst_corrs, corr_cap, n_inst);
 }
@@ -787,11 +825,16 @@ int b200_icp_align(b200_ctx *ctx, const float *source, int ns, int sstride, b200
 }
 
 /* ------------------------------------------------------------------ resident pipeline */
-int b200_model_create_shot(b200_ctx *ctx, const float *xyz, int n, int stride, const float *kp, int K, int kstride,
-                           const b200_shot_params *p, b200_model **out) {
-  API_ENTER(ctx);
+}  // extern "C"
+
+namespace {
+// normals + SHOT352 of the model keypoints; with h, also their BOARD frames (from ctx's rand() stream, whose state
+// after them the model records) and the Hough votes
+int model_create(b200_ctx *ctx, const float *xyz, int n, int stride, const float *kp, int K, int kstride,
+                 const b200_shot_params *p, const b200_hough_params *h, b200_model **out) {
   if (!out) return ctx->fail(B200_ERR_INVALID, "model_create: null output");
   B200_TRY(check_params(ctx, p));
+  if (h) B200_TRY(check_hough_params(ctx, h));
   b200_cloud *cloud = nullptr;
   B200_TRY(cloud_upload(ctx, xyz, n, stride, false, &cloud));
   b200_model *m = new b200_model();
@@ -809,6 +852,15 @@ int b200_model_create_shot(b200_ctx *ctx, const float *xyz, int n, int stride, c
     if ((rc = dev_shot(ctx, cloud, normals.p, m->kp.p, K, p->descr_radius, m->desc.p, nullptr, false)) != B200_OK)
       break;
     if ((rc = match_prepare_model(ctx, m)) != B200_OK) break;
+    if (h) {
+      if (!ctx->rand_seeded) board_rand_seed(ctx, 1u);
+      if ((rc = m->rf.alloc(ctx, (size_t)std::max(K, 1) * 9)) != B200_OK) break;
+      if ((rc = m->votes.alloc(ctx, (size_t)std::max(K, 1) * 3)) != B200_OK) break;
+      if ((rc = dev_board_lrf(ctx, cloud, normals.p, m->kp.p, K, h->rf_radius, &h->board, m->rf.p)) != B200_OK) break;
+      if ((rc = dev_hough_model_votes(ctx, m->kp.p, m->rf.p, K, m->votes.p)) != B200_OK) break;
+      memcpy(m->rand_state, ctx->rand_state, sizeof(m->rand_state));
+      m->has_frames = true;
+    }
     cudaError_t e = ctx->sync();
     if (e != cudaSuccess) rc = ctx->fail_cuda(e, "model_create sync", __FILE__, __LINE__);
   } while (0);
@@ -818,6 +870,30 @@ int b200_model_create_shot(b200_ctx *ctx, const float *xyz, int n, int stride, c
     return rc;
   }
   *out = m;
+  return B200_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int b200_model_create_shot(b200_ctx *ctx, const float *xyz, int n, int stride, const float *kp, int K, int kstride,
+                           const b200_shot_params *p, b200_model **out) {
+  API_ENTER(ctx);
+  return model_create(ctx, xyz, n, stride, kp, K, kstride, p, nullptr, out);
+}
+
+int b200_model_create_shot_hough(b200_ctx *ctx, const float *xyz, int n, int stride, const float *kp, int K, int kstride,
+                                 const b200_shot_params *p, const b200_hough_params *h, b200_model **out) {
+  API_ENTER(ctx);
+  return model_create(ctx, xyz, n, stride, kp, K, kstride, p, h, out);
+}
+
+int b200_model_download_frames(b200_ctx *ctx, const b200_model *m, float *rf) {
+  API_ENTER(ctx);
+  if (!m || !m->has_frames) return ctx->fail(B200_ERR_INVALID, "model_download_frames: the model has no frames");
+  if (m->K > 0 && !rf) return ctx->fail(B200_ERR_INVALID, "model_download_frames: null output");
+  B200_TRY(download(ctx, rf, m->rf.p, (size_t)m->K * 9));
+  B200_CUDA(ctx, ctx->sync());
   return B200_OK;
 }
 
@@ -845,34 +921,47 @@ int b200_model_download(b200_ctx *ctx, const b200_model *m, float *desc, float *
   return B200_OK;
 }
 
-int b200_dev_register_scene_shot(b200_ctx *ctx, const b200_model *model, const float *d_scene_xyz, int n, int stride,
-                                 const float *d_scene_kp, int Ks, int kstride, const b200_shot_params *p,
-                                 float *d_transforms, int *d_inst_offsets, int *d_inst_counts,
-                                 b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst, b200_corr *d_corrs_out,
-                                 int *d_n_corrs, float *d_desc_out) {
-  API_ENTER(ctx);
+}  // extern "C"
+
+namespace {
+// b200_dev_register_scene_shot (h == nullptr) / b200_dev_register_scene_shot_hough
+int dev_register_scene(b200_ctx *ctx, const b200_model *model, const float *d_scene_xyz, int n, int stride,
+                       const float *d_scene_kp, int Ks, int kstride, const b200_shot_params *p, float *d_transforms,
+                       int *d_inst_offsets, int *d_inst_counts, b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst,
+                       b200_corr *d_corrs_out, int *d_n_corrs, float *d_desc_out, const b200_hough_params *h,
+                       float *d_rf_out, int *d_status) {
   if (!model || !d_transforms || !d_inst_offsets || !d_inst_counts || !d_inst_corrs || !d_n_inst || !d_corrs_out ||
-      !d_n_corrs || Ks < 0)
+      !d_n_corrs || Ks < 0 || (h && !d_status))
     return ctx->fail(B200_ERR_INVALID, "register_scene: bad arguments");
   B200_TRY(check_params(ctx, p));
+  if (h) {
+    B200_TRY(check_hough_params(ctx, h));
+    if (!model->has_frames)
+      return ctx->fail(B200_ERR_INVALID, "register_scene_hough: the model has no frames (b200_model_create_shot_hough)");
+  }
   b200_cloud *scene = nullptr;
   B200_TRY(cloud_upload(ctx, d_scene_xyz, n, stride, true, &scene));
   DevBuf<float4> dkp;
   int rc = pack_device_points(ctx, d_scene_kp, Ks, kstride, dkp);
   if (rc == B200_OK)
     rc = scene_pipeline(ctx, model, scene, dkp.p, Ks, p, d_transforms, d_inst_offsets, d_inst_counts, d_inst_corrs,
-                        corr_cap, d_n_inst, d_corrs_out, d_n_corrs, d_desc_out);
+                        corr_cap, d_n_inst, d_corrs_out, d_n_corrs, d_desc_out, h, d_rf_out, d_status);
   delete scene;
   return rc;
 }
 
-int b200_register_scene_shot(b200_ctx *ctx, const b200_model *model, const float *scene_xyz, int n, int stride,
-                             const float *scene_kp, int Ks, int kstride, const b200_shot_params *p, float *transforms,
-                             int *inst_offsets, b200_corr *inst_corrs, int corr_cap, int *n_inst, b200_corr *corrs_out,
-                             int *n_corrs) {
-  API_ENTER(ctx);
+// b200_register_scene_shot (h == nullptr) / b200_register_scene_shot_hough
+int register_scene(b200_ctx *ctx, const b200_model *model, const float *scene_xyz, int n, int stride,
+                   const float *scene_kp, int Ks, int kstride, const b200_shot_params *p, float *transforms,
+                   int *inst_offsets, b200_corr *inst_corrs, int corr_cap, int *n_inst, b200_corr *corrs_out,
+                   int *n_corrs, const b200_hough_params *h, float *rf_out) {
   if (!model || !n_inst || Ks < 0) return ctx->fail(B200_ERR_INVALID, "register_scene: bad arguments");
   B200_TRY(check_params(ctx, p));
+  if (h) {
+    B200_TRY(check_hough_params(ctx, h));
+    if (!model->has_frames)
+      return ctx->fail(B200_ERR_INVALID, "register_scene_hough: the model has no frames (b200_model_create_shot_hough)");
+  }
   *n_inst = 0;
   if (n_corrs) *n_corrs = 0;
   HostTrace tr;
@@ -885,8 +974,8 @@ int b200_register_scene_shot(b200_ctx *ctx, const b200_model *model, const float
     if ((rc = upload_points(ctx, scene_kp, Ks, kstride, dkp)) != B200_OK) break;
     const int cap = std::max(Ks, 1);
     DevBuf<b200_corr> dcorrs, dic;
-    DevBuf<int> doffs, dcnts, dn, dnc;
-    DevBuf<float> dT;
+    DevBuf<int> doffs, dcnts, dn, dnc, dstatus;
+    DevBuf<float> dT, drf;
     if ((rc = dcorrs.alloc(ctx, (size_t)cap)) != B200_OK) break;
     if ((rc = dic.alloc(ctx, (size_t)cap)) != B200_OK) break;
     if ((rc = doffs.alloc(ctx, (size_t)p->max_instances + 1)) != B200_OK) break;
@@ -894,12 +983,15 @@ int b200_register_scene_shot(b200_ctx *ctx, const b200_model *model, const float
     if ((rc = dn.alloc(ctx, 1)) != B200_OK) break;
     if ((rc = dnc.alloc(ctx, 1)) != B200_OK) break;
     if ((rc = dT.alloc(ctx, (size_t)p->max_instances * 16)) != B200_OK) break;
+    if (h && (rc = dstatus.alloc(ctx, 1)) != B200_OK) break;
+    if (h && (rc = drf.alloc(ctx, (size_t)cap * 9)) != B200_OK) break;
     if ((rc = scene_pipeline(ctx, model, scene, dkp.p, Ks, p, dT.p, doffs.p, dcnts.p, dic.p, cap, dn.p, dcorrs.p,
-                             dnc.p, nullptr)) != B200_OK)
+                             dnc.p, nullptr, h, drf.p, dstatus.p)) != B200_OK)
       break;
     tr.tick("e2e pipeline issue");
-    int nc = 0;
+    int nc = 0, status = B200_OK;
     if ((rc = download(ctx, &nc, dnc.p, 1)) != B200_OK) break;
+    if (h && (rc = download(ctx, &status, dstatus.p, 1)) != B200_OK) break;
     cudaError_t e = ctx->sync();
     if (e != cudaSuccess) {
       rc = ctx->fail_cuda(e, "register_scene sync", __FILE__, __LINE__);
@@ -910,12 +1002,66 @@ int b200_register_scene_shot(b200_ctx *ctx, const b200_model *model, const float
     if (corrs_out && nc > 0) {
       if ((rc = download(ctx, corrs_out, dcorrs.p, (size_t)nc)) != B200_OK) break;
     }
+    if (rf_out && Ks > 0 && (rc = download(ctx, rf_out, drf.p, (size_t)Ks * 9)) != B200_OK) break;
+    if (status == B200_ERR_CAPACITY) {
+      const cudaError_t es = ctx->sync();  // the downloads above land before the call returns
+      rc = es != cudaSuccess ? ctx->fail_cuda(es, "register_scene sync", __FILE__, __LINE__)
+                             : ctx->fail(B200_ERR_CAPACITY, "hough3d: more than 2^27 bins (bin size too small)");
+      break;
+    }
     rc = download_instances(ctx, dT.p, doffs.p, dcnts.p, dic.p, dn.p, p->max_instances, cap, transforms, inst_offsets,
                             inst_corrs, corr_cap, n_inst);
     tr.tick("e2e download");
   } while (0);
   delete scene;
   return rc;
+}
+}  // namespace
+
+extern "C" {
+
+int b200_dev_register_scene_shot(b200_ctx *ctx, const b200_model *model, const float *d_scene_xyz, int n, int stride,
+                                 const float *d_scene_kp, int Ks, int kstride, const b200_shot_params *p,
+                                 float *d_transforms, int *d_inst_offsets, int *d_inst_counts,
+                                 b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst, b200_corr *d_corrs_out,
+                                 int *d_n_corrs, float *d_desc_out) {
+  API_ENTER(ctx);
+  return dev_register_scene(ctx, model, d_scene_xyz, n, stride, d_scene_kp, Ks, kstride, p, d_transforms, d_inst_offsets,
+                            d_inst_counts, d_inst_corrs, corr_cap, d_n_inst, d_corrs_out, d_n_corrs, d_desc_out, nullptr,
+                            nullptr, nullptr);
+}
+
+int b200_dev_register_scene_shot_hough(b200_ctx *ctx, const b200_model *model, const float *d_scene_xyz, int n,
+                                       int stride, const float *d_scene_kp, int Ks, int kstride,
+                                       const b200_shot_params *p, const b200_hough_params *h, float *d_transforms,
+                                       int *d_inst_offsets, int *d_inst_counts, b200_corr *d_inst_corrs, int corr_cap,
+                                       int *d_n_inst, b200_corr *d_corrs_out, int *d_n_corrs, float *d_desc_out,
+                                       float *d_rf_out, int *d_status) {
+  API_ENTER(ctx);
+  if (!h) return ctx->fail(B200_ERR_INVALID, "null Hough params");
+  return dev_register_scene(ctx, model, d_scene_xyz, n, stride, d_scene_kp, Ks, kstride, p, d_transforms, d_inst_offsets,
+                            d_inst_counts, d_inst_corrs, corr_cap, d_n_inst, d_corrs_out, d_n_corrs, d_desc_out, h,
+                            d_rf_out, d_status);
+}
+
+int b200_register_scene_shot(b200_ctx *ctx, const b200_model *model, const float *scene_xyz, int n, int stride,
+                             const float *scene_kp, int Ks, int kstride, const b200_shot_params *p, float *transforms,
+                             int *inst_offsets, b200_corr *inst_corrs, int corr_cap, int *n_inst, b200_corr *corrs_out,
+                             int *n_corrs) {
+  API_ENTER(ctx);
+  return register_scene(ctx, model, scene_xyz, n, stride, scene_kp, Ks, kstride, p, transforms, inst_offsets, inst_corrs,
+                        corr_cap, n_inst, corrs_out, n_corrs, nullptr, nullptr);
+}
+
+int b200_register_scene_shot_hough(b200_ctx *ctx, const b200_model *model, const float *scene_xyz, int n, int stride,
+                                   const float *scene_kp, int Ks, int kstride, const b200_shot_params *p,
+                                   const b200_hough_params *h, float *transforms, int *inst_offsets,
+                                   b200_corr *inst_corrs, int corr_cap, int *n_inst, b200_corr *corrs_out, int *n_corrs,
+                                   float *rf_out) {
+  API_ENTER(ctx);
+  if (!h) return ctx->fail(B200_ERR_INVALID, "null Hough params");
+  return register_scene(ctx, model, scene_xyz, n, stride, scene_kp, Ks, kstride, p, transforms, inst_offsets, inst_corrs,
+                        corr_cap, n_inst, corrs_out, n_corrs, h, rf_out);
 }
 
 /* ------------------------------------------------------------------ resident FPFH pipeline */
@@ -1161,18 +1307,11 @@ LanePool &lane_pool(int device) {
   static LanePool pools[64];
   return pools[(device >= 0 && device < 64) ? device : 0];
 }
-}  // namespace
 
-int b200_register_scene_batch_shot(int device, const b200_model *model, int n_scenes, const float *const *scene_xyz,
-                                   const int *n_points, int stride, const float *const *scene_kp, const int *n_kp,
-                                   int kstride, const b200_shot_params *p, int lanes, float *const *transforms,
-                                   int *const *inst_offsets, b200_corr *const *inst_corrs, const int *corr_cap,
-                                   int *n_inst, b200_corr *const *corrs_out, int *n_corrs, int *status) {
-  if (!model || n_scenes < 0 || lanes < 1 || lanes > 16 || !p ||
-      (n_scenes > 0 && (!scene_xyz || !n_points || !scene_kp || !n_kp || !n_inst || !status))) {
-    g_error = "register_scene_batch: bad arguments";
-    return B200_ERR_INVALID;
-  }
+// The lane driver of the batch calls: `lanes` pooled contexts of `device`, one host thread each; lane l registers
+// scenes l, l + lanes, ... through scene(ctx, s), whose return code goes to status[s].  Returns the first status
+// other than B200_OK / B200_ERR_CAPACITY (with that lane's error text), else B200_OK.
+int run_lanes(int device, int n_scenes, int lanes, int *status, const std::function<int(b200_ctx *, int)> &scene) {
   if (n_scenes == 0) return B200_OK;
   lanes = std::min(lanes, n_scenes);
   LanePool &pool = lane_pool(device);
@@ -1188,14 +1327,7 @@ int b200_register_scene_batch_shot(int device, const b200_model *model, int n_sc
   for (int l = 0; l < lanes; ++l) pool.ctxs[(size_t)l]->blocking_sync = hw != 0 && (unsigned)lanes > hw;
   auto work = [&](int lane) {
     b200_ctx *c = pool.ctxs[(size_t)lane];
-    for (int s = lane; s < n_scenes; s += lanes) {
-      int nc = 0;
-      status[s] = b200_register_scene_shot(c, model, scene_xyz[s], n_points[s], stride, scene_kp[s], n_kp[s], kstride, p,
-                                           transforms ? transforms[s] : nullptr, inst_offsets ? inst_offsets[s] : nullptr,
-                                           inst_corrs ? inst_corrs[s] : nullptr, corr_cap ? corr_cap[s] : 0, &n_inst[s],
-                                           corrs_out ? corrs_out[s] : nullptr, &nc);
-      if (n_corrs) n_corrs[s] = nc;
-    }
+    for (int s = lane; s < n_scenes; s += lanes) status[s] = scene(c, s);
   };
   std::vector<std::thread> threads;
   for (int l = 1; l < lanes; ++l) threads.emplace_back(work, l);
@@ -1208,6 +1340,57 @@ int b200_register_scene_batch_shot(int device, const b200_model *model, int n_sc
       return status[s];
     }
   return B200_OK;
+}
+
+bool batch_args_ok(const b200_model *model, int n_scenes, const float *const *scene_xyz, const int *n_points,
+                   const float *const *scene_kp, const int *n_kp, const b200_shot_params *p, int lanes, int *n_inst,
+                   int *status) {
+  return model && n_scenes >= 0 && lanes >= 1 && lanes <= 16 && p &&
+         !(n_scenes > 0 && (!scene_xyz || !n_points || !scene_kp || !n_kp || !n_inst || !status));
+}
+}  // namespace
+
+int b200_register_scene_batch_shot(int device, const b200_model *model, int n_scenes, const float *const *scene_xyz,
+                                   const int *n_points, int stride, const float *const *scene_kp, const int *n_kp,
+                                   int kstride, const b200_shot_params *p, int lanes, float *const *transforms,
+                                   int *const *inst_offsets, b200_corr *const *inst_corrs, const int *corr_cap,
+                                   int *n_inst, b200_corr *const *corrs_out, int *n_corrs, int *status) {
+  if (!batch_args_ok(model, n_scenes, scene_xyz, n_points, scene_kp, n_kp, p, lanes, n_inst, status)) {
+    g_error = "register_scene_batch: bad arguments";
+    return B200_ERR_INVALID;
+  }
+  return run_lanes(device, n_scenes, lanes, status, [&](b200_ctx *c, int s) {
+    int nc = 0;
+    const int rc = b200_register_scene_shot(c, model, scene_xyz[s], n_points[s], stride, scene_kp[s], n_kp[s], kstride, p,
+                                            transforms ? transforms[s] : nullptr, inst_offsets ? inst_offsets[s] : nullptr,
+                                            inst_corrs ? inst_corrs[s] : nullptr, corr_cap ? corr_cap[s] : 0, &n_inst[s],
+                                            corrs_out ? corrs_out[s] : nullptr, &nc);
+    if (n_corrs) n_corrs[s] = nc;
+    return rc;
+  });
+}
+
+int b200_register_scene_batch_shot_hough(int device, const b200_model *model, int n_scenes,
+                                         const float *const *scene_xyz, const int *n_points, int stride,
+                                         const float *const *scene_kp, const int *n_kp, int kstride,
+                                         const b200_shot_params *p, const b200_hough_params *h, int lanes,
+                                         float *const *transforms, int *const *inst_offsets,
+                                         b200_corr *const *inst_corrs, const int *corr_cap, int *n_inst,
+                                         b200_corr *const *corrs_out, int *n_corrs, int *status) {
+  if (!batch_args_ok(model, n_scenes, scene_xyz, n_points, scene_kp, n_kp, p, lanes, n_inst, status) || !h) {
+    g_error = "register_scene_batch_hough: bad arguments";
+    return B200_ERR_INVALID;
+  }
+  return run_lanes(device, n_scenes, lanes, status, [&](b200_ctx *c, int s) {
+    int nc = 0;
+    const int rc = b200_register_scene_shot_hough(
+        c, model, scene_xyz[s], n_points[s], stride, scene_kp[s], n_kp[s], kstride, p, h,
+        transforms ? transforms[s] : nullptr, inst_offsets ? inst_offsets[s] : nullptr,
+        inst_corrs ? inst_corrs[s] : nullptr, corr_cap ? corr_cap[s] : 0, &n_inst[s], corrs_out ? corrs_out[s] : nullptr,
+        &nc, nullptr);
+    if (n_corrs) n_corrs[s] = nc;
+    return rc;
+  });
 }
 
 int b200_lanes_release(int device) {

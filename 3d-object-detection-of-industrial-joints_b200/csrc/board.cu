@@ -698,11 +698,18 @@ void glibc_seed(unsigned seed, uint32_t st[31]) {
   for (int i = 0; i < 31; ++i) st[i] = r[313 + i];
 }
 
-int glibc_next(uint32_t st[31]) {
-  const uint32_t o = st[0] + st[28];
-  for (int i = 0; i < 30; ++i) st[i] = st[i + 1];
-  st[30] = o;
-  return (int)(o >> 1);
+// the next `count` rand() values of the stream st (st[0] oldest), which is advanced past them
+void glibc_fill(uint32_t st[31], int *out, int count) {
+  uint32_t r[31];
+  memcpy(r, st, sizeof(r));
+  int h = 0;  // st[k] == r[(h + k) % 31]
+  for (int i = 0; i < count; ++i) {
+    const uint32_t o = r[h] + r[(h + 28) % 31];
+    r[h] = o;
+    h = (h + 1) % 31;
+    out[i] = (int)(o >> 1);
+  }
+  for (int k = 0; k < 31; ++k) st[k] = r[(h + k) % 31];
 }
 
 }  // namespace
@@ -712,50 +719,54 @@ void board_rand_seed(b200_ctx *ctx, unsigned seed) {
   ctx->rand_seeded = true;
 }
 
-// d_normals: one row of 4 floats per surface point, original order.  d_rf: K x 9.  Synchronises the stream.
-int dev_board_lrf(b200_ctx *ctx, b200_cloud *c, const float *d_normals, const float4 *d_kp, int K, double radius,
-                  const b200_board_params *p, float *d_rf) {
+// d_normals: one row of 4 floats per surface point, original order.  d_rf: K x 9.  The random axes draw from
+// rand_state, which is advanced by exactly two values per keypoint with a full support.  Host waits: one
+// readback_small (the support maxima, which size the CTA kernel's shared memory, and the number of full supports).
+int dev_board_lrf_from(b200_ctx *ctx, b200_cloud *c, const float *d_normals, const float4 *d_kp, int K, double radius,
+                       const b200_board_params *p, uint32_t rand_state[31], float *d_rf) {
   if (!(radius > 0.0)) return ctx->fail(B200_ERR_INVALID, "board_lrf: radius must be > 0");
   if (p->check_margin_array_size < 1 || p->check_margin_array_size > BOARD_MAX_SECTORS)
     return ctx->fail(B200_ERR_INVALID, "board_lrf: check_margin_array_size must be in 1..64");
   const bool second = p->tangent_radius != 0.0f && (double)p->tangent_radius != radius;
   if (K <= 0) return B200_OK;
+  StageScope st_(ctx, ST_BOARD);
   const GridView *g;
   B200_TRY(cloud_grid_for_radius(c, radius, &g));
-  DevBuf<int> counts, flags, rank, rnd;
-  DevBuf<unsigned long long> stats;
+  DevBuf<int> counts, counts2, flags, rank, rnd;
+  DevBuf<unsigned long long> info;  // [0] support max, [2] x-axis support max (second search), [4] full supports
   B200_TRY(counts.alloc(ctx, (size_t)K));
   B200_TRY(flags.alloc(ctx, (size_t)K));
   B200_TRY(rank.alloc(ctx, (size_t)K));
-  B200_TRY(stats.alloc(ctx, 2));
-  B200_TRY(dev_radius_count(ctx, *g, d_kp, K, radius, counts.p, stats.p));
+  B200_TRY(info.alloc(ctx, 5));
+  B200_TRY(info.zero());
+  B200_TRY(dev_radius_count(ctx, *g, d_kp, K, radius, counts.p, info.p));
+  if (second) {  // the x-axis support may be larger than the plane-fit support
+    B200_TRY(counts2.alloc(ctx, (size_t)K));
+    B200_TRY(dev_radius_count(ctx, *g, d_kp, K, (double)p->tangent_radius, counts2.p, info.p + 2));
+  }
   board_flags_kernel<<<ceil_div(K, 256), 256, 0, ctx->stream>>>(counts.p, K, flags.p);
   B200_LAUNCHED(ctx);
-  DevBuf<int> total;
-  B200_TRY(total.alloc(ctx, 1));
-  B200_TRY(exclusive_scan_i32(ctx, flags.p, rank.p, K, total.p));
-  unsigned long long hstats[2];
-  int n_full = 0;
-  B200_CUDA(ctx, cudaMemcpyAsync(hstats, stats.p, sizeof(hstats), cudaMemcpyDeviceToHost, ctx->stream));
-  B200_CUDA(ctx, cudaMemcpyAsync(&n_full, total.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  B200_CUDA(ctx, ctx->sync());
-  int max_count = (int)hstats[0];
-  if (second) {  // the x-axis support may be larger than the plane-fit support
-    DevBuf<int> counts2;
-    B200_TRY(counts2.alloc(ctx, (size_t)K));
-    B200_TRY(dev_radius_count(ctx, *g, d_kp, K, (double)p->tangent_radius, counts2.p, stats.p));
-    B200_CUDA(ctx, cudaMemcpyAsync(hstats, stats.p, sizeof(hstats), cudaMemcpyDeviceToHost, ctx->stream));
-    B200_CUDA(ctx, ctx->sync());
-    max_count = std::max(max_count, (int)hstats[0]);
+  B200_TRY(exclusive_scan_i32(ctx, flags.p, rank.p, K, reinterpret_cast<int *>(info.p + 4)));
+  unsigned long long hinfo[5];
+  B200_TRY(readback_small(ctx, info.p, hinfo, sizeof(hinfo)));
+  const int max_count = second ? (int)std::max(hinfo[0], hinfo[2]) : (int)hinfo[0];
+  const int n_full = (int)(unsigned)hinfo[4];
+  // two rand() values per keypoint with a full support, in keypoint order (PCL's serial loop), staged in the
+  // context's pinned buffer.  Refilling it here is safe: the readback_small above drained the stream, so the copy
+  // an earlier call enqueued from it has completed.
+  B200_TRY(rnd.alloc(ctx, (size_t)std::max(2 * n_full, 1)));
+  if (p->find_holes && n_full > 0) {
+    const size_t need = (size_t)2 * n_full;
+    if (ctx->board_draws_cap < need) {
+      if (ctx->board_draws) cudaFreeHost(ctx->board_draws);
+      ctx->board_draws = nullptr;
+      ctx->board_draws_cap = 0;
+      B200_CUDA(ctx, cudaHostAlloc((void **)&ctx->board_draws, need * sizeof(int), cudaHostAllocDefault));
+      ctx->board_draws_cap = need;
+    }
+    glibc_fill(rand_state, ctx->board_draws, (int)need);
+    B200_CUDA(ctx, cudaMemcpyAsync(rnd.p, ctx->board_draws, need * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   }
-  // two rand() values per keypoint with a full support, in keypoint order (PCL's serial loop)
-  std::vector<int> hr((size_t)std::max(2 * n_full, 1), 0);
-  if (p->find_holes) {
-    if (!ctx->rand_seeded) board_rand_seed(ctx, 1u);
-    for (int i = 0; i < 2 * n_full; ++i) hr[(size_t)i] = glibc_next(ctx->rand_state);
-  }
-  B200_TRY(rnd.alloc(ctx, hr.size()));
-  B200_CUDA(ctx, cudaMemcpyAsync(rnd.p, hr.data(), sizeof(int) * hr.size(), cudaMemcpyHostToDevice, ctx->stream));
   BoardArgs a;
   a.second_search = second ? 1 : 0;
   a.tangent_r2 = (float)((double)p->tangent_radius * (double)p->tangent_radius);
@@ -770,7 +781,6 @@ int dev_board_lrf(b200_ctx *ctx, b200_cloud *c, const float *d_normals, const fl
   // two-radius form (setTangentRadius, never used by the reference) stays with the CTA kernel
   const char *sel = getenv("B200_BOARD");
   const bool warp_path = !second && !(sel && !strcmp(sel, "cta"));
-  int rc = B200_OK;
   if (warp_path) {
     const size_t smem_w = sizeof(BwSmem) * BW_WARPS;
     B200_CUDA(ctx, ensure_dyn_smem(board_warp_kernel, smem_w));
@@ -802,6 +812,12 @@ int dev_board_lrf(b200_ctx *ctx, b200_cloud *c, const float *d_normals, const fl
                                                          rank.p, rnd.p, d_rf, counts.p, min_count);
     B200_LAUNCHED(ctx);
   }
-  B200_CUDA(ctx, ctx->sync());  // hr is a host vector
-  return rc;
+  return B200_OK;
+}
+
+// b200_board_lrf: draws from the context's stream (srand(1) unless reseeded), which then continues after them
+int dev_board_lrf(b200_ctx *ctx, b200_cloud *c, const float *d_normals, const float4 *d_kp, int K, double radius,
+                  const b200_board_params *p, float *d_rf) {
+  if (p->find_holes && !ctx->rand_seeded) board_rand_seed(ctx, 1u);
+  return dev_board_lrf_from(ctx, c, d_normals, d_kp, K, radius, p, ctx->rand_state, d_rf);
 }

@@ -32,6 +32,8 @@ enum b200_stage {
   ST_GC_GROUP,
   ST_GC_RANSAC,
   ST_MATCH_FILTER,  // nested inside ST_MATCH: the tcgen05 pre-filter kernel alone
+  ST_BOARD,         // BOARD reference frames (board.cu)
+  ST_HOUGH,         // Hough voting and maxima (hough.cu); its RANSAC is ST_GC_RANSAC
   ST_COUNT
 };
 
@@ -139,6 +141,8 @@ struct b200_ctx {
   void *mailbox_dev = nullptr;
   uint32_t rand_state[31] = {0};  // glibc rand() stream for BOARD's random axis (board.cu)
   bool rand_seeded = false;
+  int *board_draws = nullptr;  // pinned staging of BOARD's rand() draws (board.cu)
+  size_t board_draws_cap = 0;
   double last_mean_nbrs = 0.0;
   int last_max_nbrs = 0;
   float last_match_err_ratio = 0.f;  // max observed approximation error / assumed bound (profiling only)
@@ -361,6 +365,11 @@ struct b200_model {
   DevBuf<float> desc;  // K x D
   DevBuf<float4> kp;   // K keypoints
   TcModelPrep tc;      // filled by match_prepare_model for libraries large enough for the tensor-core path
+  // Hough branch (b200_model_create_shot_hough)
+  bool has_frames = false;
+  DevBuf<float> rf;             // K x 9 BOARD frames of the keypoints
+  DevBuf<float> votes;          // K x 3 Hough3DGrouping::train() votes
+  uint32_t rand_state[31] = {0};  // the creating context's rand() stream right after the frames
 };
 
 struct b200_library {
@@ -484,12 +493,16 @@ int dev_ransac_instances(b200_ctx *ctx, const b200_corr *d_corrs, const float4 *
                          double threshold, float *d_T, int max_inst, int *d_inst_counts, b200_corr *d_inst_corrs,
                          int corr_cap);
 // hough.cu
-int dev_hough3d(b200_ctx *ctx, const float4 *d_model_kp, const float *d_model_rf, int Km, const float4 *d_scene_kp,
-                const float *d_scene_rf, const b200_corr *d_corrs, int C, double bin_size, double threshold, float *d_T,
-                int max_inst, int *d_inst_offsets, int *d_inst_counts, b200_corr *d_inst_corrs, int corr_cap,
-                int *d_n_inst);
+int dev_hough_model_votes(b200_ctx *ctx, const float4 *d_model_kp, const float *d_model_rf, int Km, float *d_votes);
+// correspondence count: *d_C (at most C_cap); *d_status = B200_ERR_CAPACITY when the space has more than 2^27 bins
+int dev_hough3d(b200_ctx *ctx, const float4 *d_model_kp, const float *d_model_votes, const float4 *d_scene_kp,
+                const float *d_scene_rf, const b200_corr *d_corrs, const int *d_C, int C_cap, double bin_size,
+                double threshold, float *d_T, int max_inst, int *d_inst_offsets, int *d_inst_counts,
+                b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst, int *d_status);
 // board.cu
 void board_rand_seed(b200_ctx *ctx, unsigned seed);
+int dev_board_lrf_from(b200_ctx *ctx, b200_cloud *c, const float *d_normals, const float4 *d_kp, int K, double radius,
+                       const b200_board_params *p, uint32_t rand_state[31], float *d_rf);
 int dev_board_lrf(b200_ctx *ctx, b200_cloud *c, const float *d_normals, const float4 *d_kp, int K, double radius,
                   const b200_board_params *p, float *d_rf);
 // icp.cu

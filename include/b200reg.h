@@ -192,7 +192,8 @@ B200_API int b200_desc_index_knn(b200_ctx *ctx, const b200_desc_index *index, co
  * (x, y, z axes); NaN rows for keypoints with fewer than 6 support points.  With find_holes PCL draws two rand()
  * values per keypoint with a full support, in keypoint order, from the process-wide stream; here the stream
  * (glibc's generator) belongs to the context: a new context is srand(1), b200_ctx_srand reseeds it, and successive
- * calls continue it (model frames, then scene frames, like the reference's two compute() calls). */
+ * calls continue it (model frames, then scene frames, like the reference's two compute() calls).  The resident Hough
+ * branch (b200_model_create_shot_hough) instead fixes the scene frames' stream per model: see there. */
 typedef struct b200_board_params {
   int find_holes;
   float tangent_radius; /* 0: PCL's code path when setTangentRadius is never called */
@@ -315,6 +316,63 @@ B200_API int b200_register_scene_batch_shot(int device, const b200_model *model,
 /* The lane contexts of b200_register_scene_batch_shot (streams, arenas: about 1.3 GB each for a 1 M-point scene) stay
  * alive between batches; this frees the ones of `device`. */
 B200_API int b200_lanes_release(int device);
+
+/* ---------------------------------------------------------------- resident Hough branch -- */
+/* The reference's default branch (use_hough_ = true: SHOT.cpp:433-470, SHOT_demo.cpp:540-577): BOARD frames of the
+ * model and scene keypoints, then Hough3DGrouping, on the resident pipeline. */
+typedef struct {
+  double rf_radius;          /* BOARDLocalReferenceFrameEstimation::setRadiusSearch (rf_rad_) */
+  b200_board_params board;   /* the reference sets find_holes = 1 */
+  double bin_size;           /* Hough3DGrouping::setHoughBinSize (cg_size_) */
+  double threshold;          /* setHoughThreshold (cg_thresh_; negative = fraction of the largest bin) */
+} b200_hough_params;
+
+/* What b200_model_create_shot builds (identical descriptors), plus, kept on the device: the BOARD frames of the model
+ * keypoints (over the model cloud and the normals computed there) and Hough3DGrouping::train()'s votes.
+ * The rand() stream: the model's frames draw from ctx's stream exactly as b200_board_lrf does (ctx's stream then
+ * continues after them), and the model records the stream's state after its frames.  EVERY scene registered against
+ * the model draws its frames from that recorded state, so a registration gives what a fresh process doing
+ * srand(seed) -> model frames -> scene frames computes, whatever the scene order, lane count or context.  (A
+ * long-running PCL process instead keeps one stream going across its callbacks; b200_board_lrf offers that.) */
+B200_API int b200_model_create_shot_hough(b200_ctx *ctx, const float *xyz, int n, int stride, const float *kp, int K,
+                                          int kstride, const b200_shot_params *p, const b200_hough_params *h,
+                                          b200_model **out);
+/* rf: K x 9.  B200_ERR_INVALID for a model without frames (not made by b200_model_create_shot_hough). */
+B200_API int b200_model_download_frames(b200_ctx *ctx, const b200_model *m, float *rf);
+
+/* Scene side of the Hough branch in one call: normals -> SHOT352 -> correspondence search (as in
+ * b200_register_scene_shot) -> BOARD frames of the scene keypoints over the scene cloud and its normals ->
+ * Hough3DGrouping -> RANSAC poses.  Outputs as b200_register_scene_shot; p->gc_size / p->gc_threshold are not read.
+ * rf_out (Ks x 9, nullable): the scene frames.  B200_ERR_CAPACITY when the Hough space would exceed 2^27 bins (no
+ * instance; the correspondences are still returned) or there are more than p->max_instances instances (the first
+ * ones are kept).  B200_ERR_INVALID for a model without frames. */
+B200_API int b200_register_scene_shot_hough(b200_ctx *ctx, const b200_model *model, const float *scene_xyz, int n,
+                                            int stride, const float *scene_kp, int Ks, int kstride,
+                                            const b200_shot_params *p, const b200_hough_params *h, float *transforms,
+                                            int *inst_offsets, b200_corr *inst_corrs, int corr_cap, int *n_inst,
+                                            b200_corr *corrs_out, int *n_corrs, float *rf_out);
+
+/* Device-pointer, asynchronous form (as b200_dev_register_scene_shot).  d_rf_out (Ks x 9) may be NULL; *d_status (a
+ * device int) receives B200_OK, or B200_ERR_CAPACITY when the Hough space would exceed 2^27 bins. */
+B200_API int b200_dev_register_scene_shot_hough(b200_ctx *ctx, const b200_model *model, const float *d_scene_xyz, int n,
+                                                int stride, const float *d_scene_kp, int Ks, int kstride,
+                                                const b200_shot_params *p, const b200_hough_params *h,
+                                                float *d_transforms, int *d_inst_offsets, int *d_inst_counts,
+                                                b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst,
+                                                b200_corr *d_corrs_out, int *d_n_corrs, float *d_desc_out,
+                                                float *d_rf_out, int *d_status);
+
+/* Lanes form, arguments and outputs as b200_register_scene_batch_shot plus h.  Results are those of
+ * b200_register_scene_shot_hough scene by scene: the rand() draws and every grouping step are the same.  One exception:
+ * a BOARD frame can differ in its last bit between two builds of the same scene cloud.  This happens for about 1 row in
+ * 50 000 on 1 M-point scenes (DESIGN §7). */
+B200_API int b200_register_scene_batch_shot_hough(int device, const b200_model *model, int n_scenes,
+                                                  const float *const *scene_xyz, const int *n_points, int stride,
+                                                  const float *const *scene_kp, const int *n_kp, int kstride,
+                                                  const b200_shot_params *p, const b200_hough_params *h, int lanes,
+                                                  float *const *transforms, int *const *inst_offsets,
+                                                  b200_corr *const *inst_corrs, const int *corr_cap, int *n_inst,
+                                                  b200_corr *const *corrs_out, int *n_corrs, int *status);
 
 /* ---------------------------------------------------------------- multi-view library ----- */
 /* The reference recognises against a set of rendered partial views of the CAD models: CAD_desc.cpp:231-370
