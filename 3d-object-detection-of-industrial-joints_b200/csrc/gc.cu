@@ -12,16 +12,17 @@
 // (rejected candidates never influence later decisions).  So:
 //   1. gc_adjacency_kernel evaluates the pairwise test once for all pairs into a C x C bitmap
 //      (all SMs; this is the O(C^2) part).
-//   2. gc_group_kernel (one CTA, 16 warps) takes the next 16 untaken seeds, one per warp; a warp
-//      intersects its seed's bitmap row with ~taken, lists the candidates in ascending order and grows
-//      the set with warp ballots (candidates' points in registers).  Warp 0 then walks the 16 results
-//      in order: the first seed whose set touches an element committed earlier in the walk is
-//      inexact, everything before it commits, and the next window restarts there.  On the benchmark
-//      scene (25 k correspondences, 3 770 instances) that is ~530 rounds of a few microseconds instead
-//      of 4 276 sequential seed scans.
-// RANSAC runs afterwards, one warp per instance: lane 0 draws the sample sequence (the RNG stream is
-// inherently serial), the lanes fit and score one sample each, lane 0 then replays the adaptive
-// termination logic in order and discards the samples past the stopping point.
+//   2. gc_group_cluster_kernel (one 8-CTA thread-block cluster) takes the next 8 untaken seeds, one per
+//      CTA, and grows each set speculatively against the current flags: candidates = row(seed) & ~taken,
+//      the lowest candidate is admitted and its row ANDed in, and the last 64 or fewer candidates are
+//      finished in registers.  Every CTA then walks the 8 results in the same order: the first seed whose
+//      set touches an element committed earlier in the walk is inexact, everything before it commits,
+//      and the next window restarts there.  On the benchmark scene (25 k correspondences, 3 770
+//      instances) that is 678 rounds instead of 4 276 sequential seed scans.
+// RANSAC runs afterwards, one CTA per instance in two size classes (32 threads up to 96 members, 128
+// threads above): thread 0 draws the sample sequence (the RNG stream is inherently serial), the threads
+// fit and score one sample each, thread 0 then replays the adaptive termination logic in order and
+// discards the samples past the stopping point.
 #include <stdlib.h>
 #include <string.h>
 
@@ -321,22 +322,32 @@ __global__ void __launch_bounds__(ADJ_THREADS)
   }
 }
 
-// ---- greedy grouping: one CTA, up to GW seeds evaluated speculatively per round -------------------
-constexpr int GW = 16;                 // seeds (one per warp) per round
-constexpr int GG_THREADS = GW * 32;
-constexpr int G_MC = 64;               // member indices kept in shared memory per seed
-constexpr int G_HS = 4096;             // commit hash table slots (>= 4 x GW x G_MC)
-constexpr int G_LIST = 64;             // candidates finished in registers
+// ---- greedy grouping on a thread-block cluster ----------------------------------------------------
+// The whole greedy growth of a seed runs on bitmaps: candidates = row(seed) & ~taken; the lowest
+// candidate j is admitted (it fits every member so far by construction) and candidates &= row(j);
+// repeat until at most G_LIST candidates are left, which are listed in ascending position and
+// finished in registers.  Rows are padded to a multiple of 128 words.
+// A round evaluates the next GCL untaken seeds speculatively, one per CTA of the cluster: CTA r
+// evaluates window seed r with all of its 128 threads (thread t handles the 16-byte pieces t,
+// t + 128, ... of a bitmap row).  Every CTA keeps its own copy of the `taken` bitmap and of the
+// running totals; after the evaluation each CTA writes its result (size + members) into every CTA's
+// shared memory through DSMEM, one cluster barrier later all CTAs walk the window identically, so the
+// copies never diverge and one barrier per round suffices (results are double-buffered by round parity).
+constexpr int GCL = 8;            // cluster size = seeds per round
+constexpr int GCL_THREADS = 128;
+constexpr int G_MC = 64;          // member indices kept in shared memory per seed
+constexpr int G_LIST = 64;        // candidates finished in registers
 
 struct GroupArgs {
   const unsigned *adj;
   const float4 *mp;
   const float4 *sp;
-  int *overflow;      // [GW][C_cap] member indices past G_MC
+  int *overflow;      // [GCL][C_cap] member indices past G_MC
   int *members;       // [C_cap] committed member lists, concatenated
   int *inst_offsets;  // [max_inst + 1]
   int *n_inst_out;
-  long long *dbg;     // nullable (B200_GC_TIMING builds): per warp [rounds, window, eval, commit] cycles
+  long long *dbg;     // nullable (B200_GC_TIMING builds): per CTA [window, first row, admissions, list,
+                      // list + greedy, cluster sync, commit] cycles and the round count
 };
 
 __device__ __forceinline__ int warp_incl_scan(int v, int lane) {
@@ -348,8 +359,6 @@ __device__ __forceinline__ int warp_incl_scan(int v, int lane) {
   return v;
 }
 
-__device__ __forceinline__ unsigned gc_hash(int m) { return ((unsigned)m * 2654435761u) >> 20; }  // 12 bits
-
 // lowest set position of a 128-bit group that starts at position base, or INT_MAX
 __device__ __forceinline__ int first_bit128(const uint4 &w, int base) {
   if (w.x) return base + __ffs(w.x) - 1;
@@ -358,373 +367,6 @@ __device__ __forceinline__ int first_bit128(const uint4 &w, int base) {
   if (w.w) return base + 96 + __ffs(w.w) - 1;
   return 0x7fffffff;
 }
-
-// The whole greedy growth of a seed runs on bitmaps: candidates = row(seed) & ~taken; the lowest
-// candidate j is admitted (it fits every member so far by construction) and candidates &= row(j);
-// repeat until no candidate is left.  A warp owns one seed; lane l handles the 16-byte groups
-// l, l + 32, ... of the row (coalesced), the candidate bitmap lives in shared memory, the next
-// admission is a warp-wide integer min.  Rows are padded to a multiple of 128 words (32 groups).
-__global__ void __launch_bounds__(GG_THREADS, 1)
-    gc_group_kernel(GroupArgs ga, const int *__restrict__ d_C, int C_cap, int dyn_smem_bytes, double gc_size, float g_lo,
-                    float g_hi, int gc_threshold, int max_inst, const int *__restrict__ gate) {
-  extern __shared__ __align__(16) unsigned char s_raw[];
-  if (gate && *gate == 0) return;  // the stream kernel has done the scene
-  __shared__ int s_seed[GW], s_size[GW], s_conf[GW];
-  __shared__ int s_nwin, s_big;
-  __shared__ int s_hkey[G_HS], s_hval[G_HS];
-  __shared__ int s_mem[GW][G_MC];
-  __shared__ int s_list[GW][64];
-  __shared__ float4 s_newm[GW], s_news[GW];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int C = min(*d_C, C_cap);
-  const int row_words = gc_row_words(C);
-  const int nq = row_words >> 7;  // 16-byte groups per lane
-  // seeds per round: as many candidate bitmaps as fit beside the taken bitmap (the launch sized the
-  // dynamic shared memory for the capacity; the actual count is usually much smaller)
-  const int gw = min(GW, dyn_smem_bytes / (row_words * 4) - 1);
-  // dynamic shared memory: taken bitmap | one candidate bitmap per evaluating warp
-  uint4 *s_taken4 = reinterpret_cast<uint4 *>(s_raw);                            // [row_words / 4]
-  unsigned *s_taken = reinterpret_cast<unsigned *>(s_raw);
-  uint4 *my_cb4 = s_taken4 + (size_t)(row_words >> 2) * (1 + warp);              // [row_words / 4], warp < gw
-
-  for (int w = tid; w < row_words; w += GG_THREADS) {
-    const int j0 = w * 32;
-    s_taken[w] = (j0 + 32 <= C) ? 0u : ((j0 >= C) ? ~0u : ~((1u << (C - j0)) - 1u));  // padding counts as taken
-  }
-  for (int h = tid; h < G_HS; h += GG_THREADS) {
-    s_hkey[h] = -1;
-    s_hval[h] = 0x7fffffff;
-  }
-  if (tid == 0) ga.inst_offsets[0] = 0;
-  // replicated in every thread (all threads derive the same values from shared memory each round)
-  int cur = 0, n_inst = 0, total = 0;
-  __syncthreads();
-
-  int *my_mem = s_mem[warp];
-  int *my_over = ga.overflow + (size_t)warp * C_cap;
-
-#ifdef B200_GC_TIMING
-  long long t_win = 0, t_eval = 0, t_commit = 0, n_rounds = 0, t_wait = 0;
-#define GC_CLOCK(v) const long long v = clock64()
-#define GC_ACC(acc, expr) acc += (expr)
-#else
-#define GC_CLOCK(v)
-#define GC_ACC(acc, expr)
-#endif
-  while (true) {
-    GC_CLOCK(c0);
-    // ---- window: the next gw untaken positions at or after cur (warp 0) ----
-    if (warp == 0) {
-      int n = 0;
-      for (int wb = cur >> 5; wb < row_words && n < gw; wb += 32) {
-        const int wi = wb + lane;
-        unsigned bits = (wi < row_words) ? ~s_taken[wi] : 0u;
-        if (wi == (cur >> 5)) bits &= ~((1u << (cur & 31)) - 1u);
-        const int cnt = __popc(bits);
-        const int incl = warp_incl_scan(cnt, lane);
-        int o = n + incl - cnt;
-        while (bits && o < gw) {
-          const int b = __ffs(bits) - 1;
-          bits &= bits - 1;
-          s_seed[o++] = wi * 32 + b;
-        }
-        n += __shfl_sync(0xffffffffu, incl, 31);
-      }
-      if (lane == 0) {
-        s_nwin = min(n, gw);
-        s_big = 0;
-      }
-    }
-    __syncthreads();
-    const int nwin = s_nwin;
-    if (nwin == 0) break;
-    GC_CLOCK(c1);
-    GC_ACC(t_win, c1 - c0);
-    GC_ACC(n_rounds, 1);
-
-    // ---- evaluate: warp w grows the consensus set of seed w against the current flags ----
-    if (warp < nwin) {
-      const int seed = s_seed[warp];
-      int size = 1;
-      if (lane == 0) my_mem[0] = seed;
-      int first = 0x7fffffff, my_cnt = 0;
-      {
-        const uint4 *row4 = reinterpret_cast<const uint4 *>(ga.adj + (size_t)seed * row_words);
-        for (int q0 = 0; q0 < nq; q0 += 8) {  // all loads of a block are issued before the first use
-          uint4 x[8];
-#pragma unroll
-          for (int i = 0; i < 8; ++i)
-            if (q0 + i < nq) x[i] = __ldg(row4 + (q0 + i) * 32 + lane);
-#pragma unroll
-          for (int i = 0; i < 8; ++i)
-            if (q0 + i < nq) {
-              const int g = (q0 + i) * 32 + lane;
-              const uint4 t = s_taken4[g];
-              const uint4 w = make_uint4(x[i].x & ~t.x, x[i].y & ~t.y, x[i].z & ~t.z, x[i].w & ~t.w);
-              my_cb4[g] = w;
-              my_cnt += __popc(w.x) + __popc(w.y) + __popc(w.z) + __popc(w.w);
-              if (first == 0x7fffffff) first = first_bit128(w, g * 128);
-            }
-        }
-      }
-      first = __reduce_min_sync(0xffffffffu, first);
-      int n_cand = __reduce_add_sync(0xffffffffu, my_cnt);
-      // bitmap admissions while many candidates remain (each costs one row read)
-      while (n_cand > 64) {
-        const int j = first;
-        if (lane == 0) {
-          if (size < G_MC)
-            my_mem[size] = j;
-          else
-            my_over[size] = j;
-        }
-        ++size;
-        const uint4 *rowj4 = reinterpret_cast<const uint4 *>(ga.adj + (size_t)j * row_words);
-        first = 0x7fffffff;
-        my_cnt = 0;
-        for (int q0 = j >> 12; q0 < nq; q0 += 8) {  // groups before j's hold no candidates any more
-          uint4 y[8];
-#pragma unroll
-          for (int i = 0; i < 8; ++i)
-            if (q0 + i < nq) y[i] = __ldg(rowj4 + (q0 + i) * 32 + lane);
-#pragma unroll
-          for (int i = 0; i < 8; ++i)
-            if (q0 + i < nq) {
-              const int g = (q0 + i) * 32 + lane;
-              uint4 w = my_cb4[g];
-              w.x &= y[i].x, w.y &= y[i].y, w.z &= y[i].z, w.w &= y[i].w;
-              my_cb4[g] = w;
-              my_cnt += __popc(w.x) + __popc(w.y) + __popc(w.z) + __popc(w.w);
-              if (first == 0x7fffffff) first = first_bit128(w, g * 128);
-            }
-        }
-        first = __reduce_min_sync(0xffffffffu, first);
-        n_cand = __reduce_add_sync(0xffffffffu, my_cnt);
-      }
-      if (n_cand > 0) {
-        // at most 64 candidates left: list them in ascending position (each lane expands a contiguous
-        // slice of the shared-memory bitmap), fetch their points once and finish the greedy growth in
-        // registers — no further memory round trips
-        __syncwarp();
-        const unsigned *cb = reinterpret_cast<const unsigned *>(my_cb4);
-        const int wpl = row_words >> 5, w_lo = lane * wpl;
-        const int w_min = first >> 5;  // nothing before the first candidate
-        int cnt = 0;
-        for (int w = max(w_lo, w_min); w < w_lo + wpl; ++w) cnt += __popc(cb[w]);
-        const int incl = warp_incl_scan(cnt, lane);
-        if (cnt) {
-          int o = incl - cnt;
-          for (int w = max(w_lo, w_min); w < w_lo + wpl; ++w) {
-            unsigned bits = cb[w];
-            while (bits) {
-              s_list[warp][o++] = w * 32 + __ffs(bits) - 1;
-              bits &= bits - 1;
-            }
-          }
-        }
-        __syncwarp();
-        int j[2];
-        float4 mj[2], sj[2];
-        unsigned alive = 0;
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-          const int idx = u * 32 + lane;
-          if (idx < n_cand) {
-            j[u] = s_list[warp][idx];
-            mj[u] = ga.mp[j[u]];
-            sj[u] = ga.sp[j[u]];
-            alive |= 1u << u;
-          }
-        }
-        while (true) {
-          unsigned bal = __ballot_sync(0xffffffffu, alive & 1u);
-          int usel = 0;
-          if (!bal) {
-            bal = __ballot_sync(0xffffffffu, alive & 2u);
-            usel = 1;
-            if (!bal) break;
-          }
-          const int owner = __ffs(bal) - 1;
-          if (lane == owner) {
-            const int jj = usel ? j[1] : j[0];
-            s_newm[warp] = usel ? mj[1] : mj[0];
-            s_news[warp] = usel ? sj[1] : sj[0];
-            if (size < G_MC)
-              my_mem[size] = jj;
-            else
-              my_over[size] = jj;
-            alive &= ~(1u << usel);
-          }
-          __syncwarp();
-          const float4 mk = s_newm[warp], sk = s_news[warp];
-          ++size;
-#pragma unroll
-          for (int u = 0; u < 2; ++u)
-            if (((alive >> u) & 1u) && !gc_fits(mk, sk, mj[u], sj[u], g_lo, g_hi, gc_size)) alive &= ~(1u << u);
-          __syncwarp();
-        }
-      }
-      if (lane == 0) {
-        s_size[warp] = size;
-        if (size > G_MC) s_big = 1;
-      }
-      __syncwarp();
-      // successful seeds publish their members: hash slot value = lowest window position holding it
-      if (size > gc_threshold && size <= G_MC) {
-        for (int kk = lane; kk < size; kk += 32) {
-          const int m = my_mem[kk];
-          unsigned h = gc_hash(m);
-          while (true) {
-            const int old = atomicCAS(&s_hkey[h], -1, m);
-            if (old == -1 || old == m) {
-              atomicMin(&s_hval[h], warp);
-              break;
-            }
-            h = (h + 1) & (G_HS - 1);
-          }
-        }
-      }
-    }
-    GC_CLOCK(c2);
-    GC_ACC(t_eval, c2 - c1);
-    __threadfence_block();
-    __syncthreads();
-    GC_CLOCK(c3);
-    GC_ACC(t_wait, c3 - c2);
-
-    // ---- commit: walk the window in order; a seed whose set touches an element claimed by an earlier
-    // successful seed of this window is the first inexact one: everything before it is what the
-    // sequential algorithm computes, the next window restarts there ----
-    const bool slow = s_big != 0;
-    int pstar = nwin;
-    int my_off = -1, my_inst = 0;
-    if (!slow) {
-      if (warp < nwin) {
-        const int size = s_size[warp];
-        bool hit = false;
-        for (int kk = lane; kk < size; kk += 32) {
-          const int m = my_mem[kk];
-          unsigned h = gc_hash(m);
-          while (true) {
-            const int key = s_hkey[h];
-            if (key == -1) break;
-            if (key == m) {
-              hit = s_hval[h] < warp;
-              break;
-            }
-            h = (h + 1) & (G_HS - 1);
-          }
-          if (hit) break;
-        }
-        const bool conflict = __any_sync(0xffffffffu, hit);
-        if (lane == 0) s_conf[warp] = conflict ? 1 : 0;
-      }
-      __syncthreads();
-      // every thread resolves the window identically
-      int run_total = total, run_inst = n_inst;
-      for (int r = 0; r < nwin; ++r) {
-        if (s_conf[r]) {
-          pstar = r;
-          break;
-        }
-        const int sz = s_size[r];
-        if (sz > gc_threshold) {
-          if (r == warp) {
-            my_off = run_total;
-            my_inst = run_inst;
-          }
-          run_total += sz;
-          ++run_inst;
-        }
-      }
-      total = run_total;
-      n_inst = run_inst;
-      cur = (pstar < nwin) ? s_seed[pstar] : s_seed[nwin - 1] + 1;
-      if (warp < nwin && my_off >= 0) {
-        const int sz = s_size[warp];
-        for (int kk = lane; kk < sz; kk += 32) {
-          const int m = my_mem[kk];
-          atomicOr(&s_taken[m >> 5], 1u << (m & 31));
-          ga.members[my_off + kk] = m;
-        }
-        if (lane == 0 && my_inst < max_inst) ga.inst_offsets[my_inst + 1] = my_off + sz;
-      }
-      __syncthreads();  // all probes done before the table is cleared
-      for (int h = tid; h < G_HS; h += GG_THREADS) {
-        s_hkey[h] = -1;
-        s_hval[h] = 0x7fffffff;
-      }
-    } else {
-      // a set larger than the shared-memory member list: sequential walk by warp 0
-      __shared__ int s_res[4];
-      if (warp == 0) {
-        int run_total = total, run_inst = n_inst;
-        for (int r = 0; r < nwin; ++r) {
-          const int sz = s_size[r];
-          bool conflict = false;
-          for (int k0 = 0; k0 < sz; k0 += 32) {
-            const int kk = k0 + lane;
-            int m = -1;
-            if (kk < sz) m = (kk < G_MC) ? s_mem[r][kk] : __ldcg(ga.overflow + (size_t)r * C_cap + kk);
-            const bool hit = m >= 0 && ((s_taken[m >> 5] >> (m & 31)) & 1u);
-            if (__any_sync(0xffffffffu, hit)) conflict = true;
-          }
-          if (conflict) {
-            pstar = r;
-            break;
-          }
-          if (sz > gc_threshold) {
-            for (int k0 = 0; k0 < sz; k0 += 32) {
-              const int kk = k0 + lane;
-              if (kk < sz) {
-                const int m = (kk < G_MC) ? s_mem[r][kk] : __ldcg(ga.overflow + (size_t)r * C_cap + kk);
-                atomicOr(&s_taken[m >> 5], 1u << (m & 31));
-                ga.members[run_total + kk] = m;
-              }
-            }
-            if (lane == 0 && run_inst < max_inst) ga.inst_offsets[run_inst + 1] = run_total + sz;
-            run_total += sz;
-            ++run_inst;
-          }
-          __syncwarp();
-        }
-        if (lane == 0) {
-          s_res[0] = run_total;
-          s_res[1] = run_inst;
-          s_res[2] = (pstar < nwin) ? s_seed[pstar] : s_seed[nwin - 1] + 1;
-        }
-      }
-      __syncthreads();
-      total = s_res[0];
-      n_inst = s_res[1];
-      cur = s_res[2];
-      for (int h = tid; h < G_HS; h += GG_THREADS) {
-        s_hkey[h] = -1;
-        s_hval[h] = 0x7fffffff;
-      }
-    }
-    __syncthreads();
-    GC_ACC(t_commit, clock64() - c3);
-  }
-  if (tid == 0) *ga.n_inst_out = n_inst;
-#ifdef B200_GC_TIMING
-  if (ga.dbg && lane == 0) {
-    long long *d = ga.dbg + warp * 8;
-    d[0] = n_rounds, d[1] = t_win, d[2] = t_eval, d[3] = t_commit, d[4] = t_wait;
-  }
-#endif
-}
-
-// ---- greedy grouping on a thread-block cluster ----------------------------------------------------
-// Same algorithm as gc_group_kernel, spread over the SMs of one cluster: CTA r of the cluster
-// evaluates window seed r with all of its 128 threads (thread t handles the 16-byte pieces t,
-// t + 128, ... of a bitmap row), so a round's evaluations no longer share one SM's issue slots.
-// Every CTA keeps its own copy of the `taken` bitmap and of the running totals; after the
-// evaluation each CTA writes its result (size + members) into every CTA's shared memory through
-// DSMEM, one cluster barrier later all CTAs walk the window identically, so the copies never
-// diverge and one barrier per round suffices (results are double-buffered by round parity).
-constexpr int GCL = 8;            // cluster size = seeds per round
-constexpr int GCL_THREADS = 128;
 
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
@@ -746,9 +388,8 @@ __device__ __forceinline__ void dsmem_store(unsigned addr, int v) {
 
 __global__ void __cluster_dims__(GCL, 1, 1) __launch_bounds__(GCL_THREADS, 1)
     gc_group_cluster_kernel(GroupArgs ga, const int *__restrict__ d_C, int C_cap, double gc_size, float g_lo, float g_hi,
-                            int gc_threshold, int max_inst, const int *__restrict__ gate) {
+                            int gc_threshold, int max_inst) {
   extern __shared__ __align__(16) unsigned char s_raw[];
-  if (gate && *gate == 0) return;  // the stream kernel has done the scene (uniform over the cluster)
   __shared__ int s_res[2][GCL][1 + G_MC];  // published results by round parity: [0] size, then members
   __shared__ int s_seed[GCL];
   __shared__ int s_nwin;
@@ -1053,637 +694,6 @@ __global__ void __cluster_dims__(GCL, 1, 1) __launch_bounds__(GCL_THREADS, 1)
     for (int i = 0; i < 8; ++i) ga.dbg[rank * 8 + i] = tc_[i];
 #endif
   if (rank == 0 && tid == 0) *ga.n_inst_out = n_inst;
-}
-
-// ---- greedy grouping as a stream on one SM (experimental: B200_GC_GROUP=stream) --------------------
-// The round-based kernels above pay, per round of eight seeds, two or three dependent trips to the bitmap rows
-// plus a cluster barrier: 7.8 us per round, 678 rounds on the target scene.  Here nothing that touches global
-// memory is on the sequential chain.  One CTA, three kinds of warps:
-//   * the dispatcher (warp 0) walks the `taken` flags and hands the next position that is not taken yet to the
-//     next production ticket, at most GS_NSLOT tickets ahead of the last commit;
-//   * producer warps stage a seed each: the seed's bitmap row is read once (lane l owns a contiguous 1/32 of the
-//     row, so the candidates a lane finds are consecutive in the ascending list and one warp scan places them),
-//     what is taken already is dropped, the list and the candidates' model / scene points go into a ring buffer in
-//     shared memory (32-candidate blocks: index + 6 coordinates, one 128-byte line per field); with the points the
-//     producer reads each candidate's bit of the FIRST candidate's bitmap row (bit 31 of its index): the first
-//     admission's tests — three quarters of all pair tests of a seed — come off the bitmap instead of being
-//     recomputed.  Ring space is handed out in ticket order, so the chunk of the seed the consumers wait for is
-//     always allocated before any later one and the ring cannot deadlock;
-//   * consumer warps take the staged seeds round-robin.  A consumer filters the list against the live `taken` flags
-//     and grows the consensus set in the points domain entirely out of shared memory (lowest live candidate by
-//     redux.min, its points broadcast, every lane tests the candidates it owns: PCL's loop over j, in j order),
-//     then waits for its turn to commit.  At its turn every earlier seed has committed: if the seed was taken in the
-//     meantime it is dropped; if one of the set's members was taken the growth is repeated (from shared memory, no
-//     load); otherwise the set is exactly what the sequential algorithm computes (a set grown against older flags
-//     stays exact as long as none of its members has been taken since).  Inside the turn only the flags and the
-//     running totals are updated; the member list goes to global memory after the turn has been passed on.
-// Hand-overs are mbarriers (count 1, one phase per use of a slot).  A seed with more than GS_LCAP live candidates,
-// or a scene with more than 32 768 correspondences, or a hand-over that a watchdog finds stuck, sends the scene to
-// the round-based kernel instead (flag on the device, no host round trip).
-// MEASURED (target scene: 5 578 tickets for 4 276 seeds, 183 candidates per seed on average, 1 285 at most, 5.9
-// members per set, 4 % of the sets grown twice): byte-identical, but 8.3 ms against the cluster kernel's 5.5 ms, so
-// the cluster kernel stays the default.  Why, with numbers: profiles/summary_r02.md (polling warps took 58 % of the
-// issue slots and saturated the XU pipe with S2R; a suspend-time hint wakes 2 us late; after both were fixed the
-// commit turn — 1 900 cycles of dependent shared-memory operations in one warp — and the 47 KB of code shared by 24
-// warps in different phases bound the kernel).
-constexpr int GS_PROD = 15;
-constexpr int GS_CONS = 8;
-constexpr int GS_THREADS = (1 + GS_PROD + GS_CONS) * 32;
-constexpr int GS_NSLOT = 32;            // seeds staged or being staged (> GS_PROD)
-constexpr int GS_LCAP = 2048;           // candidates per seed: 64 per lane, one 64-bit mask
-constexpr int GS_MAXQ = 8;              // 16-byte row pieces per lane: rows of up to 32 768 positions
-constexpr int GS_BLK = 7 * 128;         // bytes of a 32-candidate block
-constexpr int GS_NBLK = 224;            // ring blocks (196 KB)
-constexpr int GS_MAX_ROW_WORDS = GS_MAXQ * 128;
-
-struct StreamState {
-  unsigned long long bar_disp[GS_NSLOT];    // ticket t has its position
-  unsigned long long bar_alloc[GS_NSLOT];   // ticket t may take ring space
-  unsigned long long bar_ready[GS_NSLOT];   // slot staged
-  unsigned long long bar_commit[GS_NSLOT];  // ticket u may commit
-  unsigned long long bar_free[GS_NSLOT];    // slot's previous ticket committed
-  int seed[GS_NSLOT], n[GS_NSLOT], blk[GS_NSLOT], vend[GS_NSLOT];
-  int issue;             // next production ticket
-  int alloc_done;        // tickets that have their ring space
-  int commit_done;       // tickets committed
-  int ring_head;         // virtual block counters: [ring_tail, ring_head) is in use
-  int ring_tail;
-  int take;              // next consumer ticket
-  int end_ticket;        // first ticket past the last position
-  int abort;
-  int total, n_inst;
-};
-
-__device__ __forceinline__ int ld_vol(const int *p) { return *reinterpret_cast<const volatile int *>(p); }
-__device__ __forceinline__ void st_vol(int *p, int v) { *reinterpret_cast<volatile int *>(p) = v; }
-__device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(unsigned bar) {
-  asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}" ::"r"(bar) : "memory");
-}
-// true once the phase with this parity has completed; the hardware parks the warp for a short, system-defined time
-// (about 0.1 us on B200) before it answers "not yet"
-__device__ __forceinline__ bool mbar_try_wait(unsigned bar, unsigned parity) {
-  unsigned ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-
-// A hand-over that takes longer than about two seconds cannot be a healthy pipeline: the kernel then raises
-// `abort`, records where it was (fallback[1..]) and the round-based kernel does the scene.
-__device__ __noinline__ void gs_give_up(StreamState &S, int *fallback, int code, int ticket) {
-  if (atomicCAS(&S.abort, 0, 1) == 0) {
-    fallback[1] = code;
-    fallback[2] = ticket;
-    fallback[3] = ld_vol(&S.issue), fallback[4] = ld_vol(&S.commit_done);
-    fallback[5] = ld_vol(&S.ring_head), fallback[6] = ld_vol(&S.ring_tail);
-    fallback[7] = ld_vol(&S.end_ticket);
-    __threadfence();
-    fallback[0] = 1;
-  }
-}
-// The wait loop is two instructions (try_wait, branch); abort flag and watchdog are looked at every 1024 tries.
-// sleep_ns > 0: for waits nobody downstream is waiting on (the pipeline is several tickets deep there) the warp
-// sleeps between two looks, so that the shared-memory pipe is left to the warps that work.
-// (A suspend-time hint of 20 us parks the warp properly but wakes it about 2 us after the arrival.  A loop that
-// also read the clock and the abort flag each time took 58 % of the SM's issue slots and saturated the XU pipe with
-// its S2R.  The kernel's code must stay small: 24 warps in different phases share a 32 KB instruction cache.)
-__device__ __noinline__ void gs_wait(StreamState &S, int *fallback, unsigned bar, unsigned parity, unsigned sleep_ns, int code,
-                                     int ticket) {
-  if (mbar_try_wait(bar, parity)) return;
-  long long t0 = 0;
-  unsigned tries = 0;
-  while (!mbar_try_wait(bar, parity)) {
-    if (sleep_ns) __nanosleep(sleep_ns);
-    if ((++tries & 1023u) == 0) {
-      if (ld_vol(&S.abort)) return;
-      if (t0 == 0)
-        t0 = clock64();
-      else if (clock64() - t0 > 4000000000ll) {
-        gs_give_up(S, fallback, code, ticket);
-        return;
-      }
-    }
-  }
-}
-#define GS_GIVE_UP(code, ticket) gs_give_up(S, fallback, (code), (ticket))
-#define GS_WAIT(bar, parity, code, ticket) gs_wait(S, fallback, (bar), (parity), 0u, (code), (ticket))
-#define GS_WAIT_COARSE(bar, parity, ns, code, ticket) gs_wait(S, fallback, (bar), (parity), (ns), (code), (ticket))
-
-// A consumer's result: the admitted candidates as a mask over the chunk's blocks (bit k of lane l = list position
-// 32 k + l; 64 blocks = two words), the set size (seed included), and whether the seed was found taken.
-struct StreamEval {
-  unsigned mlo, mhi;
-  int size;
-  bool skip;
-};
-
-__device__ __forceinline__ bool gs_taken(const unsigned *s_taken, int j) {
-  return ((ld_vol(reinterpret_cast<const int *>(s_taken) + (j >> 5)) >> (j & 31)) & 1) != 0;
-}
-
-// Growth of one seed's set by one warp from its staged chunk.  Candidate at list position q lives in block q >> 5,
-// lane q & 31; lane l owns the positions congruent to l.
-__device__ __forceinline__ StreamEval stream_grow(const unsigned *s_taken, const unsigned char *chunk, int seed, int n, int lane,
-                                               float g_lo, float g_hi, double gc_size) {
-  StreamEval r;
-  r.mlo = r.mhi = 0u;
-  r.size = 1;
-  // one answer for the warp: the flag may flip (another consumer's commit) between two lanes' reads
-  r.skip = __any_sync(0xffffffffu, gs_taken(s_taken, seed));
-  if (r.skip) return r;
-  unsigned alo = 0u, ahi = 0u, flo = 0u, fhi = 0u;
-  const int nb = (n + 31) >> 5;
-  for (int k = 0; k < nb; ++k) {
-    if (k * 32 + lane < n) {
-      const unsigned w = *reinterpret_cast<const unsigned *>(chunk + k * GS_BLK + lane * 4);
-      const unsigned bit = 1u << (k & 31);
-      const bool live = !gs_taken(s_taken, (int)(w & 0x7fffffffu));
-      if (k < 32) {
-        if (live) alo |= bit;
-        if (w >> 31) flo |= bit;
-      } else {
-        if (live) ahi |= bit;
-        if (w >> 31) fhi |= bit;
-      }
-    }
-  }
-  bool first = true;
-  while (true) {
-    const int mine = alo ? (((__ffs((int)alo) - 1) << 5) | lane) : (ahi ? (((__ffs((int)ahi) + 31) << 5) | lane) : 0x7fffffff);
-    const int c = __reduce_min_sync(0xffffffffu, mine);
-    if (c == 0x7fffffff) break;
-    const int ck = c >> 5, cl = c & 31;
-    if (lane == cl) {
-      if (ck < 32) {
-        r.mlo |= 1u << ck;
-        alo &= ~(1u << ck);
-      } else {
-        r.mhi |= 1u << (ck - 32);
-        ahi &= ~(1u << (ck - 32));
-      }
-    }
-    ++r.size;
-    if (first && c == 0) {  // the list's first candidate: its tests were read off the bitmap by the producer
-      alo &= flo;
-      ahi &= fhi;
-      first = false;
-      continue;
-    }
-    first = false;
-    const float *cb = reinterpret_cast<const float *>(chunk + ck * GS_BLK) + cl;
-    const float4 mk = make_float4(cb[32], cb[64], cb[96], 0.f);
-    const float4 sk = make_float4(cb[128], cb[160], cb[192], 0.f);
-#pragma unroll 1
-    for (int h = 0; h < 2; ++h) {
-      unsigned a = h ? ahi : alo, keep = a;
-      const unsigned char *hb = chunk + h * 32 * GS_BLK;
-      while (a) {
-        const int kk = __ffs((int)a) - 1;
-        a &= a - 1;
-        const float *pb = reinterpret_cast<const float *>(hb + kk * GS_BLK) + lane;
-        const float4 mj = make_float4(pb[32], pb[64], pb[96], 0.f);
-        const float4 sj = make_float4(pb[128], pb[160], pb[192], 0.f);
-        if (!gc_fits(mk, sk, mj, sj, g_lo, g_hi, gc_size)) keep &= ~(1u << kk);
-      }
-      if (h)
-        ahi = keep;
-      else
-        alo = keep;
-      if (nb <= 32) break;
-    }
-  }
-  return r;
-}
-
-// Writes the positions of the set bits of one 64-bit piece of a candidate row (first position `base`) into the
-// chunk's index list from list position o on; returns the next list position.
-__device__ __forceinline__ int stream_list_piece(unsigned long long v, int base, unsigned char *chunk, int o) {
-  while (v) {
-    const int b = __ffsll((long long)v) - 1;
-    v &= v - 1;
-    *reinterpret_cast<unsigned *>(chunk + (o >> 5) * GS_BLK + (o & 31) * 4) = (unsigned)(base + b);
-    ++o;
-  }
-  return o;
-}
-
-struct StreamCommit {
-  unsigned *s_taken;
-  StreamState *S;
-  int *members;
-  int *inst_offsets;
-  int gc_threshold, max_inst;
-  float g_lo, g_hi;
-  double gc_size;
-  long long *tq;  // timing builds
-};
-
-// The in-order part of a consumer's work (it holds the commit turn) and the write-out behind it.
-// Returns after the turn has been passed on and the slot released.
-__device__ __forceinline__ void stream_commit(const StreamCommit &cc, StreamEval ev, const unsigned char *chunk, int seed, int n,
-                                           int lane, unsigned bar_next_commit, int ticket, unsigned bar_free, int vend) {
-  StreamState &S = *cc.S;
-#ifdef B200_GC_TIMING
-  long long c_a = clock64();
-#endif
-  // members into registers (two per lane; a lane with more makes the set a `wide` one)
-  int j0 = -1, j1 = -1, k0 = 0, k1 = 0;
-  bool wide = false;
-  if (!ev.skip) {
-    bool bad = gs_taken(cc.s_taken, seed);
-    for (int pass = 0; pass < 2; ++pass) {
-      j0 = j1 = -1;
-      wide = false;
-      int cnt = 0;
-#pragma unroll 1
-      for (int h = 0; h < 2; ++h) {
-        unsigned a = h ? ev.mhi : ev.mlo;
-        while (a) {
-          const int kk = __ffs((int)a) - 1 + h * 32;
-          a &= a - 1;
-          const int j = (int)(*reinterpret_cast<const unsigned *>(chunk + kk * GS_BLK + lane * 4) & 0x7fffffffu);
-          bad = bad || gs_taken(cc.s_taken, j);
-          if (cnt == 0)
-            j0 = j, k0 = kk;
-          else if (cnt == 1)
-            j1 = j, k1 = kk;
-          else
-            wide = true;
-          ++cnt;
-        }
-      }
-      if (pass == 1 || !__any_sync(0xffffffffu, bad)) break;
-      if (__any_sync(0xffffffffu, gs_taken(cc.s_taken, seed))) {  // the seed itself went
-        ev.skip = true;
-        break;
-      }
-      ev = stream_grow(cc.s_taken, chunk, seed, n, lane, cc.g_lo, cc.g_hi, cc.gc_size);  // exact now: nothing is in flight before us
-#ifdef B200_GC_TIMING
-      cc.tq[6] += 1;
-#endif
-      bad = false;
-    }
-  }
-#ifdef B200_GC_TIMING
-  {
-    const long long c_b = clock64();
-    cc.tq[4] += c_b - c_a;
-    c_a = c_b;
-  }
-#endif
-  const bool emit = !ev.skip && ev.size > cc.gc_threshold;
-  wide = __any_sync(0xffffffffu, wide);
-  int total = 0, ninst = 0;
-  const unsigned lt_mask = (1u << lane) - 1u;
-  if (emit) {
-    if (lane == 0) {
-      total = ld_vol(&S.total), ninst = ld_vol(&S.n_inst);
-      st_vol(&S.total, total + ev.size);
-      st_vol(&S.n_inst, ninst + 1);
-      atomicOr(&cc.s_taken[seed >> 5], 1u << (seed & 31));
-    }
-    if (!wide) {
-      if (j0 >= 0) atomicOr(&cc.s_taken[j0 >> 5], 1u << (j0 & 31));
-      if (j1 >= 0) atomicOr(&cc.s_taken[j1 >> 5], 1u << (j1 & 31));
-    } else {
-      // a set with more than two members in some lane: flags and member list straight from the chunk, inside the turn
-      total = __shfl_sync(0xffffffffu, total, 0);
-      int run = 1;
-#pragma unroll 1
-      for (int h = 0; h < 2; ++h) {
-        const unsigned mine = h ? ev.mhi : ev.mlo;
-        unsigned any = __reduce_or_sync(0xffffffffu, mine);
-        while (any) {
-          const int kb = __ffs((int)any) - 1;
-          any &= any - 1;
-          const bool in = (mine >> kb) & 1u;
-          const unsigned bal = __ballot_sync(0xffffffffu, in);
-          if (in) {
-            const int j = (int)(*reinterpret_cast<const unsigned *>(chunk + (kb + h * 32) * GS_BLK + lane * 4) & 0x7fffffffu);
-            cc.members[total + run + __popc(bal & lt_mask)] = j;
-            atomicOr(&cc.s_taken[j >> 5], 1u << (j & 31));
-          }
-          run += __popc(bal);
-        }
-      }
-    }
-  }
-  __syncwarp();
-  if (lane == 0) {
-    st_vol(&S.ring_tail, vend);
-    st_vol(&S.commit_done, ticket + 1);
-    mbar_arrive(bar_next_commit);  // the next ticket's turn
-    mbar_arrive(bar_free);         // the slot may be staged again
-  }
-#ifdef B200_GC_TIMING
-  {
-    const long long c_b = clock64();
-    cc.tq[5] += c_b - c_a;
-    c_a = c_b;
-  }
-#endif
-  // ---- behind the turn: the member list ----
-  if (emit) {
-    total = __shfl_sync(0xffffffffu, total, 0);
-    ninst = __shfl_sync(0xffffffffu, ninst, 0);
-    if (lane == 0) {
-      cc.members[total] = seed;
-      if (ninst < cc.max_inst) cc.inst_offsets[ninst + 1] = total + ev.size;
-    }
-    if (!wide) {
-      int run = 1;
-#pragma unroll 1
-      for (int h = 0; h < 2; ++h) {
-        const unsigned mine = h ? ev.mhi : ev.mlo;
-        unsigned any = __reduce_or_sync(0xffffffffu, mine);
-        while (any) {
-          const int kb = __ffs((int)any) - 1;
-          any &= any - 1;
-          const bool in = (mine >> kb) & 1u;
-          const unsigned bal = __ballot_sync(0xffffffffu, in);
-          if (in) cc.members[total + run + __popc(bal & lt_mask)] = (j0 >= 0 && k0 == kb + h * 32) ? j0 : j1;
-          run += __popc(bal);
-        }
-      }
-    }
-  }
-}
-
-__global__ void __launch_bounds__(GS_THREADS, 1)
-    gc_group_stream_kernel(GroupArgs ga, const int *__restrict__ d_C, int C_cap, double gc_size, float g_lo, float g_hi,
-                           int gc_threshold, int max_inst, int *__restrict__ fallback) {
-  extern __shared__ __align__(16) unsigned char s_raw[];
-  __shared__ __align__(8) StreamState S;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int C = min(*d_C, C_cap);
-  const int row_words = gc_row_words(C);
-  if (row_words > GS_MAX_ROW_WORDS) {  // uniform
-    if (tid == 0) *fallback = 1;
-    return;
-  }
-  const int nq = row_words >> 7;
-  unsigned *s_taken = reinterpret_cast<unsigned *>(s_raw);
-  const uint4 *s_taken4 = reinterpret_cast<const uint4 *>(s_raw);
-  unsigned char *ring = s_raw + GS_MAX_ROW_WORDS * 4;
-  const unsigned bar0 = (unsigned)__cvta_generic_to_shared(&S.bar_disp[0]);
-  const unsigned BAR_DISP = bar0, BAR_ALLOC = bar0 + 8 * GS_NSLOT, BAR_READY = bar0 + 16 * GS_NSLOT,
-                 BAR_COMMIT = bar0 + 24 * GS_NSLOT, BAR_FREE = bar0 + 32 * GS_NSLOT;
-
-  for (int w = tid; w < row_words; w += GS_THREADS) {
-    const int j0 = w * 32;
-    s_taken[w] = (j0 + 32 <= C) ? 0u : ((j0 >= C) ? ~0u : ~((1u << (C - j0)) - 1u));  // padding counts as taken
-  }
-  if (tid < 5 * GS_NSLOT) mbar_init(bar0 + 8 * tid, 1);
-  if (tid == 0) {
-    S.issue = S.alloc_done = S.commit_done = S.ring_head = S.ring_tail = 0;
-    S.take = 0;
-    S.end_ticket = 0x7fffffff;
-    S.abort = 0;
-    S.total = S.n_inst = 0;
-    ga.inst_offsets[0] = 0;
-  }
-  __syncthreads();
-  if (tid == 0) {  // ticket 0 has no predecessor
-    mbar_arrive(BAR_ALLOC);
-    mbar_arrive(BAR_COMMIT);
-  }
-#ifdef B200_GC_TIMING
-  long long tq[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  long long tl = clock64();
-#define ST(i)                      \
-  do {                             \
-    const long long n__ = clock64(); \
-    tq[i] += n__ - tl;             \
-    tl = n__;                      \
-  } while (0)
-#else
-#define ST(i)
-#endif
-
-  if (warp == 0) {
-    // ------------------------------------------------ dispatcher ----------------------------------------------
-    if (lane == 0) {
-      int pos = 0, ends = 0;
-      for (int t = 0;; ++t) {
-        const int s = t & (GS_NSLOT - 1);
-        if (t >= GS_NSLOT) GS_WAIT_COARSE(BAR_FREE + 8 * s, ((t / GS_NSLOT) - 1) & 1, 100, 1, t);
-        ST(0);
-        if (ld_vol(&S.abort)) break;
-        int p = -1;
-        int w = pos >> 5;
-        unsigned bits = 0u;
-        if (w < row_words) {
-          bits = ~s_taken[w] & ~((1u << (pos & 31)) - 1u);
-          while (!bits && ++w < row_words) bits = ~s_taken[w];
-        }
-        if (bits) {
-          p = w * 32 + __ffs(bits) - 1;
-          pos = p + 1;
-        } else {
-          pos = row_words * 32;
-          if (ends == 0) st_vol(&S.end_ticket, t);
-          ++ends;
-        }
-        st_vol(&S.seed[s], p);
-        mbar_arrive(BAR_DISP + 8 * s);
-        ST(1);
-#ifdef B200_GC_TIMING
-        tq[7] += 1;
-#endif
-        if (ends == GS_PROD) break;  // every producer gets one end marker (and passes it on to a consumer)
-      }
-    }
-  } else if (warp <= GS_PROD) {
-    // ------------------------------------------------ producer ------------------------------------------------
-    while (true) {
-      int t = 0, p = -1;
-      if (lane == 0) {
-        t = atomicAdd(&S.issue, 1);
-        GS_WAIT_COARSE(BAR_DISP + 8 * (t & (GS_NSLOT - 1)), (t / GS_NSLOT) & 1, 100, 2, t);
-        p = ld_vol(&S.seed[t & (GS_NSLOT - 1)]);
-      }
-      t = __shfl_sync(0xffffffffu, t, 0);
-      p = __shfl_sync(0xffffffffu, p, 0);
-      ST(0);
-      if (ld_vol(&S.abort)) break;
-      const int s = t & (GS_NSLOT - 1), sn = (t + 1) & (GS_NSLOT - 1);
-      const unsigned par = (t / GS_NSLOT) & 1;
-      if (p < 0) {  // past the last position: an end marker for the consumer that draws this ticket
-        if (lane == 0) mbar_arrive(BAR_READY + 8 * s);
-        break;
-      }
-      // the seed's row without what is taken already; lane l owns pieces [l nq, (l + 1) nq): its candidates are
-      // consecutive in the ascending list.  Pieces that are taken completely are not read.
-      const uint4 *row4 = reinterpret_cast<const uint4 *>(ga.adj + (size_t)p * row_words) + lane * nq;
-      const uint4 *tk4 = s_taken4 + lane * nq;
-      uint4 x[GS_MAXQ];
-#pragma unroll
-      for (int i = 0; i < GS_MAXQ; ++i) {
-        x[i] = make_uint4(0u, 0u, 0u, 0u);
-        if (i < nq) {
-          const uint4 tk = tk4[i];
-          if ((tk.x & tk.y & tk.z & tk.w) != ~0u) x[i] = __ldg(row4 + i);
-        }
-      }
-      int cnt = 0;
-#pragma unroll
-      for (int i = GS_MAXQ - 1; i >= 0; --i) {
-        if (i < nq) {
-          const uint4 tk = tk4[i];
-          x[i].x &= ~tk.x, x[i].y &= ~tk.y, x[i].z &= ~tk.z, x[i].w &= ~tk.w;
-          cnt += __popc(x[i].x) + __popc(x[i].y) + __popc(x[i].z) + __popc(x[i].w);
-        }
-      }
-      const int incl = warp_incl_scan(cnt, lane);
-      int o = incl - cnt;
-      const int n0 = __shfl_sync(0xffffffffu, incl, 31);
-      ST(1);
-      // ring space, in ticket order
-      const int nb = (n0 + 31) >> 5;
-      int start = 0;
-      if (lane == 0) {
-        while (t - ld_vol(&S.alloc_done) > 2 && !ld_vol(&S.abort)) __nanosleep(150);  // only the next two look at the barrier
-        GS_WAIT(BAR_ALLOC + 8 * s, par, 3, t);
-        if (n0 > GS_LCAP) {
-          *fallback = 1;
-          st_vol(&S.abort, 1);
-        }
-        int H = ld_vol(&S.ring_head);
-        start = H % GS_NBLK;
-        if (nb > 0 && start + nb > GS_NBLK) {
-          H += GS_NBLK - start;
-          start = 0;
-        }
-        if (H + nb - ld_vol(&S.ring_tail) > GS_NBLK) {
-          const long long t0 = clock64();
-          while (H + nb - ld_vol(&S.ring_tail) > GS_NBLK && !ld_vol(&S.abort)) {
-            __nanosleep(200);
-            if (clock64() - t0 > 4000000000ll) {
-              GS_GIVE_UP(4, t);
-              break;
-            }
-          }
-        }
-        st_vol(&S.blk[s], start);
-        st_vol(&S.vend[s], H + nb);
-        st_vol(&S.ring_head, H + nb);
-        st_vol(&S.alloc_done, t + 1);
-        mbar_arrive(BAR_ALLOC + 8 * sn);
-      }
-      start = __shfl_sync(0xffffffffu, start, 0);
-      ST(2);
-      if (ld_vol(&S.abort)) break;
-      unsigned char *chunk = ring + (size_t)start * GS_BLK;
-      // candidate indices in ascending order
-#pragma unroll
-      for (int i = 0; i < GS_MAXQ; ++i) {
-        if (i < nq) {
-          const int base = (lane * nq + i) * 128;
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            const unsigned long long v = h ? (((unsigned long long)x[i].w << 32) | x[i].z) : (((unsigned long long)x[i].y << 32) | x[i].x);
-            if (v) o = stream_list_piece(v, base + h * 64, chunk, o);
-          }
-        }
-      }
-      __syncwarp();
-      ST(3);
-      // their points, and whether they fit the first candidate (its bitmap row: bit 31 of the index)
-      const unsigned *rowc = ga.adj + (size_t)(nb ? *reinterpret_cast<const unsigned *>(chunk) : 0u) * row_words;  // list[0]
-      for (int k0 = 0; k0 < nb; k0 += 4) {
-        int j[4];
-        float4 m[4], sc[4];
-        unsigned fw[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const int k = k0 + u;
-          j[u] = (k < nb && k * 32 + lane < n0) ? *reinterpret_cast<const int *>(chunk + k * GS_BLK + lane * 4) : -1;
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u)
-          if (j[u] >= 0) {
-            m[u] = __ldg(ga.mp + j[u]);
-            sc[u] = __ldg(ga.sp + j[u]);
-            fw[u] = __ldg(rowc + (j[u] >> 5));
-          }
-#pragma unroll
-        for (int u = 0; u < 4; ++u)
-          if (j[u] >= 0) {
-            unsigned char *blk = chunk + (k0 + u) * GS_BLK;
-            float *pb = reinterpret_cast<float *>(blk) + lane;
-            if ((fw[u] >> (j[u] & 31)) & 1u) *reinterpret_cast<unsigned *>(blk + lane * 4) = (unsigned)j[u] | 0x80000000u;
-            pb[32] = m[u].x, pb[64] = m[u].y, pb[96] = m[u].z;
-            pb[128] = sc[u].x, pb[160] = sc[u].y, pb[192] = sc[u].z;
-          }
-      }
-      __syncwarp();
-      if (lane == 0) {
-        st_vol(&S.n[s], n0);
-        mbar_arrive(BAR_READY + 8 * s);
-      }
-      ST(4);
-#ifdef B200_GC_TIMING
-      tq[7] += 1;
-#endif
-    }
-  } else {
-    // ------------------------------------------------ consumer ------------------------------------------------
-    StreamCommit cc;
-    cc.s_taken = s_taken;
-    cc.S = &S;
-    cc.members = ga.members;
-    cc.inst_offsets = ga.inst_offsets;
-    cc.gc_threshold = gc_threshold;
-    cc.max_inst = max_inst;
-    cc.g_lo = g_lo, cc.g_hi = g_hi, cc.gc_size = gc_size;
-    cc.tq = nullptr;
-#ifdef B200_GC_TIMING
-    cc.tq = tq;
-#endif
-    // Tickets are dealt round-robin (consumer c takes c, c + GS_CONS, ...).  Only the consumers whose turn is at most
-    // two commits away look at their barrier; the others sleep on the commit counter.
-    const int cw = warp - 1 - GS_PROD;
-    for (int u = cw;; u += GS_CONS) {
-      if (lane == 0) GS_WAIT_COARSE(BAR_READY + 8 * (u & (GS_NSLOT - 1)), (u / GS_NSLOT) & 1, 40, 5, u);
-      __syncwarp();
-      ST(0);
-      const int s = u & (GS_NSLOT - 1);
-      const int seed = ld_vol(&S.seed[s]);
-      const bool aborted = ld_vol(&S.abort) != 0;
-      if (aborted || seed < 0) {  // past the last position (or giving up)
-        if (!aborted && u == ld_vol(&S.end_ticket) && lane == 0) {  // every seed before the end has committed: result count
-          GS_WAIT(BAR_COMMIT + 8 * s, (u / GS_NSLOT) & 1, 6, u);
-          if (!ld_vol(&S.abort)) *ga.n_inst_out = ld_vol(&S.n_inst);
-        }
-        break;
-      }
-      const int n = ld_vol(&S.n[s]), vend = ld_vol(&S.vend[s]);
-      const unsigned char *chunk = ring + (size_t)ld_vol(&S.blk[s]) * GS_BLK;
-      const StreamEval ev = stream_grow(s_taken, chunk, seed, n, lane, g_lo, g_hi, gc_size);
-      ST(1);
-      if (lane == 0) {
-        while (u - ld_vol(&S.commit_done) > 2 && !ld_vol(&S.abort)) __nanosleep(100);  // only the next two look at the barrier
-        GS_WAIT(BAR_COMMIT + 8 * s, (u / GS_NSLOT) & 1, 7, u);
-      }
-      __syncwarp();
-      ST(2);
-      stream_commit(cc, ev, chunk, seed, n, lane, BAR_COMMIT + 8 * ((u + 1) & (GS_NSLOT - 1)), u, BAR_FREE + 8 * s, vend);
-      ST(3);
-#ifdef B200_GC_TIMING
-      tq[7] += 1;
-#endif
-    }
-  }
-#ifdef B200_GC_TIMING
-  if (ga.dbg && lane == 0)
-    for (int i = 0; i < 8; ++i) ga.dbg[warp * 8 + i] = tq[i];
-#endif
 }
 
 // ---- RANSAC pose per instance -------------------------------------------------------------------
@@ -2188,7 +1198,7 @@ int dev_gc(b200_ctx *ctx, const float4 *d_model_kp, const float4 *d_scene_kp, co
   DevBuf<b200_corr> sorted;
   DevBuf<float4> mp, sp;
   DevBuf<unsigned> adj;
-  DevBuf<int> overflow, members, fb, sort_fb;
+  DevBuf<int> overflow, members, sort_fb;
   B200_TRY(sorted.alloc(ctx, (size_t)C_eff));
   B200_TRY(sort_fb.alloc(ctx, 1));
   B200_TRY(mp.alloc(ctx, (size_t)C_eff));
@@ -2227,9 +1237,8 @@ int dev_gc(b200_ctx *ctx, const float4 *d_model_kp, const float4 *d_scene_kp, co
     gc_adjacency_kernel<<<grid, ADJ_THREADS, 0, ctx->stream>>>(mp.p, sp.p, d_C, C_eff, gc_size, g_lo, g_hi, adj.p);
     B200_LAUNCHED(ctx);
   }
-  B200_TRY(overflow.alloc(ctx, (size_t)std::max(GW, GCL) * C_eff));
+  B200_TRY(overflow.alloc(ctx, (size_t)GCL * C_eff));
   B200_TRY(members.alloc(ctx, (size_t)C_eff));
-  B200_TRY(fb.alloc(ctx, 16));
   GroupArgs ga;
   ga.adj = adj.p;
   ga.mp = mp.p;
@@ -2242,7 +1251,7 @@ int dev_gc(b200_ctx *ctx, const float4 *d_model_kp, const float4 *d_scene_kp, co
   const bool debug = getenv("B200_GC_DEBUG") != nullptr;
   ga.dbg = nullptr;
   if (debug) {
-    B200_TRY(dbg.alloc(ctx, 256));
+    B200_TRY(dbg.alloc(ctx, GCL * 8));
     B200_TRY(dbg.zero());
     ga.dbg = dbg.p;
   }
@@ -2251,60 +1260,16 @@ int dev_gc(b200_ctx *ctx, const float4 *d_model_kp, const float4 *d_scene_kp, co
   if (ctx->wide) ctx->wide->leave();
   {
     StageScope st_(ctx, ST_GC_GROUP);
-    const size_t row_bytes = (size_t)row_words_cap * sizeof(unsigned);
-    const char *sel = getenv("B200_GC_GROUP");  // "cluster" (default) | "cta" | "stream" (experimental, see its header)
-    const bool use_stream = sel && !strcmp(sel, "stream") && row_words_cap <= GS_MAX_ROW_WORDS;
-    const int *gate = nullptr;
-    if (use_stream) {
-      // one CTA: producer warps stage the seeds' candidates in shared memory, consumer warps grow and commit in order.
-      // A scene it cannot take (a seed with more than GS_LCAP live candidates) raises the flag and the round-based
-      // kernel launched behind it does the scene instead; otherwise that launch returns at once.
-      B200_CUDA(ctx, cudaMemsetAsync(fb.p, 0, 16 * sizeof(int), ctx->stream));
-      const size_t smem = (size_t)GS_MAX_ROW_WORDS * 4 + (size_t)GS_NBLK * GS_BLK;
-      B200_CUDA(ctx, ensure_dyn_smem(gc_group_stream_kernel, smem));
-      gc_group_stream_kernel<<<1, GS_THREADS, smem, ctx->stream>>>(ga, d_C, C_eff, gc_size, g_lo, g_hi, gc_threshold, max_inst,
-                                                                  fb.p);
-      B200_LAUNCHED(ctx);
-      gate = fb.p;
-    }
-    const bool use_cluster = !(sel && !strcmp(sel, "cta")) && 2 * row_bytes <= 200 * 1024;
-    if (use_cluster) {
-      // one 8-CTA cluster: a seed per CTA; shared memory = taken bitmap + candidate bitmap
-      const size_t smem = 2 * row_bytes;
-      B200_CUDA(ctx, ensure_dyn_smem(gc_group_cluster_kernel, smem));
-      gc_group_cluster_kernel<<<GCL, GCL_THREADS, smem, ctx->stream>>>(ga, d_C, C_eff, gc_size, g_lo, g_hi, gc_threshold,
-                                                                      max_inst, gate);
-      B200_LAUNCHED(ctx);
-    } else {
-      // single CTA: the taken bitmap plus one candidate bitmap per concurrently evaluated seed
-      const size_t budget = 160 * 1024;
-      if (2 * row_bytes > budget) return ctx->fail(B200_ERR_CAPACITY, "gc: too many correspondences for the grouping kernel");
-      const size_t smem = std::min(budget, row_bytes * (size_t)(1 + GW));
-      B200_CUDA(ctx, ensure_dyn_smem(gc_group_kernel, smem));
-      gc_group_kernel<<<1, GG_THREADS, smem, ctx->stream>>>(ga, d_C, C_eff, (int)smem, gc_size, g_lo, g_hi, gc_threshold,
-                                                            max_inst, gate);
-      B200_LAUNCHED(ctx);
-    }
+    // one 8-CTA cluster: a seed per CTA; shared memory = taken bitmap + candidate bitmap (at most 2 x 64 KiB: GC_MAX_C
+    // caps a row at 16 384 words)
+    const size_t smem = 2 * (size_t)row_words_cap * sizeof(unsigned);
+    B200_CUDA(ctx, ensure_dyn_smem(gc_group_cluster_kernel, smem));
+    gc_group_cluster_kernel<<<GCL, GCL_THREADS, smem, ctx->stream>>>(ga, d_C, C_eff, gc_size, g_lo, g_hi, gc_threshold,
+                                                                    max_inst);
+    B200_LAUNCHED(ctx);
   }
   if (debug) {
-    int f[16];
-    B200_CUDA(ctx, cudaMemcpyAsync(f, fb.p, sizeof(f), cudaMemcpyDeviceToHost, ctx->stream));
-    B200_CUDA(ctx, ctx->sync());
-    fprintf(stderr, "gc_group stream: handed over %d, wait %d ticket %d | issue %d take %d head %d tail %d end %d\n", f[0], f[1], f[2],
-            f[3], f[4], f[5], f[6], f[7]);
-  }
-  if (debug && getenv("B200_GC_STREAM_TIMING")) {
-    long long h[256];
-    B200_CUDA(ctx, cudaMemcpyAsync(h, dbg.p, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-    B200_CUDA(ctx, ctx->sync());
-    for (int w = 0; w < 1 + GS_PROD + GS_CONS; ++w)
-      fprintf(stderr,
-              w == 0 ? "dispatcher %2d: wait-free %lld pick %lld (%lld %lld %lld %lld %lld) tickets %lld\n"
-                     : (w <= GS_PROD ? "producer %2d: wait-turn %lld row %lld wait-ring %lld list %lld gather %lld (%lld %lld) slots %lld\n"
-                                     : "consumer %2d: wait-ready %lld grow %lld wait-commit %lld commit %lld [validate %lld in-turn %lld] regrown %lld slots %lld\n"),
-              w, h[w * 8], h[w * 8 + 1], h[w * 8 + 2], h[w * 8 + 3], h[w * 8 + 4], h[w * 8 + 5], h[w * 8 + 6], h[w * 8 + 7]);
-  } else if (debug) {
-    long long h[GW * 8];
+    long long h[GCL * 8];
     B200_CUDA(ctx, cudaMemcpyAsync(h, dbg.p, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
     B200_CUDA(ctx, ctx->sync());
     for (int w = 0; w < GCL; ++w)

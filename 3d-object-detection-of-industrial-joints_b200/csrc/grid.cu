@@ -275,8 +275,7 @@ int cloud_grid_for_knn(b200_cloud *c, int k, const GridView **out) {
     // 1.0 k -> 1.35, 1.5 k -> 1.58, 3 k -> 1.89 (smaller cells need the second ring too often, larger ones scan more);
     // with the heap and the slab pruning of search.cuh: 0.5 k -> 1.24, 0.7 k -> 1.09, 1.0 k -> 1.03, 1.4 k -> 1.09,
     // 2 k -> 1.16, 3 k -> 1.28
-    const char *cf = getenv("B200_KNN_CELL");  // points per surface cell as a multiple of k (tuning knob)
-    double target = std::max(2.0, (cf ? atof(cf) : 1.0) * k);
+    double target = std::max(2.0, 1.0 * k);
     float cell = (float)sqrt(area * target / std::max(c->n_valid, 1));
     B200_TRY(build_grid(c, cell, c->knn_grid));
     c->knn_grid_k = k;

@@ -22,11 +22,9 @@
 // with a bitonic sort: 2.45 ms, 1 331 M; (c) one query per thread with a density-estimated cut instead of the sorted
 // insertion: 2.4-3.5 ms — against 1.35 ms and 893 M here.  The ballot/compaction bookkeeping of the cooperative
 // forms costs about one warp instruction per candidate-query pair, more than the per-thread insertion they remove
-// (62 % of this kernel's instructions, search.cuh), so the per-thread kernel stays.  A sixth variant keeps the per-thread
-// form but replaces the insertion: the K smallest distances in registers by a min/max chain, then a second pass
-// that collects and orders the K winners (knn_query_2pass, opt-in): 1.45 ms — with 32 queries per warp some lane
-// passes the admission test at almost every candidate, so the 2 K-instruction chain runs about as often as the
-// insertion loop did.
+// (62 % of this kernel's instructions, search.cuh), so the per-thread kernel stays.  A two-pass form of the search (the K
+// smallest distances in registers, then a second pass collecting the winners) measured 1.45 ms against this kernel's
+// 1.32 ms (DESIGN.md section 4).
 #include <stdlib.h>
 #include <string.h>
 
@@ -107,8 +105,6 @@ __global__ void fill_nan_kernel(float *p, size_t n) {
 
 // kNN mode.  q == nullptr: the queries are the indexed surface points themselves, visited in cell
 // order (thread i takes g.pts[i]); results are scattered to the original row.
-// K2 > 0: the two-pass search of search.cuh for k == K2 (shared memory sized for K2 + KNN2_SLACK keys per thread).
-template <int K2>
 __global__ void normals_knn_kernel(GridView g, const float4 *__restrict__ q, int nq, int k, float vpx, float vpy,
                                    float vpz, float4 *__restrict__ out) {
   extern __shared__ unsigned char smem_raw[];
@@ -127,13 +123,7 @@ __global__ void normals_knn_kernel(GridView g, const float4 *__restrict__ q, int
   }
   float4 o = make_float4(nanf32(), nanf32(), nanf32(), nanf32());
   if (finite3(p.x, p.y, p.z)) {
-    int cnt;
-    if (K2 > 0) {
-      cnt = knn_query_2pass<(K2 > 0 ? K2 : 1)>(g, p.x, p.y, p.z, sk, T, K2 + KNN2_SLACK);
-      if (cnt < 0) cnt = knn_query(g, p.x, p.y, p.z, k, sk, T);  // more ties at the k-th distance than the list takes
-    } else {
-      cnt = knn_query(g, p.x, p.y, p.z, k, sk, T);
-    }
+    const int cnt = knn_query(g, p.x, p.y, p.z, k, sk, T);
     if (cnt >= 3) {
       float accu[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
       for (int j = 0; j < cnt; ++j) {
@@ -379,16 +369,10 @@ int dev_normals(b200_ctx *ctx, b200_cloud *c, const float4 *d_q, int nq, bool q_
     if (k > 1024) return ctx->fail(B200_ERR_INVALID, "normals: k must be <= 1024");
     const GridView *g;
     B200_TRY(cloud_grid_for_knn(c, k, &g));
-    // B200_NORMALS_KNN=2pass: the two-pass search of search.cuh for k = 10 / 20 (bit-identical; measured 1.45 ms
-    // against 1.32 ms for the sorted-insertion search on the 1 M-point scene, so it is not the default; the tests
-    // compare the two).
-    const char *sel = getenv("B200_NORMALS_KNN");
-    const bool two_pass = (k == 10 || k == 20) && sel && !strcmp(sel, "2pass");
     size_t smem;
-    const int T = knn_threads_for(two_pass ? k + KNN2_SLACK : k, &smem);
+    const int T = knn_threads_for(k, &smem);
     if (smem > ctx->smem_optin) return ctx->fail(B200_ERR_INVALID, "normals: k too large for shared memory");
-    auto kern = two_pass ? (k == 10 ? normals_knn_kernel<10> : normals_knn_kernel<20>) : normals_knn_kernel<0>;
-    B200_CUDA(ctx, ensure_dyn_smem(kern, smem));
+    B200_CUDA(ctx, ensure_dyn_smem(normals_knn_kernel, smem));
     StageScope st_(ctx, ST_NORMALS);
     if (q_is_surface) {
       // rows with non-finite coordinates are not in the grid: they keep NaN normals (PCL: is_dense=false)
@@ -397,11 +381,12 @@ int dev_normals(b200_ctx *ctx, b200_cloud *c, const float4 *d_q, int nq, bool q_
         B200_LAUNCHED(ctx);
       }
       if (c->n_valid > 0) {
-        kern<<<ceil_div(c->n_valid, T), T, smem, ctx->stream>>>(*g, nullptr, c->n_valid, k, vpx, vpy, vpz, out);
+        normals_knn_kernel<<<ceil_div(c->n_valid, T), T, smem, ctx->stream>>>(*g, nullptr, c->n_valid, k, vpx, vpy, vpz,
+                                                                              out);
         B200_LAUNCHED(ctx);
       }
     } else {
-      kern<<<ceil_div(nq, T), T, smem, ctx->stream>>>(*g, d_q, nq, k, vpx, vpy, vpz, out);
+      normals_knn_kernel<<<ceil_div(nq, T), T, smem, ctx->stream>>>(*g, d_q, nq, k, vpx, vpy, vpz, out);
       B200_LAUNCHED(ctx);
     }
     return B200_OK;

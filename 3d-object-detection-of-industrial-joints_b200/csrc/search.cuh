@@ -196,119 +196,9 @@ __device__ inline int knn_query(const GridView &g, float qx, float qy, float qz,
   return cnt;
 }
 
-// Two-pass form of knn_query for a compile-time K (the k's the reference's programs use most: 10 and 20).
-// 62 % of knn_query's instructions are the sorted insertion into the shared-memory list: every candidate that passes
-// the "nearer than the current k-th" test in ANY lane makes the whole warp walk a load / compare / store loop of
-// that lane's shift length.  Here the first pass keeps only the K smallest DISTANCES, in registers, as a sorted
-// array maintained by a min/max chain (two FMNMX per slot, no memory, no data-dependent trip count): it yields the
-// exact k-th smallest distance d_K of the certified block.  The second pass walks the same cells again (they are in
-// L1) and appends every candidate with d2 <= d_K to the shared-memory list (K of them plus ties at d_K), which is
-// then ordered once by (d2, index), all lanes together.  The result is knn_query's, bit for bit.
-// MEASURED (1 M points, k = 20): 1.45 - 1.8 ms against knn_query's 1.32 - 1.36 ms although it executes 20 % fewer warp
-// instructions (710 M against 881 M) with more lanes active (16.7 against 10.8 of 32): the candidate loop now has so
-// little work per load that it waits on the loads (long_scoreboard 4.0 per issue against 2.3; issue-active 51 %
-// against 65 %); four loads in flight per step did not change that (1.76 ms).  Opt-in only (normals.cu); kept as the
-// record of the experiment and because the tests pin it bit for bit against the insertion form.
-// sk: this thread's column of a [cap][T] array, cap >= K + KNN2_SLACK.  Returns the count (<= K), or -1 when more
-// than cap candidates tie into the list (the caller falls back to knn_query).
-constexpr int KNN2_SLACK = 4;   // 12 cost a third of the resident warps (shared memory); more ties than this fall back
-
-template <class F>
-__device__ __forceinline__ void knn_for_shell(const GridView &g, int cx, int cy, int cz, int R, F &&run) {
-  const int z0 = max(cz - R, 0), z1 = min(cz + R, g.dz - 1);
-  const int y0 = max(cy - R, 0), y1 = min(cy + R, g.dy - 1);
-  const int x0 = max(cx - R, 0), x1 = min(cx + R, g.dx - 1);
-  for (int z = z0; z <= z1; ++z)
-    for (int y = y0; y <= y1; ++y) {
-      const bool face = (abs(z - cz) == R) || (abs(y - cy) == R);
-      const int row = g.dx * (y + g.dy * z);
-      if (face) {
-        run(row + x0, row + x1);
-      } else {
-        if (cx - R >= 0) run(row + cx - R, row + cx - R);
-        if (cx + R <= g.dx - 1) run(row + cx + R, row + cx + R);  // R > 0 here (R == 0 is a face row)
-      }
-    }
-}
-
-template <int K>
-__device__ inline int knn_query_2pass(const GridView &g, float qx, float qy, float qz, unsigned long long *sk, int T, int cap) {
-  const float4 *__restrict__ pts = g.pts;
-  const int *__restrict__ cs = g.cell_start;
-  if (g.n <= 0) return 0;
-  const int cx = grid_coord(qx, g.lox, g.inv_h, g.dx);
-  const int cy = grid_coord(qy, g.loy, g.inv_h, g.dy);
-  const int cz = grid_coord(qz, g.loz, g.inv_h, g.dz);
-  const int maxR = max(g.dx, max(g.dy, g.dz));
-  const float margin = 4e-6f * (g.coord_scale + fabsf(qx) + fabsf(qy) + fabsf(qz)) + 1e-5f * g.h;
-  const float INF = __int_as_float(0x7f800000);
-  float l[K];  // the K smallest squared distances seen so far, ascending
-#pragma unroll
-  for (int j = 0; j < K; ++j) l[j] = INF;
-  int Rf = 0;
-  for (int R = 0; R <= maxR; ++R) {
-    Rf = R;
-    knn_for_shell(g, cx, cy, cz, R, [&](int c0, int c1) {
-      const int s = cs[c0], e = cs[c1 + 1];
-      for (int j = s; j < e; ++j) {
-        const float4 p = pts[j];
-        float x = sqdist3(qx, qy, qz, p.x, p.y, p.z);
-        if (x < l[K - 1]) {
-#pragma unroll
-          for (int t = 0; t < K; ++t) {
-            const float lo = fminf(l[t], x);
-            x = fmaxf(l[t], x);
-            l[t] = lo;
-          }
-        }
-      }
-    });
-    const bool whole = (max(cz - R, 0) == 0 && min(cz + R, g.dz - 1) == g.dz - 1 && max(cy - R, 0) == 0 &&
-                        min(cy + R, g.dy - 1) == g.dy - 1 && max(cx - R, 0) == 0 && min(cx + R, g.dx - 1) == g.dx - 1);
-    if (whole) break;
-    if (l[K - 1] < INF) {
-      // everything outside the scanned block is at least `cert` away from the query
-      float cert = 3.0e38f;
-      if (cx - R > 0) cert = fminf(cert, qx - (g.lox + (float)(cx - R) * g.h));
-      if (cx + R < g.dx - 1) cert = fminf(cert, (g.lox + (float)(cx + R + 1) * g.h) - qx);
-      if (cy - R > 0) cert = fminf(cert, qy - (g.loy + (float)(cy - R) * g.h));
-      if (cy + R < g.dy - 1) cert = fminf(cert, (g.loy + (float)(cy + R + 1) * g.h) - qy);
-      if (cz - R > 0) cert = fminf(cert, qz - (g.loz + (float)(cz - R) * g.h));
-      if (cz + R < g.dz - 1) cert = fminf(cert, (g.loz + (float)(cz + R + 1) * g.h) - qz);
-      cert -= margin;
-      if (cert > 0.f && l[K - 1] < cert * cert * 0.99999f) break;
-    }
-  }
-  // second pass: everything at or below the k-th distance, in scan order
-  const float dK = l[K - 1];
-  int m = 0;
-  for (int R = 0; R <= Rf; ++R)
-    knn_for_shell(g, cx, cy, cz, R, [&](int c0, int c1) {
-      const int s = cs[c0], e = cs[c1 + 1];
-      for (int j = s; j < e; ++j) {
-        const float4 p = pts[j];
-        const float d = sqdist3(qx, qy, qz, p.x, p.y, p.z);
-        if (d <= dK) {
-          if (m < cap) sk[m * T] = ((unsigned long long)__float_as_uint(d) << 32) | (unsigned)orig_index(p);
-          ++m;
-        }
-      }
-    });
-  if (m > cap) return -1;
-  // (d2, index) order: FLANN's DistanceIndex::operator<
-  for (int i = 1; i < m; ++i) {
-    const unsigned long long key = sk[i * T];
-    int pos = i;
-    while (pos > 0) {
-      const unsigned long long pk = sk[(pos - 1) * T];
-      if (pk < key) break;
-      sk[pos * T] = pk;
-      --pos;
-    }
-    sk[pos * T] = key;
-  }
-  return min(m, K);
-}
+// A two-pass form of knn_query (the K smallest distances in registers by a min/max chain, then a second pass that
+// collects the winners) executed 20 % fewer instructions but measured 1.45 ms against 1.32 ms on the 1 M-point scene,
+// k = 20, because its candidate loop waits on its loads (DESIGN.md section 4).
 
 // Cell range of the ball around q, padded so that float rounding can never exclude a point the
 // distance test would accept.  Returns false if the ball misses the grid entirely.
