@@ -352,17 +352,9 @@ __global__ void __launch_bounds__(BOARD_THREADS)
 
   unsigned long long *key;
   int *pos;
-  float *f_cos, *f_ang;
-  if (glob_key) {
-    key = glob_key + (size_t)blockIdx.x * cap;
-    pos = glob_pos + (size_t)blockIdx.x * cap;
-    f_cos = glob_f + (size_t)blockIdx.x * cap * 2;
-  } else {
-    key = reinterpret_cast<unsigned long long *>(smem_raw);
-    pos = reinterpret_cast<int *>(smem_raw + (size_t)cap * 8);
-    f_cos = reinterpret_cast<float *>(smem_raw + (size_t)cap * 12);
-  }
-  f_ang = f_cos + cap;
+  cta_list(smem_raw, glob_key, glob_pos, cap, key, pos);
+  float *f_cos = glob_key ? glob_f + (size_t)blockIdx.x * cap * 2 : reinterpret_cast<float *>(smem_raw + (size_t)cap * 12);
+  float *f_ang = f_cos + cap;
   const int tid = threadIdx.x;
   const float4 *__restrict__ pts = g.pts;
   const int S = a.sectors;
@@ -500,7 +492,6 @@ __global__ void __launch_bounds__(BW_WARPS * 32)
   const int lane = threadIdx.x & 31;
   const int nwarps = gridDim.x * BW_WARPS;
   const float4 *__restrict__ pts = g.pts;
-  const int *__restrict__ cs = g.cell_start;
   const int S = a.sectors;
   const float radius2 = a.tangent_radius * a.tangent_radius;
   const float margin_distance2 = a.margin_thresh * a.margin_thresh * radius2;
@@ -515,42 +506,7 @@ __global__ void __launch_bounds__(BW_WARPS * 32)
     }
     const float4 c4 = kp[i];
     const float c[3] = {c4.x, c4.y, c4.z};
-    // ---- gather (cnt neighbours: the count pass ran the same test on the same points)
-    int n = 0;
-    {
-      int x0, x1, y0, y1, z0, z1;
-      if (ball_cell_range(g, c4.x, c4.y, c4.z, radius_f, x0, x1, y0, y1, z0, z1)) {
-        for (int zc = z0; zc <= z1; ++zc)
-          for (int yc = y0; yc <= y1; ++yc) {
-            const int base = g.dx * (yc + g.dy * zc);
-            const int s0 = cs[base + x0], e = cs[base + x1 + 1];
-            for (int j0 = s0; j0 < e; j0 += 128) {
-              float4 p[4];
-#pragma unroll
-              for (int u = 0; u < 4; ++u) {
-                const int j = j0 + 32 * u + lane;
-                p[u] = (j < e) ? pts[j] : make_float4(0.f, 0.f, 0.f, 0.f);
-              }
-#pragma unroll
-              for (int u = 0; u < 4; ++u) {
-                const int j = j0 + 32 * u + lane;
-                const float d2 = sqdist3(c4.x, c4.y, c4.z, p[u].x, p[u].y, p[u].z);
-                const bool hit = j < e && d2 < r2;
-                const unsigned m = __ballot_sync(0xffffffffu, hit);
-                if (hit) {
-                  const int slot = n + __popc(m & ((1u << lane) - 1u));
-                  if (slot < BW_CAP) {
-                    sm.key[slot] = nbr_key(d2, orig_index(p[u]));
-                    sm.pos[slot] = j;
-                  }
-                }
-                n += __popc(m);
-              }
-            }
-          }
-      }
-    }
-    if (n > BW_CAP) n = BW_CAP;  // cannot happen
+    const int n = warp_gather_radius<BW_CAP>(g, c4, radius_f, r2, sm.key, sm.pos, lane);
     __syncwarp();  // the support stays in gather order: nothing below depends on the order (BoardScan2)
     // ---- planeFitting: float64 centroid and scatter
     double m[3] = {0.0, 0.0, 0.0}, nm[3] = {0.0, 0.0, 0.0};

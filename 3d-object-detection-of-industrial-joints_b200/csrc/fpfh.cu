@@ -149,13 +149,7 @@ __global__ void __launch_bounds__(FPFH_THREADS)
   __shared__ int s_bins[33];
   unsigned long long *key;
   int *pos;
-  if (glob_key) {
-    key = glob_key + (size_t)blockIdx.x * cap;
-    pos = glob_pos + (size_t)blockIdx.x * cap;
-  } else {
-    key = reinterpret_cast<unsigned long long *>(smem_raw);
-    pos = reinterpret_cast<int *>(smem_raw + (size_t)cap * sizeof(unsigned long long));
-  }
+  cta_list(smem_raw, glob_key, glob_pos, cap, key, pos);
   const int tid = threadIdx.x;
   const double kPi = 3.14159265358979323846;
   const float d_pi = 1.0f / (2.0f * (float)kPi);
@@ -201,13 +195,7 @@ __global__ void __launch_bounds__(FPFH_THREADS)
   __shared__ float s_tile[32 * 33];
   unsigned long long *key;
   int *pos;
-  if (glob_key) {
-    key = glob_key + (size_t)blockIdx.x * cap;
-    pos = glob_pos + (size_t)blockIdx.x * cap;
-  } else {
-    key = reinterpret_cast<unsigned long long *>(smem_raw);
-    pos = reinterpret_cast<int *>(smem_raw + (size_t)cap * sizeof(unsigned long long));
-  }
+  cta_list(smem_raw, glob_key, glob_pos, cap, key, pos);
   const int tid = threadIdx.x;
   for (int i = blockIdx.x; i < nq; i += gridDim.x) {
     if (counts[i] < min_count) continue;  // smaller neighbourhoods: fpfh_weight_warp_kernel
@@ -283,45 +271,6 @@ struct FwSmem {
   int bins[36];
 };
 
-// neighbours of c with d2 < r2 appended in scan order: pos (and keys when WITH_KEYS); returns the count
-template <bool WITH_KEYS>
-__device__ __forceinline__ int fw_gather(const GridView &g, const float4 c, float radius, float r2, FwSmem &sm, int lane) {
-  const float4 *__restrict__ pts = g.pts;
-  const int *__restrict__ cs = g.cell_start;
-  int n = 0;
-  int x0, x1, y0, y1, z0, z1;
-  if (!ball_cell_range(g, c.x, c.y, c.z, radius, x0, x1, y0, y1, z0, z1)) return 0;
-  for (int z = z0; z <= z1; ++z)
-    for (int y = y0; y <= y1; ++y) {
-      const int base = g.dx * (y + g.dy * z);
-      const int s0 = cs[base + x0], e = cs[base + x1 + 1];
-      for (int j0 = s0; j0 < e; j0 += 128) {
-        float4 p[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const int j = j0 + 32 * u + lane;
-          p[u] = (j < e) ? pts[j] : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const int j = j0 + 32 * u + lane;
-          const float d2 = sqdist3(c.x, c.y, c.z, p[u].x, p[u].y, p[u].z);
-          const bool hit = j < e && d2 < r2;
-          const unsigned m = __ballot_sync(0xffffffffu, hit);
-          if (hit) {
-            const int slot = n + __popc(m & ((1u << lane) - 1u));
-            if (slot < FW_CAP) {
-              if (WITH_KEYS) sm.key[slot] = nbr_key(d2, orig_index(p[u]));
-              sm.pos[slot] = j;
-            }
-          }
-          n += __popc(m);
-        }
-      }
-    }
-  return min(n, FW_CAP);
-}
-
 // Pass 1 for surface points (cell order) with need[s] and at most FW_CAP neighbours
 __global__ void __launch_bounds__(FW_WARPS * 32)
     spfh_warp_kernel(GridView g, const float4 *__restrict__ nrm, const int *__restrict__ need,
@@ -336,7 +285,7 @@ __global__ void __launch_bounds__(FW_WARPS * 32)
     if (!need[s] || counts[s] > FW_CAP) continue;
     const float4 p = g.pts[s];
     const float4 np = nrm[s];
-    const int n = fw_gather<false>(g, p, radius, r2, sm, lane);
+    const int n = warp_gather_radius<FW_CAP>(g, p, radius, r2, nullptr, sm.pos, lane);
     sm.bins[lane] = 0;
     if (lane < 4) sm.bins[32 + lane] = 0;
     __syncwarp();
@@ -380,28 +329,8 @@ __global__ void __launch_bounds__(FW_WARPS * 32)
       for (int b = lane; b < 33; b += 32) out[row * 33 + b] = nanf32();
       continue;
     }
-    const int n = fw_gather<true>(g, c, radius, r2, sm, lane);
-    int np = 32;
-    while (np < n) np <<= 1;
-    for (int t = n + lane; t < np; t += 32) {
-      sm.key[t] = ~0ull;
-      sm.pos[t] = -1;
-    }
-    __syncwarp();
-    for (int k = 2; k <= np; k <<= 1)
-      for (int j = k >> 1; j > 0; j >>= 1) {
-        for (int t = lane; t < (np >> 1); t += 32) {
-          const int a = ((t & ~(j - 1)) << 1) | (t & (j - 1));
-          const int b = a | j;
-          const bool up = ((a & k) == 0);
-          const unsigned long long ka = sm.key[a], kb = sm.key[b];
-          if ((ka > kb) == up) {
-            sm.key[a] = kb;
-            sm.key[b] = ka;
-          }
-        }
-        __syncwarp();
-      }
+    const int n = warp_gather_radius<FW_CAP>(g, c, radius, r2, sm.key, nullptr, lane);
+    warp_bitonic_sort(sm.key, nullptr, n, lane);
     // lane l < 11 owns bins l, l + 11, l + 22: float32 sums in (d2, index) order, float64 block sums beside them
     float acc[3] = {0.f, 0.f, 0.f};
     double part[3] = {0.0, 0.0, 0.0};

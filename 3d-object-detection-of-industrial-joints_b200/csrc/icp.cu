@@ -38,9 +38,9 @@ __global__ void __launch_bounds__(ICP_THREADS)
   float d2 = 0.f;
   if (finite3(p.x, p.y, p.z)) {
     const int cnt = knn_query(g, p.x, p.y, p.z, 1, sk + threadIdx.x, ICP_THREADS);
-    if (cnt == 1 && !(knn_d2(sk[threadIdx.x]) > max_d2)) {
-      t = knn_orig(sk[threadIdx.x]);  // original row of the target cloud
-      d2 = knn_d2(sk[threadIdx.x]);
+    if (cnt == 1 && !(key_d2(sk[threadIdx.x]) > max_d2)) {
+      t = key_orig(sk[threadIdx.x]);  // original row of the target cloud
+      d2 = key_d2(sk[threadIdx.x]);
     }
   }
   tgt_idx[i] = t;

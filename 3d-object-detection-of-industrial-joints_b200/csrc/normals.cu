@@ -127,7 +127,7 @@ __global__ void normals_knn_kernel(GridView g, const float4 *__restrict__ q, int
     if (cnt >= 3) {
       float accu[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
       for (int j = 0; j < cnt; ++j) {
-        const float4 n = g.raw[knn_orig(sk[j * T])];
+        const float4 n = g.raw[key_orig(sk[j * T])];
         accu[0] += n.x * n.x;
         accu[1] += n.x * n.y;
         accu[2] += n.x * n.z;
@@ -160,13 +160,7 @@ __global__ void __launch_bounds__(128) normals_radius_kernel(GridView g, const f
   __shared__ float4 s_pts[128];
   unsigned long long *key;
   int *pos;
-  if (glob_key) {
-    key = glob_key + (size_t)blockIdx.x * cap;
-    pos = glob_pos + (size_t)blockIdx.x * cap;
-  } else {
-    key = reinterpret_cast<unsigned long long *>(smem_raw);
-    pos = reinterpret_cast<int *>(smem_raw + (size_t)cap * sizeof(unsigned long long));
-  }
+  cta_list(smem_raw, glob_key, glob_pos, cap, key, pos);
   for (int i = blockIdx.x; i < nq; i += gridDim.x) {
     if (counts[i] < min_count) continue;  // done by normals_radius_warp_kernel
     const float4 p = q[i];
@@ -245,7 +239,6 @@ __global__ void __launch_bounds__(NRW_WARPS * 32)
   const int lane = threadIdx.x & 31;
   const int nwarps = gridDim.x * NRW_WARPS;
   const float4 *__restrict__ pts = g.pts;
-  const int *__restrict__ cs = g.cell_start;
   // which components of a staged point (x, y, z, 1) this lane multiplies: xx xy xz yy yz zz x y z
   const int ia = (lane < 3) ? 0 : (lane < 5) ? 1 : (lane == 5) ? 2 : (lane < 9 ? lane - 6 : 0);
   const int ib = (lane < 3) ? lane : (lane < 5) ? lane - 2 : (lane == 5) ? 2 : 3;
@@ -257,65 +250,9 @@ __global__ void __launch_bounds__(NRW_WARPS * 32)
       if (lane == 0) out[i] = make_float4(nanf32(), nanf32(), nanf32(), nanf32());
       continue;
     }
-    // ---- gather (the count pass found cnt <= CAP neighbours: the same test on the same points)
-    int n = 0;
-    int x0, x1, y0, y1, z0, z1;
-    if (ball_cell_range(g, c.x, c.y, c.z, radius, x0, x1, y0, y1, z0, z1)) {
-      for (int z = z0; z <= z1; ++z)
-        for (int y = y0; y <= y1; ++y) {
-          const int base = g.dx * (y + g.dy * z);
-          const int s0 = cs[base + x0], e = cs[base + x1 + 1];
-          for (int j0 = s0; j0 < e; j0 += 128) {
-            float4 p[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-              const int j = j0 + 32 * u + lane;
-              p[u] = (j < e) ? pts[j] : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-              const int j = j0 + 32 * u + lane;
-              const float d2 = sqdist3(c.x, c.y, c.z, p[u].x, p[u].y, p[u].z);
-              const bool hit = j < e && d2 < r2;
-              const unsigned m = __ballot_sync(0xffffffffu, hit);
-              if (hit) {
-                const int slot = n + __popc(m & ((1u << lane) - 1u));
-                if (slot < CAP) {
-                  sm.key[slot] = nbr_key(d2, orig_index(p[u]));
-                  sm.pos[slot] = j;
-                }
-              }
-              n += __popc(m);
-            }
-          }
-        }
-    }
-    if (n > CAP) n = CAP;  // cannot happen: cnt is the same count
-    // ---- order by (d2, index): FLANN's result order
-    int np = 32;
-    while (np < n) np <<= 1;
-    for (int t = n + lane; t < np; t += 32) {
-      sm.key[t] = ~0ull;
-      sm.pos[t] = -1;
-    }
-    __syncwarp();
-    for (int k = 2; k <= np; k <<= 1)
-      for (int j = k >> 1; j > 0; j >>= 1) {
-        for (int t = lane; t < (np >> 1); t += 32) {
-          const int a = ((t & ~(j - 1)) << 1) | (t & (j - 1));
-          const int b = a | j;
-          const bool up = ((a & k) == 0);
-          const unsigned long long ka = sm.key[a], kb = sm.key[b];
-          if ((ka > kb) == up) {
-            sm.key[a] = kb;
-            sm.key[b] = ka;
-            const int pa = sm.pos[a];
-            sm.pos[a] = sm.pos[b];
-            sm.pos[b] = pa;
-          }
-        }
-        __syncwarp();
-      }
+    // ---- gather (cnt <= CAP neighbours), then order by (d2, index): FLANN's result order
+    const int n = warp_gather_radius<CAP>(g, c, radius, r2, sm.key, sm.pos, lane);
+    warp_bitonic_sort(sm.key, sm.pos, n, lane);
     // ---- the points in that order (w = 1: the plain sums read it as their second factor)
     for (int t = lane; t < n; t += 32) {
       const float4 v = pts[sm.pos[t]];

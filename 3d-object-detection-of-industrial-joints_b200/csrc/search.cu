@@ -23,8 +23,8 @@ __global__ void knn_search_kernel(GridView g, const float4 *__restrict__ q, int 
   for (int j = 0; j < k; ++j) {
     const bool have = j < cnt;
     const unsigned long long key = have ? sk[j * T] : 0ull;
-    idx[(size_t)i * k + j] = have ? knn_orig(key) : -1;
-    d2[(size_t)i * k + j] = have ? knn_d2(key) : __int_as_float(0x7f800000);
+    idx[(size_t)i * k + j] = have ? key_orig(key) : -1;
+    d2[(size_t)i * k + j] = have ? key_d2(key) : __int_as_float(0x7f800000);
   }
 }
 
@@ -55,13 +55,7 @@ __global__ void __launch_bounds__(128) radius_fill_kernel(GridView g, const floa
   __shared__ int s_count;
   unsigned long long *key;
   int *pos;
-  if (glob_key) {
-    key = glob_key + (size_t)blockIdx.x * cap;
-    pos = glob_pos + (size_t)blockIdx.x * cap;
-  } else {
-    key = reinterpret_cast<unsigned long long *>(smem_raw);
-    pos = reinterpret_cast<int *>(smem_raw + (size_t)cap * sizeof(unsigned long long));
-  }
+  cta_list(smem_raw, glob_key, glob_pos, cap, key, pos);
   for (int i = blockIdx.x; i < nq; i += gridDim.x) {
     if (offsets[i + 1] - offsets[i] < (long long)min_count) continue;  // shorter lists: radius_fill_warp_kernel
     const float4 p = q[i];
@@ -88,61 +82,12 @@ __global__ void __launch_bounds__(RFW_WARPS * 32)
   unsigned long long *key = s_key[threadIdx.x >> 5];
   const int lane = threadIdx.x & 31;
   const int nwarps = gridDim.x * RFW_WARPS;
-  const float4 *__restrict__ pts = g.pts;
-  const int *__restrict__ cs = g.cell_start;
   for (int i = blockIdx.x * RFW_WARPS + (threadIdx.x >> 5); i < nq; i += nwarps) {
     const long long o = offsets[i];
     const long long cnt = offsets[i + 1] - o;
     if (cnt == 0 || cnt > RFW_CAP) continue;
-    const float4 c = q[i];
-    int n = 0;
-    int x0, x1, y0, y1, z0, z1;
-    if (ball_cell_range(g, c.x, c.y, c.z, radius, x0, x1, y0, y1, z0, z1)) {
-      for (int z = z0; z <= z1; ++z)
-        for (int y = y0; y <= y1; ++y) {
-          const int base = g.dx * (y + g.dy * z);
-          const int s0 = cs[base + x0], e = cs[base + x1 + 1];
-          for (int j0 = s0; j0 < e; j0 += 128) {
-            float4 p[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-              const int j = j0 + 32 * u + lane;
-              p[u] = (j < e) ? pts[j] : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-              const int j = j0 + 32 * u + lane;
-              const float dd = sqdist3(c.x, c.y, c.z, p[u].x, p[u].y, p[u].z);
-              const bool hit = j < e && dd < r2;
-              const unsigned m = __ballot_sync(0xffffffffu, hit);
-              if (hit) {
-                const int slot = n + __popc(m & ((1u << lane) - 1u));
-                if (slot < RFW_CAP) key[slot] = nbr_key(dd, orig_index(p[u]));
-              }
-              n += __popc(m);
-            }
-          }
-        }
-    }
-    if (n > RFW_CAP) n = RFW_CAP;  // cannot happen: the count pass ran the same test
-    int np = 32;
-    while (np < n) np <<= 1;
-    for (int t = n + lane; t < np; t += 32) key[t] = ~0ull;
-    __syncwarp();
-    for (int k = 2; k <= np; k <<= 1)
-      for (int j = k >> 1; j > 0; j >>= 1) {
-        for (int t = lane; t < (np >> 1); t += 32) {
-          const int a = ((t & ~(j - 1)) << 1) | (t & (j - 1));
-          const int b = a | j;
-          const bool up = ((a & k) == 0);
-          const unsigned long long ka = key[a], kb = key[b];
-          if ((ka > kb) == up) {
-            key[a] = kb;
-            key[b] = ka;
-          }
-        }
-        __syncwarp();
-      }
+    const int n = warp_gather_radius<RFW_CAP>(g, q[i], radius, r2, key, nullptr, lane);
+    warp_bitonic_sort(key, nullptr, n, lane);
     for (int j = lane; j < n; j += 32) {
       idx[o + j] = key_orig(key[j]);
       d2[o + j] = key_d2(key[j]);

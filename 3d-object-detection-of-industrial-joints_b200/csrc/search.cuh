@@ -1,30 +1,35 @@
 // search.cuh — device-side exact neighbour search on the uniform grid.
 //
-//  knn_query       one query per thread, candidate list in shared memory; replaces
-//                  KdTreeFLANN::nearestKSearch as used by NormalEstimationOMP with setKSearch
-//                  (SHOT.cpp:302-308) and by the explicit calls (SHOT.cpp:163, Edge_detection.cpp:120).
-//  gather_radius   one query per CTA, neighbours appended to a list with warp-aggregated atomics;
-//                  replaces KdTreeFLANN::radiusSearch (SHOT_VAR.cpp:356; implicit in SHOT / FPFH /
-//                  radius normals).  Acceptance is d2 < (float)(r*r), strict, on the float32
-//                  L2_Simple distance — bit-identical to FLANN's test.
-//  bitonic_sort    orders a CTA's list by (d2, original index), the order FLANN returns
-//                  (RadiusResultSet is sorted with DistanceIndex::operator<).
+//  nbr_key             a neighbour as one 64-bit key: float bits of d2 (non-negative, so the unsigned order is the
+//                      float order) in the high word, ORIGINAL row index in the low word.  One unsigned compare is
+//                      FLANN's (distance, index) order (RadiusResultSet is sorted with DistanceIndex::operator<);
+//                      key_d2 / key_orig decode it.
+//  knn_query           one query per thread, candidate list in shared memory; replaces
+//                      KdTreeFLANN::nearestKSearch as used by NormalEstimationOMP with setKSearch
+//                      (SHOT.cpp:302-308) and by the explicit calls (SHOT.cpp:163, Edge_detection.cpp:120).
+//  Radius search replaces KdTreeFLANN::radiusSearch (SHOT_VAR.cpp:356; implicit in SHOT / FPFH / radius normals).
+//  Acceptance is d2 < (float)(r*r), strict, on the float32 L2_Simple distance — bit-identical to FLANN's test.
+//  cta_list            the list storage of a one-query-per-CTA kernel: shared memory or a slice of global scratch.
+//  gather_radius       one query per CTA, neighbours appended to a list with warp-aggregated atomics.
+//  count_radius_warp   one query per warp, the number of neighbours (sizes the lists of both gathers).
+//  bitonic_sort        orders a CTA's list by key.
+//  warp_gather_radius  one query per warp, neighbours appended in scan order to the warp's list by ballot compaction.
+//  warp_bitonic_sort   orders a warp's list by key, synchronised by __syncwarp only.
 #pragma once
+
+#include <type_traits>
 
 #include "common.cuh"
 
-__device__ __forceinline__ bool cand_before(float d, int o, float d2, int o2) {
-  return (d < d2) || (d == d2 && o < o2);
+__device__ __forceinline__ unsigned long long nbr_key(float d2, int orig) {
+  return ((unsigned long long)__float_as_uint(d2) << 32) | (unsigned)orig;
 }
+__device__ __forceinline__ float key_d2(unsigned long long k) { return __uint_as_float((unsigned)(k >> 32)); }
+__device__ __forceinline__ int key_orig(unsigned long long k) { return (int)(unsigned)(k & 0xffffffffull); }
 
-// Exact k nearest neighbours of (qx,qy,qz).  sk: this thread's column of a [k][T] shared array of 64-bit keys
-// (element j at [j*T]); key = float bits of d2 (non-negative, so the unsigned order is the float order) in the high
-// word, ORIGINAL row index in the low word: one unsigned compare is FLANN's (distance, index) order, and a shift
-// of the sorted list moves one 8-byte word per step.  Returns the number found (min(k, g.n)), sorted ascending.
-// Coordinates of a neighbour: g.raw[knn_orig(key)].
-__device__ __forceinline__ float knn_d2(unsigned long long key) { return __uint_as_float((unsigned)(key >> 32)); }
-__device__ __forceinline__ int knn_orig(unsigned long long key) { return (int)(unsigned)(key & 0xffffffffull); }
-
+// Exact k nearest neighbours of (qx,qy,qz).  sk: this thread's column of a [k][T] shared array of nbr_key keys
+// (element j at [j*T]): a shift of the sorted list moves one 8-byte word per step.  Returns the number found
+// (min(k, g.n)), sorted ascending.  Coordinates of a neighbour: g.raw[key_orig(key)].
 __device__ inline int knn_query(const GridView &g, float qx, float qy, float qz, int k, unsigned long long *sk, int T) {
   const float4 *__restrict__ pts = g.pts;
   const int *__restrict__ cs = g.cell_start;
@@ -66,7 +71,7 @@ __device__ inline int knn_query(const GridView &g, float qx, float qy, float qz,
     for (int j = s; j < e; ++j) {
       const float4 p = pts[j];
       const float d = sqdist3(qx, qy, qz, p.x, p.y, p.z);
-      const unsigned long long key = ((unsigned long long)__float_as_uint(d) << 32) | (unsigned)orig_index(p);
+      const unsigned long long key = nbr_key(d, orig_index(p));
       if (key >= worst) continue;
       if (cnt < k) {
         sk[cnt * T] = key;
@@ -95,13 +100,13 @@ __device__ inline int knn_query(const GridView &g, float qx, float qy, float qz,
   auto row_far = [&](int y, int z, float gx) -> bool {
     if (cnt < k) return false;
     const float gy = gap(y, cy, qy, g.loy), gz = gap(z, cz, qz, g.loz);
-    return (gx * gx + gy * gy + gz * gz) * 0.99999f > knn_d2(worst);
+    return (gx * gx + gy * gy + gz * gz) * 0.99999f > key_d2(worst);
   };
   // a row's run of cells xa..xb (it spans the query's column): the end cells are dropped while they are too far
   auto scan_row = [&](int y, int z, int row, int xa, int xb) {
     if (cnt == k) {
       const float gy = gap(y, cy, qy, g.loy), gz = gap(z, cz, qz, g.loz);
-      const float yz = gy * gy + gz * gz, w = knn_d2(worst);
+      const float yz = gy * gy + gz * gz, w = key_d2(worst);
       if (yz * 0.99999f > w) return;
       while (xa < cx) {
         const float gx = gap(xa, cx, qx, g.lox);
@@ -170,7 +175,7 @@ __device__ inline int knn_query(const GridView &g, float qx, float qy, float qz,
       if (cz - R > 0) cert = fminf(cert, qz - (g.loz + (float)(cz - R) * g.h));
       if (cz + R < g.dz - 1) cert = fminf(cert, (g.loz + (float)(cz + R + 1) * g.h) - qz);
       cert -= margin;
-      if (cert > 0.f && knn_d2(worst) < cert * cert * 0.99999f) break;
+      if (cert > 0.f && key_d2(worst) < cert * cert * 0.99999f) break;
     }
   }
   // ascending (distance, index) order: FLANN's result order
@@ -226,11 +231,18 @@ __device__ __forceinline__ bool ball_cell_range(const GridView &g, float qx, flo
   return true;
 }
 
-__device__ __forceinline__ unsigned long long nbr_key(float d2, int orig) {
-  return ((unsigned long long)__float_as_uint(d2) << 32) | (unsigned)orig;
+// List storage of a one-query-per-CTA kernel: `cap` keys, then `cap` positions, in the dynamic shared memory smem; or,
+// when glob_key is set (lists too long for shared memory), this CTA's slices of the global scratch glob_key / glob_pos.
+__device__ __forceinline__ void cta_list(unsigned char *smem, unsigned long long *glob_key, int *glob_pos, int cap,
+                                         unsigned long long *&key, int *&pos) {
+  if (glob_key) {
+    key = glob_key + (size_t)blockIdx.x * cap;
+    pos = glob_pos + (size_t)blockIdx.x * cap;
+  } else {
+    key = reinterpret_cast<unsigned long long *>(smem);
+    pos = reinterpret_cast<int *>(smem + (size_t)cap * sizeof(unsigned long long));
+  }
 }
-__device__ __forceinline__ float key_d2(unsigned long long k) { return __uint_as_float((unsigned)(k >> 32)); }
-__device__ __forceinline__ int key_orig(unsigned long long k) { return (int)(unsigned)(k & 0xffffffffull); }
 
 // CTA-cooperative radius gather.  Every thread of the block must call it.  key/pos: list storage
 // with room for `cap` entries (shared or global).  Returns the total number of neighbours; only the
@@ -327,6 +339,86 @@ __device__ inline void bitonic_sort(unsigned long long *key, int *pos, int n) {
         }
       }
       __syncthreads();
+    }
+}
+
+// One-warp radius gather: the neighbours of c (the count pass's guard and test, so their number is what
+// count_radius_warp returned) are appended to the warp's list in scan order — cell rows z-major, then y, each row's
+// points in cell order — as keys and / or positions in g.pts; key or pos may be nullptr.  Returns min(count, CAP);
+// only the first CAP are stored.  Every lane of the warp must call it.  BOARD's warp kernel adds its float64 sums in
+// this order: changing the order changes its frames.  (A nullptr argument is told apart by its type, so the compiler
+// drops the store; a run-time test of a pointer into shared memory is not folded away.)
+template <int CAP, class KeyPtr, class PosPtr>
+__device__ __forceinline__ int warp_gather_radius(const GridView &g, const float4 c, float radius, float r2, KeyPtr key,
+                                                  PosPtr pos, int lane) {
+  int n = 0;
+  int x0, x1, y0, y1, z0, z1;
+  if (finite3(c.x, c.y, c.z) && g.n > 0 && ball_cell_range(g, c.x, c.y, c.z, radius, x0, x1, y0, y1, z0, z1)) {
+    const float4 *__restrict__ pts = g.pts;
+    const int *__restrict__ cs = g.cell_start;
+    for (int z = z0; z <= z1; ++z)
+      for (int y = y0; y <= y1; ++y) {
+        const int base = g.dx * (y + g.dy * z);
+        const int s0 = cs[base + x0], e = cs[base + x1 + 1];
+        // four 32-point chunks per trip, their loads issued before the first ballot (a trip per chunk made every
+        // chunk wait for its own L2 round trip: SHOT's largest stall)
+        for (int j0 = s0; j0 < e; j0 += 128) {
+          float4 p[4];
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            const int j = j0 + 32 * u + lane;
+            p[u] = (j < e) ? pts[j] : make_float4(0.f, 0.f, 0.f, 0.f);
+          }
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            const int j = j0 + 32 * u + lane;
+            const float d2 = sqdist3(c.x, c.y, c.z, p[u].x, p[u].y, p[u].z);
+            const bool hit = j < e && d2 < r2;
+            const unsigned m = __ballot_sync(0xffffffffu, hit);
+            if (hit) {
+              const int slot = n + __popc(m & ((1u << lane) - 1u));
+              if (slot < CAP) {
+                if constexpr (!std::is_null_pointer_v<KeyPtr>) key[slot] = nbr_key(d2, orig_index(p[u]));
+                if constexpr (!std::is_null_pointer_v<PosPtr>) pos[slot] = j;
+              }
+            }
+            n += __popc(m);
+          }
+        }
+      }
+  }
+  return min(n, CAP);
+}
+
+// One-warp bitonic sort of n (key, pos) pairs, ascending key, synchronised by __syncwarp only; pos may be nullptr.
+// The arrays must have room for the next power of two >= max(n, 32).  Every lane of the warp must call it.
+template <class PosPtr>
+__device__ __forceinline__ void warp_bitonic_sort(unsigned long long *key, PosPtr pos, int n, int lane) {
+  int np = 32;
+  while (np < n) np <<= 1;
+  for (int t = n + lane; t < np; t += 32) {
+    key[t] = ~0ull;
+    if constexpr (!std::is_null_pointer_v<PosPtr>) pos[t] = -1;
+  }
+  __syncwarp();
+  for (int k = 2; k <= np; k <<= 1)
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      for (int t = lane; t < (np >> 1); t += 32) {
+        const int a = ((t & ~(j - 1)) << 1) | (t & (j - 1));
+        const int b = a | j;
+        const bool up = ((a & k) == 0);
+        const unsigned long long ka = key[a], kb = key[b];
+        if ((ka > kb) == up) {
+          key[a] = kb;
+          key[b] = ka;
+          if constexpr (!std::is_null_pointer_v<PosPtr>) {
+            const int pa = pos[a];
+            pos[a] = pos[b];
+            pos[b] = pa;
+          }
+        }
+      }
+      __syncwarp();
     }
 }
 

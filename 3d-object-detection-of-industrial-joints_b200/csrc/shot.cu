@@ -199,13 +199,7 @@ __global__ void __launch_bounds__(SHOT_THREADS)
 
   unsigned long long *key;
   int *pos;
-  if (glob_key) {
-    key = glob_key + (size_t)blockIdx.x * cap;
-    pos = glob_pos + (size_t)blockIdx.x * cap;
-  } else {
-    key = reinterpret_cast<unsigned long long *>(smem_raw);
-    pos = reinterpret_cast<int *>(smem_raw + (size_t)cap * sizeof(unsigned long long));
-  }
+  cta_list(smem_raw, glob_key, glob_pos, cap, key, pos);
   const int tid = threadIdx.x;
   const float4 *__restrict__ pts = g.pts;
 
@@ -494,7 +488,6 @@ __global__ void __launch_bounds__(SW_THREADS, 3)
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   ShotWarpSmem &sm = reinterpret_cast<ShotWarpSmem *>(smem_raw)[warp];
   const float4 *__restrict__ pts = g.pts;
-  const int *__restrict__ cs = g.cell_start;
 
   const double radius3_4 = (radius * 3) / 4, radius1_4 = radius / 4, radius1_2 = radius / 2;
   const float r12f = (float)radius1_2, r34f = (float)radius3_4, r14f = (float)radius1_4;
@@ -513,40 +506,7 @@ __global__ void __launch_bounds__(SW_THREADS, 3)
     if (counts[i] > SW_CAP) continue;  // left to shot_kernel
     const float4 c = kp[i];
 
-    // ---- gather: neighbours with d2 < r2, appended in scan order ----
-    int n = 0;
-    {
-      int x0, x1, y0, y1, z0, z1;
-      if (finite3(c.x, c.y, c.z) && g.n > 0 && ball_cell_range(g, c.x, c.y, c.z, radius_f, x0, x1, y0, y1, z0, z1)) {
-        for (int z = z0; z <= z1; ++z)
-          for (int y = y0; y <= y1; ++y) {
-            const int base = g.dx * (y + g.dy * z);
-            const int s0 = cs[base + x0], e = cs[base + x1 + 1];
-            // four 32-point chunks per trip, their loads issued before the first ballot (a trip per chunk made every
-            // chunk wait for its own L2 round trip: the kernel's largest stall)
-            for (int j0 = s0; j0 < e; j0 += 128) {
-              float4 p[4];
-#pragma unroll
-              for (int u = 0; u < 4; ++u) {
-                const int j = j0 + 32 * u + lane;
-                p[u] = (j < e) ? pts[j] : make_float4(0.f, 0.f, 0.f, 0.f);
-              }
-#pragma unroll
-              for (int u = 0; u < 4; ++u) {
-                const int j = j0 + 32 * u + lane;
-                const bool hit = j < e && sqdist3(c.x, c.y, c.z, p[u].x, p[u].y, p[u].z) < r2;
-                const unsigned m = __ballot_sync(0xffffffffu, hit);
-                if (hit) {
-                  const int slot = n + __popc(m & ((1u << lane) - 1u));
-                  if (slot < SW_CAP) sm.pos[slot] = j;
-                }
-                n += __popc(m);
-              }
-            }
-          }
-      }
-    }
-    if (n > SW_CAP) n = SW_CAP;  // cannot happen: counts[i] is the same count
+    const int n = warp_gather_radius<SW_CAP>(g, c, radius_f, r2, nullptr, sm.pos, lane);
     for (int b = lane; b < SHOT_LEN; b += 32) sm.hist[b] = 0;
     __syncwarp();
 
