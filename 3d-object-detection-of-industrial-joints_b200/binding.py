@@ -283,6 +283,16 @@ def _dptr(t):
     return C.c_void_p(t.data_ptr())
 
 
+def _scene_outputs(mi, Ks, zero_offsets=False):
+    """Host output arrays of a scene registration: transforms, instance offsets, instance and scene correspondences
+    (filled by the library: no zero-fill on the caller's clock)."""
+    T = np.empty((mi, 16), dtype=np.float32)
+    off = (np.zeros if zero_offsets else np.empty)(mi + 1, dtype=np.int32)
+    ic = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
+    corrs = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
+    return T, off, ic, corrs
+
+
 class InstanceList:
     """Per-instance correspondence lists as views into the flat output buffer (pcl's
     std::vector<pcl::Correspondences>): nothing is copied or sliced until an item is asked for."""
@@ -565,6 +575,14 @@ class Context:
     def _chk(self, rc):
         if rc != OK:
             raise B200Error(rc, lib().b200_last_error(self.h).decode())
+
+    def _scene_result(self, rc, T, off, ic, corrs, mi, n_inst, n_corr):
+        """Result dict of a scene registration into _scene_outputs' arrays; ERR_CAPACITY (truncated output) returns."""
+        if rc not in (OK, ERR_CAPACITY):
+            self._chk(rc)
+        m = min(n_inst, mi)
+        return {"transforms": T[:m].reshape(m, 4, 4), "instances": InstanceList(ic, off, m), "n_instances": n_inst,
+                "corrs": corrs[:n_corr]}
 
     def close(self):
         if self.h:
@@ -851,25 +869,20 @@ class Context:
     def register_scene_shot(self, model, scene_xyz, scene_kp, params):
         """Host buffers in, host results out (b200_register_scene_shot)."""
         scene_xyz, scene_kp = _pts(scene_xyz), _pts(scene_kp)
-        mi = params.max_instances
-        Ks = len(scene_kp)
-        T = np.empty((mi, 16), dtype=np.float32)       # filled by the library (no zero-fill on the caller's clock)
-        off = np.empty(mi + 1, dtype=np.int32)
-        ic = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
-        corrs = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
+        mi, Ks = params.max_instances, len(scene_kp)
+        T, off, ic, corrs = _scene_outputs(mi, Ks)
         n_inst, n_corr = C.c_int(), C.c_int()
         rc = lib().b200_register_scene_shot(self.h, model.h, _f(scene_xyz), len(scene_xyz), scene_xyz.shape[1],
                                             _f(scene_kp), Ks, scene_kp.shape[1], C.byref(params), _f(T), _i(off),
                                             _c(ic), max(Ks, 1), C.byref(n_inst), _c(corrs), C.byref(n_corr))
-        if rc not in (OK, ERR_CAPACITY):
-            self._chk(rc)
-        m = min(n_inst.value, mi)
+        out = self._scene_result(rc, T, off, ic, corrs, mi, n_inst.value, n_corr.value)
         if rc == ERR_CAPACITY:
             import warnings
             warnings.warn("b200_register_scene_shot: output capacity exceeded (%d instances found, %d kept): %s"
-                          % (n_inst.value, m, lib().b200_last_error(self.h).decode()), RuntimeWarning, stacklevel=2)
-        return {"transforms": T[:m].reshape(m, 4, 4), "instances": InstanceList(ic, off, m),
-                "n_instances": n_inst.value, "corrs": corrs[:n_corr.value], "truncated": rc == ERR_CAPACITY}
+                          % (n_inst.value, len(out["instances"]), lib().b200_last_error(self.h).decode()),
+                          RuntimeWarning, stacklevel=2)
+        out["truncated"] = rc == ERR_CAPACITY
+        return out
 
     # ---- resident Hough branch (BOARD frames + Hough3DGrouping) ------------------------------------
     def model_create_shot_hough(self, xyz, kp, params, hough):
@@ -887,21 +900,15 @@ class Context:
         the Hough space would exceed 2^27 bins)."""
         scene_xyz, scene_kp = _pts(scene_xyz), _pts(scene_kp)
         mi, Ks = params.max_instances, len(scene_kp)
-        T = np.empty((mi, 16), dtype=np.float32)
-        off = np.zeros(mi + 1, dtype=np.int32)
-        ic = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
-        corrs = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
+        T, off, ic, corrs = _scene_outputs(mi, Ks, zero_offsets=True)
         rf = np.empty((max(Ks, 1), 9), dtype=np.float32)
         n_inst, n_corr = C.c_int(), C.c_int()
         rc = lib().b200_register_scene_shot_hough(self.h, model.h, _f(scene_xyz), len(scene_xyz), scene_xyz.shape[1],
                                                   _f(scene_kp), Ks, scene_kp.shape[1], C.byref(params), C.byref(hough),
                                                   _f(T), _i(off), _c(ic), max(Ks, 1), C.byref(n_inst), _c(corrs),
                                                   C.byref(n_corr), _f(rf))
-        if rc not in (OK, ERR_CAPACITY):
-            self._chk(rc)
-        m = min(n_inst.value, mi)
-        return {"transforms": T[:m].reshape(m, 4, 4), "instances": InstanceList(ic, off, m),
-                "n_instances": n_inst.value, "corrs": corrs[:n_corr.value], "rf": rf[:Ks], "status": rc}
+        out = self._scene_result(rc, T, off, ic, corrs, mi, n_inst.value, n_corr.value)
+        return dict(out, rf=rf[:Ks], status=rc)
 
     def dev_register_scene_shot_hough(self, model, d_xyz, n, stride, d_kp, Ks, kstride, params, hough, out):
         """All buffers resident (torch CUDA tensors in `out`, as dev_register_scene_shot, plus the device int
@@ -922,20 +929,14 @@ class Context:
     def register_scene_fpfh(self, model, scene_kp, params, want_desc=False):
         scene_kp = _pts(scene_kp)
         mi, Ks = params.max_instances, len(scene_kp)
-        T = np.empty((mi, 16), dtype=np.float32)
-        off = np.empty(mi + 1, dtype=np.int32)
-        ic = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
-        corrs = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
+        T, off, ic, corrs = _scene_outputs(mi, Ks)
         desc = np.empty((max(Ks, 1), 33), dtype=np.float32) if want_desc else None
         n_inst, n_corr = C.c_int(), C.c_int()
         rc = lib().b200_register_scene_fpfh(self.h, model.h, _f(scene_kp), Ks, scene_kp.shape[1], C.byref(params), _f(T),
                                             _i(off), _c(ic), max(Ks, 1), C.byref(n_inst), _c(corrs), C.byref(n_corr),
                                             _f(desc) if want_desc else None)
-        if rc not in (OK, ERR_CAPACITY):
-            self._chk(rc)
-        m = min(n_inst.value, mi)
-        out = {"transforms": T[:m].reshape(m, 4, 4), "instances": InstanceList(ic, off, m),
-               "n_instances": n_inst.value, "corrs": corrs[:n_corr.value], "truncated": rc == ERR_CAPACITY}
+        out = self._scene_result(rc, T, off, ic, corrs, mi, n_inst.value, n_corr.value)
+        out["truncated"] = rc == ERR_CAPACITY
         if want_desc:
             out["desc"] = desc[:Ks]
         return out
@@ -967,20 +968,14 @@ class Context:
             return None
         scene_xyz, scene_kp = _pts(scene_xyz), _pts(scene_kp)
         mi, Ks = params.max_instances, len(scene_kp)
-        T = np.empty((mi, 16), dtype=np.float32)
-        off = np.empty(mi + 1, dtype=np.int32)
-        ic = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
-        corrs = np.empty(max(Ks, 1), dtype=CORR_DTYPE)
+        T, off, ic, corrs = _scene_outputs(mi, Ks)
         n_inst, n_corr = C.c_int(), C.c_int()
         rc = lib().b200_register_scene_shot_sharded(
             self.h, model.h, int(root), _f(scene_xyz), len(scene_xyz), scene_xyz.shape[1], _f(scene_kp), Ks,
             scene_kp.shape[1], C.byref(params), _f(T), _i(off), _c(ic), max(Ks, 1), C.byref(n_inst), _c(corrs),
             C.byref(n_corr))
-        if rc not in (OK, ERR_CAPACITY):
-            self._chk(rc)
-        m = min(n_inst.value, mi)
-        return {"transforms": T[:m].reshape(m, 4, 4), "instances": InstanceList(ic, off, m),
-                "n_instances": n_inst.value, "corrs": corrs[:n_corr.value], "truncated": rc == ERR_CAPACITY}
+        out = self._scene_result(rc, T, off, ic, corrs, mi, n_inst.value, n_corr.value)
+        return dict(out, truncated=rc == ERR_CAPACITY)
 
     def dev_register_scene_shot(self, model, d_xyz, n, stride, d_kp, Ks, kstride, params, out):
         """All buffers resident (torch CUDA tensors in `out`), asynchronous (b200_dev_register_scene_shot)."""

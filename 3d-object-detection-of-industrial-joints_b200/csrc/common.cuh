@@ -11,6 +11,7 @@
 #include <array>
 #include <mutex>
 #include <map>
+#include <memory>
 #include <utility>
 #include <vector>
 #include <cstdio>
@@ -459,7 +460,7 @@ int write_small(b200_ctx *ctx, void *d_dst, const void *h_src, size_t bytes);
 // scan.cu
 int exclusive_scan_i32(b200_ctx *ctx, const int *d_in, int *d_out, int n, int *d_total /*nullable*/);
 // grid.cu
-int cloud_upload(b200_ctx *ctx, const float *xyz, int n, int stride, bool on_device, b200_cloud **out);
+int cloud_upload(b200_ctx *ctx, const float *xyz, int n, int stride, bool on_device, std::unique_ptr<b200_cloud> &out);
 int cloud_grid_for_knn(b200_cloud *c, int k, const GridView **out);
 int cloud_grid_for_radius(b200_cloud *c, double radius, const GridView **out);
 int pack_points(b200_ctx *ctx, const float *d_xyz, int n, int stride, float4 *d_out);
@@ -488,17 +489,35 @@ int match_prepare_model(b200_ctx *ctx, b200_model *m);  // no-op for small libra
 int match_prepare_rows(b200_ctx *ctx, const float *d_desc, int K, int D, TcModelPrep *t);
 int dev_nearest1(b200_ctx *ctx, const float *d_model, int Km, const unsigned char *mvalid_p, const TcModelPrep *prep,
                  const float *d_q, int nq, int D, int *d_idx, float *d_d2);
+
+// Device result of one grouping run (dev_gc, dev_hough3d): per instance its 4x4 pose (T, max_inst x 16), the start of
+// its correspondences (offsets, max_inst + 1) and how many RANSAC kept (counts, max_inst); the kept correspondences
+// (corrs, corr_cap entries) and the number of instances found (*n, which may exceed max_inst).
+struct InstanceOut {
+  float *T;
+  int max_inst;
+  int *offsets;
+  int *counts;
+  b200_corr *corrs;
+  int corr_cap;
+  int *n;
+  // the zero count, offsets and counts every grouping run starts from
+  int clear(b200_ctx *ctx) const {
+    B200_CUDA(ctx, cudaMemsetAsync(n, 0, sizeof(int), ctx->stream));
+    B200_CUDA(ctx, cudaMemsetAsync(offsets, 0, sizeof(int) * ((size_t)max_inst + 1), ctx->stream));
+    B200_CUDA(ctx, cudaMemsetAsync(counts, 0, sizeof(int) * (size_t)max_inst, ctx->stream));
+    return B200_OK;
+  }
+};
+
 int dev_ransac_instances(b200_ctx *ctx, const b200_corr *d_corrs, const float4 *d_mp, const float4 *d_sp,
-                         const int *d_members, const int *d_inst_offsets, const int *d_n_inst, int C_cap,
-                         double threshold, float *d_T, int max_inst, int *d_inst_counts, b200_corr *d_inst_corrs,
-                         int corr_cap);
+                         const int *d_members, int C_cap, double threshold, const InstanceOut &out);
 // hough.cu
 int dev_hough_model_votes(b200_ctx *ctx, const float4 *d_model_kp, const float *d_model_rf, int Km, float *d_votes);
 // correspondence count: *d_C (at most C_cap); *d_status = B200_ERR_CAPACITY when the space has more than 2^27 bins
 int dev_hough3d(b200_ctx *ctx, const float4 *d_model_kp, const float *d_model_votes, const float4 *d_scene_kp,
                 const float *d_scene_rf, const b200_corr *d_corrs, const int *d_C, int C_cap, double bin_size,
-                double threshold, float *d_T, int max_inst, int *d_inst_offsets, int *d_inst_counts,
-                b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst, int *d_status);
+                double threshold, const InstanceOut &out, int *d_status);
 // board.cu
 void board_rand_seed(b200_ctx *ctx, unsigned seed);
 int dev_board_lrf_from(b200_ctx *ctx, b200_cloud *c, const float *d_normals, const float4 *d_kp, int K, double radius,
@@ -529,5 +548,4 @@ int dev_concat_lists(b200_ctx *ctx, const b200_corr *d_gathered, const int *d_co
 int dev_offset_scene_index(b200_ctx *ctx, b200_corr *d_corrs, const int *d_n, int cap, int offset);
 // gc.cu
 int dev_gc(b200_ctx *ctx, const float4 *d_model_kp, const float4 *d_scene_kp, const b200_corr *d_corrs,
-           const int *d_C, int C_cap, double gc_size, int gc_threshold, float *d_T, int max_inst,
-           int *d_inst_offsets, int *d_inst_counts, b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst);
+           const int *d_C, int C_cap, double gc_size, int gc_threshold, const InstanceOut &out);

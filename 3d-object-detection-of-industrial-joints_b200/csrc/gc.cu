@@ -1173,12 +1173,9 @@ __global__ void __launch_bounds__(RS_THREADS, (RS_THREADS == 32) ? 20 : 5)
 }  // namespace
 
 int dev_gc(b200_ctx *ctx, const float4 *d_model_kp, const float4 *d_scene_kp, const b200_corr *d_corrs,
-           const int *d_C, int C_cap, double gc_size, int gc_threshold, float *d_T, int max_inst, int *d_inst_offsets,
-           int *d_inst_counts, b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst) {
-  if (max_inst < 1) return ctx->fail(B200_ERR_INVALID, "gc: max_inst must be >= 1");
-  B200_CUDA(ctx, cudaMemsetAsync(d_n_inst, 0, sizeof(int), ctx->stream));
-  B200_CUDA(ctx, cudaMemsetAsync(d_inst_offsets, 0, sizeof(int) * ((size_t)max_inst + 1), ctx->stream));
-  B200_CUDA(ctx, cudaMemsetAsync(d_inst_counts, 0, sizeof(int) * (size_t)max_inst, ctx->stream));
+           const int *d_C, int C_cap, double gc_size, int gc_threshold, const InstanceOut &out) {
+  if (out.max_inst < 1) return ctx->fail(B200_ERR_INVALID, "gc: max_inst must be >= 1");
+  B200_TRY(out.clear(ctx));
   if (C_cap <= 0) return B200_OK;
   // The consistency bitmap is C x C bits.  Up to GC_ASYNC_CAP correspondences it is sized for the
   // capacity and the whole stage stays asynchronous; above that the actual count is read back first, so that the
@@ -1245,8 +1242,8 @@ int dev_gc(b200_ctx *ctx, const float4 *d_model_kp, const float4 *d_scene_kp, co
   ga.sp = sp.p;
   ga.overflow = overflow.p;
   ga.members = members.p;
-  ga.inst_offsets = d_inst_offsets;
-  ga.n_inst_out = d_n_inst;
+  ga.inst_offsets = out.offsets;
+  ga.n_inst_out = out.n;
   DevBuf<long long> dbg;
   const bool debug = getenv("B200_GC_DEBUG") != nullptr;
   ga.dbg = nullptr;
@@ -1265,7 +1262,7 @@ int dev_gc(b200_ctx *ctx, const float4 *d_model_kp, const float4 *d_scene_kp, co
     const size_t smem = 2 * (size_t)row_words_cap * sizeof(unsigned);
     B200_CUDA(ctx, ensure_dyn_smem(gc_group_cluster_kernel, smem));
     gc_group_cluster_kernel<<<GCL, GCL_THREADS, smem, ctx->stream>>>(ga, d_C, C_eff, gc_size, g_lo, g_hi, gc_threshold,
-                                                                    max_inst);
+                                                                    out.max_inst);
     B200_LAUNCHED(ctx);
   }
   if (debug) {
@@ -1277,17 +1274,14 @@ int dev_gc(b200_ctx *ctx, const float4 *d_model_kp, const float4 *d_scene_kp, co
               w, h[w * 8], h[w * 8 + 1], h[w * 8 + 2], h[w * 8 + 3], h[w * 8 + 4], h[w * 8 + 5], h[w * 8 + 6], h[w * 8 + 7]);
   }
 
-  return dev_ransac_instances(ctx, sorted.p, mp.p, sp.p, members.p, d_inst_offsets, d_n_inst, C_eff, gc_size, d_T, max_inst,
-                              d_inst_counts, d_inst_corrs, corr_cap);
+  return dev_ransac_instances(ctx, sorted.p, mp.p, sp.p, members.p, C_eff, gc_size, out);
 }
 
 // RANSAC pose + correspondence filtering for a set of instances (shared by geometric-consistency and
 // Hough grouping).  corrs: the correspondence records the member indices refer to; mp / sp: model and
 // scene keypoint of every correspondence; members: concatenated member lists, inst_offsets[i]..[i+1].
 int dev_ransac_instances(b200_ctx *ctx, const b200_corr *d_corrs, const float4 *d_mp, const float4 *d_sp,
-                         const int *d_members, const int *d_inst_offsets, const int *d_n_inst, int C_cap,
-                         double threshold, float *d_T, int max_inst, int *d_inst_counts, b200_corr *d_inst_corrs,
-                         int corr_cap) {
+                         const int *d_members, int C_cap, double threshold, const InstanceOut &out) {
   DevBuf<int> shuffled, last_pos, flags;
   if (!ctx->mt_state) {
     unsigned host_state[624];
@@ -1304,19 +1298,19 @@ int dev_ransac_instances(b200_ctx *ctx, const b200_corr *d_corrs, const float4 *
   rb.mp = d_mp;
   rb.sp = d_sp;
   rb.members = d_members;
-  rb.inst_offsets = d_inst_offsets;
-  rb.n_inst = d_n_inst;
+  rb.inst_offsets = out.offsets;
+  rb.n_inst = out.n;
   rb.mt_init = ctx->mt_state;
   rb.shuffled = shuffled.p;
   rb.last_pos = last_pos.p;
   rb.flags = flags.p;
-  rb.T_out = d_T;
-  rb.inst_counts = d_inst_counts;
-  rb.inst_corrs = d_inst_corrs;
+  rb.T_out = out.T;
+  rb.inst_counts = out.counts;
+  rb.inst_corrs = out.corrs;
   StageScope st_(ctx, ST_GC_RANSAC);
-  gc_ransac_kernel<32><<<max_inst, 32, 0, ctx->stream>>>(rb, max_inst, corr_cap, threshold, 10000);
+  gc_ransac_kernel<32><<<out.max_inst, 32, 0, ctx->stream>>>(rb, out.max_inst, out.corr_cap, threshold, 10000);
   B200_LAUNCHED(ctx);
-  gc_ransac_kernel<128><<<max_inst, 128, 0, ctx->stream>>>(rb, max_inst, corr_cap, threshold, 10000);
+  gc_ransac_kernel<128><<<out.max_inst, 128, 0, ctx->stream>>>(rb, out.max_inst, out.corr_cap, threshold, 10000);
   B200_LAUNCHED(ctx);
   return B200_OK;
 }

@@ -211,46 +211,36 @@ int pack_points(b200_ctx *ctx, const float *d_xyz, int n, int stride, float4 *d_
   return B200_OK;
 }
 
-int cloud_upload(b200_ctx *ctx, const float *xyz, int n, int stride, bool on_device, b200_cloud **out) {
-  if (!out || n < 0 || stride < 3 || (n > 0 && !xyz)) return ctx->fail(B200_ERR_INVALID, "cloud_create: bad arguments");
-  b200_cloud *c = new b200_cloud();
+int cloud_upload(b200_ctx *ctx, const float *xyz, int n, int stride, bool on_device, std::unique_ptr<b200_cloud> &out) {
+  if (n < 0 || stride < 3 || (n > 0 && !xyz)) return ctx->fail(B200_ERR_INVALID, "cloud_create: bad arguments");
+  std::unique_ptr<b200_cloud> c(new (std::nothrow) b200_cloud());
+  if (!c) return ctx->fail(B200_ERR_NOMEM, "cloud_create: out of host memory");
   c->ctx = ctx;
   c->n = n;
-  int rc = c->raw.alloc(ctx, (size_t)std::max(n, 1));
-  if (rc != B200_OK) {
-    delete c;
-    return rc;
-  }
-  auto bail = [&](int code) {
-    delete c;
-    return code;
-  };
+  B200_TRY(c->raw.alloc(ctx, (size_t)std::max(n, 1)));
   if (n > 0) {
     if (on_device) {
-      if ((rc = pack_points(ctx, xyz, n, stride, c->raw.p)) != B200_OK) return bail(rc);
+      B200_TRY(pack_points(ctx, xyz, n, stride, c->raw.p));
     } else {
       DevBuf<float> stage;
-      if ((rc = stage.alloc(ctx, (size_t)n * stride)) != B200_OK) return bail(rc);
-      cudaError_t e = cudaMemcpyAsync(stage.p, xyz, (size_t)n * stride * sizeof(float), cudaMemcpyHostToDevice,
-                                      ctx->stream);
-      if (e != cudaSuccess) return bail(ctx->fail_cuda(e, "H2D points", __FILE__, __LINE__));
-      if ((rc = pack_points(ctx, stage.p, n, stride, c->raw.p)) != B200_OK) return bail(rc);
+      B200_TRY(stage.alloc(ctx, (size_t)n * stride));
+      B200_CUDA(ctx, cudaMemcpyAsync(stage.p, xyz, (size_t)n * stride * sizeof(float), cudaMemcpyHostToDevice,
+                                     ctx->stream));
+      B200_TRY(pack_points(ctx, stage.p, n, stride, c->raw.p));
     }
   }
   // bounding box + finite count (one 28-byte readback; the grid dimensions are sized on the host)
   DevBuf<unsigned> box;
-  if ((rc = box.alloc(ctx, 8)) != B200_OK) return bail(rc);
+  B200_TRY(box.alloc(ctx, 8));
   unsigned init[8] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u, 0u, 0u};
-  if ((rc = write_small(ctx, box.p, init, sizeof(init))) != B200_OK) return bail(rc);
+  B200_TRY(write_small(ctx, box.p, init, sizeof(init)));
   if (n > 0) {
     int blocks = std::min(ceil_div(n, 256), ctx->sm_count * 4);
     bbox_kernel<<<blocks, 256, 0, ctx->stream>>>(c->raw.p, n, box.p, reinterpret_cast<int *>(box.p + 6));
-    ctx->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return bail(ctx->fail_cuda(e, "bbox_kernel", __FILE__, __LINE__));
+    B200_LAUNCHED(ctx);
   }
   unsigned hbox[8];
-  if ((rc = readback_small(ctx, box.p, hbox, sizeof(hbox))) != B200_OK) return bail(rc);
+  B200_TRY(readback_small(ctx, box.p, hbox, sizeof(hbox)));
   c->n_valid = (int)hbox[6];
   if (c->n_valid > 0) {
     for (int a = 0; a < 3; ++a) {
@@ -260,7 +250,7 @@ int cloud_upload(b200_ctx *ctx, const float *xyz, int n, int stride, bool on_dev
   } else {
     for (int a = 0; a < 3; ++a) c->lo[a] = c->hi[a] = 0.f;
   }
-  *out = c;
+  out = std::move(c);
   return B200_OK;
 }
 

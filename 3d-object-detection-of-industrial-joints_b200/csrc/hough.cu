@@ -295,14 +295,11 @@ int dev_hough_model_votes(b200_ctx *ctx, const float4 *d_model_kp, const float *
 
 int dev_hough3d(b200_ctx *ctx, const float4 *d_model_kp, const float *d_model_votes, const float4 *d_scene_kp,
                 const float *d_scene_rf, const b200_corr *d_corrs, const int *d_C, int C_cap, double bin_size,
-                double threshold, float *d_T, int max_inst, int *d_inst_offsets, int *d_inst_counts,
-                b200_corr *d_inst_corrs, int corr_cap, int *d_n_inst, int *d_status) {
-  if (max_inst < 1) return ctx->fail(B200_ERR_INVALID, "hough3d: max_inst must be >= 1");
+                double threshold, const InstanceOut &out, int *d_status) {
+  if (out.max_inst < 1) return ctx->fail(B200_ERR_INVALID, "hough3d: max_inst must be >= 1");
   if (!(bin_size > 0.0)) return ctx->fail(B200_ERR_INVALID, "hough3d: bin size must be > 0");
   B200_CUDA(ctx, cudaMemsetAsync(d_status, 0, sizeof(int), ctx->stream));
-  B200_CUDA(ctx, cudaMemsetAsync(d_n_inst, 0, sizeof(int), ctx->stream));
-  B200_CUDA(ctx, cudaMemsetAsync(d_inst_offsets, 0, sizeof(int) * ((size_t)max_inst + 1), ctx->stream));
-  B200_CUDA(ctx, cudaMemsetAsync(d_inst_counts, 0, sizeof(int) * (size_t)max_inst, ctx->stream));
+  B200_TRY(out.clear(ctx));
   if (C_cap <= 0) return B200_OK;
   const int n = C_cap, nb = ceil_div(n, 256);
   DevBuf<int> members;
@@ -370,9 +367,10 @@ int dev_hough3d(b200_ctx *ctx, const float4 *d_model_kp, const float *d_model_vo
     B200_LAUNCHED(ctx);
     hough_flags_kernel<<<nb, 256, 0, ctx->stream>>>(votes.p, n, threshold, vmax.p, flags.p, sizes.p);
     B200_LAUNCHED(ctx);
-    B200_TRY(exclusive_scan_i32(ctx, flags.p, slots.p, n, d_n_inst));
+    B200_TRY(exclusive_scan_i32(ctx, flags.p, slots.p, n, out.n));
     B200_TRY(exclusive_scan_i32(ctx, sizes.p, starts.p, n, nullptr));
-    hough_offsets_kernel<<<nb, 256, 0, ctx->stream>>>(flags.p, slots.p, starts.p, sizes.p, n, max_inst, d_inst_offsets);
+    hough_offsets_kernel<<<nb, 256, 0, ctx->stream>>>(flags.p, slots.p, starts.p, sizes.p, n, out.max_inst,
+                                                      out.offsets);
     B200_LAUNCHED(ctx);
     hough_members_kernel<<<nb, 256, 0, ctx->stream>>>(vin, head.p, run_id.p, run_start.p, flags.p, starts.p, n,
                                                       members.p);
@@ -382,6 +380,5 @@ int dev_hough3d(b200_ctx *ctx, const float4 *d_model_kp, const float *d_model_vo
   }
   // what follows is RANSAC, one small CTA per instance: the next scene's wide stages may start beside it
   if (ctx->wide) ctx->wide->leave();
-  return dev_ransac_instances(ctx, d_corrs, mp.p, sp.p, members.p, d_inst_offsets, d_n_inst, n, bin_size, d_T, max_inst,
-                              d_inst_counts, d_inst_corrs, corr_cap);
+  return dev_ransac_instances(ctx, d_corrs, mp.p, sp.p, members.p, n, bin_size, out);
 }

@@ -722,11 +722,6 @@ int check_hv_params(b200_ctx *ctx, const b200_hv_params &P) {
   return B200_OK;
 }
 
-struct CloudHolder {  // b200_cloud with scope lifetime
-  b200_cloud *c = nullptr;
-  ~CloudHolder() { delete c; }
-};
-
 // radius normals of a device cloud (xyz rows, n x 3) on itself, rows with a NaN normal dropped:
 // out_pts / out_nrm hold *n_out compacted rows
 int normals_and_compact(b200_ctx *ctx, const float *d_xyz, int n, double radius, DevBuf<float4> &out_pts,
@@ -735,15 +730,15 @@ int normals_and_compact(b200_ctx *ctx, const float *d_xyz, int n, double radius,
   B200_TRY(out_pts.alloc(ctx, (size_t)std::max(n, 1)));
   B200_TRY(out_nrm.alloc(ctx, (size_t)std::max(n, 1)));
   if (n <= 0) return B200_OK;
-  CloudHolder ch;
-  B200_TRY(cloud_upload(ctx, d_xyz, n, 3, true, &ch.c));
+  std::unique_ptr<b200_cloud> cloud;
+  B200_TRY(cloud_upload(ctx, d_xyz, n, 3, true, cloud));
   DevBuf<float> nrm;
   DevBuf<int> flags, slots, total;
   B200_TRY(nrm.alloc(ctx, (size_t)n * 4));
   B200_TRY(flags.alloc(ctx, (size_t)n));
   B200_TRY(slots.alloc(ctx, (size_t)n));
   B200_TRY(total.alloc(ctx, 1));
-  B200_TRY(dev_normals(ctx, ch.c, ch.c->raw.p, n, true, 0, radius, nullptr, nrm.p));
+  B200_TRY(dev_normals(ctx, cloud.get(), cloud->raw.p, n, true, 0, radius, nullptr, nrm.p));
   hv_normal_flags_kernel<<<ceil_div(n, 256), 256, 0, ctx->stream>>>(reinterpret_cast<const float4 *>(nrm.p), n, flags.p);
   B200_LAUNCHED(ctx);
   B200_TRY(exclusive_scan_i32(ctx, flags.p, slots.p, n, total.p));
@@ -942,11 +937,11 @@ int b200_hv_verify(b200_ctx *ctx, b200_hv *hv, unsigned char *mask, b200_hv_info
     int ns = 0;
     B200_TRY(normals_and_compact(ctx, hv->scene_ds.p, hv->n0, (double)P.radius_normals, S, SN, &ns));
     hv->ns = ns;
-    CloudHolder scene_cloud;
+    std::unique_ptr<b200_cloud> scene_cloud;
     const GridView *sg = nullptr;
     if (ns > 0) {
-      B200_TRY(cloud_upload(ctx, reinterpret_cast<const float *>(S.p), ns, 4, true, &scene_cloud.c));
-      B200_TRY(cloud_grid_for_radius(scene_cloud.c, (double)P.inlier_threshold, &sg));
+      B200_TRY(cloud_upload(ctx, reinterpret_cast<const float *>(S.p), ns, 4, true, scene_cloud));
+      B200_TRY(cloud_grid_for_radius(scene_cloud.get(), (double)P.inlier_threshold, &sg));
     }
     // ---- addModel per hypothesis
     std::vector<int> indices, bad_information;
