@@ -44,6 +44,7 @@ EXPORTS = [
     "b200_board_lrf",
     "b200_model_create_shot_hough", "b200_model_download_frames", "b200_register_scene_shot_hough",
     "b200_dev_register_scene_shot_hough", "b200_register_scene_batch_shot_hough",
+    "b200_model_create_fpfh_hough", "b200_register_scene_fpfh_hough",
     "b200_hv_params_default", "b200_hv_create", "b200_hv_destroy", "b200_hv_set_params", "b200_hv_set_scene",
     "b200_hv_add_models", "b200_hv_verify", "b200_hv_last_size", "b200_hv_last_copy", "b200_hv_optimize",
 ]
@@ -205,6 +206,11 @@ def lib():
                                                      C.POINTER(ShotParams), C.POINTER(HoughParams), i, C.POINTER(fp),
                                                      C.POINTER(ip), C.POINTER(C.POINTER(Corr)), ip, ip,
                                                      C.POINTER(C.POINTER(Corr)), ip, ip],
+            "b200_model_create_fpfh_hough": [vp, fp, i, i, fp, i, i, C.POINTER(ShotParams), i, d, C.POINTER(HoughParams),
+                                             C.POINTER(vp)],
+            "b200_register_scene_fpfh_hough": [vp, vp, fp, i, i, fp, i, i, C.POINTER(ShotParams), i, d,
+                                               C.POINTER(HoughParams), fp, ip, C.POINTER(Corr), i, ip, C.POINTER(Corr),
+                                               ip, fp, fp],
             "b200_remove_nan": [vp, fp, i, i, fp, ip, ip],
             "b200_transform_points": [vp, fp, i, i, fp, fp],
             "b200_icp_align": [vp, fp, i, i, vp, i, d, d, d, fp, fp, fp, C.POINTER(d), ip, ip],
@@ -937,6 +943,38 @@ class Context:
                                             _f(desc) if want_desc else None)
         out = self._scene_result(rc, T, off, ic, corrs, mi, n_inst.value, n_corr.value)
         out["truncated"] = rc == ERR_CAPACITY
+        if want_desc:
+            out["desc"] = desc[:Ks]
+        return out
+
+    def model_create_fpfh_hough(self, xyz, kp, params, hough, surface_normal_k=50, surface_normal_radius=0.0):
+        """b200_model_create_fpfh_hough: the FPFH model of the keypoints plus their BOARD frames over the dense cloud
+        `xyz` (normals estimated there with surface_normal_k or surface_normal_radius; frames drawn from this
+        context's rand() stream) and the Hough votes."""
+        xyz, kp = _pts(xyz), _pts(kp)
+        h = C.c_void_p()
+        self._chk(lib().b200_model_create_fpfh_hough(self.h, _f(xyz), len(xyz), xyz.shape[1], _f(kp), len(kp),
+                                                     kp.shape[1], C.byref(params), int(surface_normal_k),
+                                                     float(surface_normal_radius), C.byref(hough), C.byref(h)))
+        return Model(self, h)
+
+    def register_scene_fpfh_hough(self, model, scene_xyz, scene_kp, params, hough, surface_normal_k=50,
+                                  surface_normal_radius=0.0, want_desc=False):
+        """Host buffers in, host results out (b200_register_scene_fpfh_hough).  As register_scene_fpfh, plus the scene
+        frames ("rf", Ks x 9) and the return code ("status": 0, or ERR_CAPACITY when the instances were truncated or
+        the Hough space would exceed 2^27 bins)."""
+        scene_xyz, scene_kp = _pts(scene_xyz), _pts(scene_kp)
+        mi, Ks = params.max_instances, len(scene_kp)
+        T, off, ic, corrs = _scene_outputs(mi, Ks, zero_offsets=True)
+        rf = np.empty((max(Ks, 1), 9), dtype=np.float32)
+        desc = np.empty((max(Ks, 1), 33), dtype=np.float32) if want_desc else None
+        n_inst, n_corr = C.c_int(), C.c_int()
+        rc = lib().b200_register_scene_fpfh_hough(self.h, model.h, _f(scene_xyz), len(scene_xyz), scene_xyz.shape[1],
+                                                  _f(scene_kp), Ks, scene_kp.shape[1], C.byref(params),
+                                                  int(surface_normal_k), float(surface_normal_radius), C.byref(hough),
+                                                  _f(T), _i(off), _c(ic), max(Ks, 1), C.byref(n_inst), _c(corrs),
+                                                  C.byref(n_corr), _f(desc) if want_desc else None, _f(rf))
+        out = dict(self._scene_result(rc, T, off, ic, corrs, mi, n_inst.value, n_corr.value), rf=rf[:Ks], status=rc)
         if want_desc:
             out["desc"] = desc[:Ks]
         return out

@@ -2,6 +2,7 @@
 // and the resident SHOT registration pipeline.  No torch types, no exceptions across the boundary.
 #include <algorithm>
 #include <functional>
+#include <initializer_list>
 #include <mutex>
 #include <thread>
 #include <array>
@@ -138,15 +139,38 @@ int check_hough_params(b200_ctx *ctx, const b200_hough_params *h) {
   return B200_OK;
 }
 
-// the checks both scene registrations (host and device buffers) make of the parameters and of a non-null model
+// the checks the SHOT scene registrations (host and device buffers, lanes) make of the parameters and of a non-null
+// model; a model of another descriptor length (FPFH: 33) would have dev_match read K x 352 floats from K x 33
 int check_registration(b200_ctx *ctx, const b200_model *model, const b200_shot_params *p, const b200_hough_params *h) {
   B200_TRY(check_params(ctx, p));
+  if (model->D != 352)
+    return ctx->fail(B200_ERR_INVALID, "register_scene_shot: the model is not a SHOT352 model (b200_model_create_shot)");
   if (!h) return B200_OK;
   B200_TRY(check_hough_params(ctx, h));
   if (!model->has_frames)
     return ctx->fail(B200_ERR_INVALID, "register_scene_hough: the model has no frames (b200_model_create_shot_hough)");
   return B200_OK;
 }
+
+// The dense cloud a BOARD frame estimation searches (setSearchSurface) and the normal estimation run on it
+// (setKSearch / setRadiusSearch): the FPFH Hough branch's surface, which is not the keypoint cloud its descriptors use.
+struct DenseSurface {
+  const float *xyz;
+  int n, stride;
+  int normal_k;
+  double normal_radius;
+  int check(b200_ctx *ctx) const {
+    if ((normal_k != 0) == (normal_radius != 0.0) || normal_k < 0 || normal_radius < 0.0)
+      return ctx->fail(B200_ERR_INVALID, "exactly one of surface_normal_k / surface_normal_radius must be positive");
+    return B200_OK;
+  }
+  // the cloud on the device and its normals (cloud->n x 4)
+  int upload(b200_ctx *ctx, std::unique_ptr<b200_cloud> &cloud, DevBuf<float> &normals) const {
+    B200_TRY(cloud_upload(ctx, xyz, n, stride, false, cloud));
+    B200_TRY(normals.alloc(ctx, (size_t)std::max(cloud->n, 1) * 4));
+    return dev_normals(ctx, cloud.get(), cloud->raw.p, cloud->n, true, normal_k, normal_radius, nullptr, normals.p);
+  }
+};
 
 // Device result of a scene registration: the correspondence list (cap entries) and, per view, its correspondence
 // count and one grouping result for max_inst instances and cap instance correspondences (out(v)).
@@ -187,6 +211,25 @@ int scene_descriptors(b200_ctx *ctx, b200_cloud *scene, const b200_shot_params *
   return dev_shot(ctx, scene, d_normals, d_kp, K, p->descr_radius, d_desc, nullptr, false);
 }
 
+// The Hough branch after the correspondence search (SHOT and FPFH pipelines): BOARD frames of the scene keypoints
+// over `surface` and its normals, drawn from the model's recorded rand() state, then Hough3DGrouping with the model's
+// votes.  d_rf_out nullable; d_status: see dev_hough3d.
+int hough_branch(b200_ctx *ctx, const b200_model *model, b200_cloud *surface, const float *d_normals,
+                 const float4 *d_kp, int Ks, const b200_hough_params *h, const b200_corr *d_corrs, const int *d_n_corrs,
+                 const InstanceOut &out, float *d_rf_out, int *d_status) {
+  DevBuf<float> rf_tmp;
+  float *d_rf = d_rf_out;
+  if (!d_rf) {
+    B200_TRY(rf_tmp.alloc(ctx, (size_t)std::max(Ks, 1) * 9));
+    d_rf = rf_tmp.p;
+  }
+  uint32_t stream_state[31];  // every scene starts from the model's recorded rand() state
+  memcpy(stream_state, model->rand_state, sizeof(stream_state));
+  B200_TRY(dev_board_lrf_from(ctx, surface, d_normals, d_kp, Ks, h->rf_radius, &h->board, stream_state, d_rf));
+  return dev_hough3d(ctx, model->kp.p, model->votes.p, d_kp, d_rf, d_corrs, d_n_corrs, Ks, h->bin_size, h->threshold,
+                     out, d_status);
+}
+
 // scene side of the pipeline on resident buffers: normals -> SHOT352 -> correspondence search, then
 // geometric-consistency grouping (h == nullptr) or the Hough branch (BOARD frames of the scene keypoints ->
 // Hough3DGrouping; d_rf_out nullable, d_status: see dev_hough3d)
@@ -208,17 +251,7 @@ int scene_pipeline(b200_ctx *ctx, const b200_model *model, b200_cloud *scene, co
   B200_TRY(dev_match(ctx, model->desc.p, model->K, d_desc, Ks, 352, p->match_mode, p->match_thr, d_corrs, d_n_corrs,
                      &model->tc));
   if (!h) return dev_gc(ctx, model->kp.p, d_kp, d_corrs, d_n_corrs, Ks, p->gc_size, p->gc_threshold, out);
-  DevBuf<float> rf_tmp;
-  float *d_rf = d_rf_out;
-  if (!d_rf) {
-    B200_TRY(rf_tmp.alloc(ctx, (size_t)std::max(Ks, 1) * 9));
-    d_rf = rf_tmp.p;
-  }
-  uint32_t stream_state[31];  // every scene starts from the model's recorded rand() state
-  memcpy(stream_state, model->rand_state, sizeof(stream_state));
-  B200_TRY(dev_board_lrf_from(ctx, scene, normals.p, d_kp, Ks, h->rf_radius, &h->board, stream_state, d_rf));
-  return dev_hough3d(ctx, model->kp.p, model->votes.p, d_kp, d_rf, d_corrs, d_n_corrs, Ks, h->bin_size, h->threshold,
-                     out, d_status);
+  return hough_branch(ctx, model, scene, normals.p, d_kp, Ks, h, d_corrs, d_n_corrs, out, d_rf_out, d_status);
 }
 
 __global__ void unpack_points_kernel(const float4 *__restrict__ in, int n, float *__restrict__ out) {
@@ -267,19 +300,26 @@ int download_instances(b200_ctx *ctx, const InstanceOut &o, float *transforms, i
   return B200_OK;
 }
 
+// An optional per-keypoint output of a scene registration (frames, descriptors): n floats, skipped when host is null.
+struct ExtraOut {
+  float *host;
+  const float *dev;
+  size_t n;
+};
+
 // Host side of a scene registration: the correspondence count (with d_status, the Hough status too) and one wait,
-// then the correspondence list, n_extra floats of an optional per-keypoint output (frames, descriptors), and the
-// instances.
-int download_result(b200_ctx *ctx, const ResultBufs &r, const int *d_status, float *extra, const float *d_extra,
-                    size_t n_extra, float *transforms, int *inst_offsets, b200_corr *inst_corrs, int corr_cap,
-                    int *n_inst, b200_corr *corrs_out, int *n_corrs) {
+// then the correspondence list, the per-keypoint outputs, and the instances.
+int download_result(b200_ctx *ctx, const ResultBufs &r, const int *d_status, std::initializer_list<ExtraOut> extras,
+                    float *transforms, int *inst_offsets, b200_corr *inst_corrs, int corr_cap, int *n_inst,
+                    b200_corr *corrs_out, int *n_corrs) {
   int nc = 0, status = B200_OK;
   B200_TRY(download(ctx, &nc, r.n_corrs.p, 1));
   if (d_status) B200_TRY(download(ctx, &status, d_status, 1));
   B200_CUDA(ctx, ctx->sync());
   if (n_corrs) *n_corrs = nc;
   if (corrs_out) B200_TRY(download(ctx, corrs_out, r.corrs.p, (size_t)nc));
-  if (extra) B200_TRY(download(ctx, extra, d_extra, n_extra));
+  for (const ExtraOut &x : extras)
+    if (x.host) B200_TRY(download(ctx, x.host, x.dev, x.n));
   if (status == B200_ERR_CAPACITY) {
     B200_CUDA(ctx, ctx->sync());  // the downloads above land before the call returns
     return ctx->fail(B200_ERR_CAPACITY, "hough3d: more than 2^27 bins (bin size too small)");
@@ -880,8 +920,21 @@ int b200_icp_align(b200_ctx *ctx, const float *source, int ns, int sstride, b200
 }  // extern "C"
 
 namespace {
-// normals + SHOT352 of the model keypoints; with h, also their BOARD frames (from ctx's rand() stream, whose state
-// after them the model records) and the Hough votes
+// The Hough side of a model (SHOT and FPFH): the BOARD frames of its keypoints over `surface` and its normals, drawn
+// from ctx's rand() stream (a context never seeded is srand(1)), the stream's state after them, and
+// Hough3DGrouping::train()'s votes.
+int model_frames(b200_ctx *ctx, b200_model *m, b200_cloud *surface, const float *d_normals, const b200_hough_params *h) {
+  if (!ctx->rand_seeded) board_rand_seed(ctx, 1u);
+  B200_TRY(m->rf.alloc(ctx, (size_t)std::max(m->K, 1) * 9));
+  B200_TRY(m->votes.alloc(ctx, (size_t)std::max(m->K, 1) * 3));
+  B200_TRY(dev_board_lrf(ctx, surface, d_normals, m->kp.p, m->K, h->rf_radius, &h->board, m->rf.p));
+  B200_TRY(dev_hough_model_votes(ctx, m->kp.p, m->rf.p, m->K, m->votes.p));
+  memcpy(m->rand_state, ctx->rand_state, sizeof(m->rand_state));
+  m->has_frames = true;
+  return B200_OK;
+}
+
+// normals + SHOT352 of the model keypoints; with h, also their BOARD frames and the Hough votes (model_frames)
 int model_create(b200_ctx *ctx, const float *xyz, int n, int stride, const float *kp, int K, int kstride,
                  const b200_shot_params *p, const b200_hough_params *h, b200_model **out) {
   if (!out) return ctx->fail(B200_ERR_INVALID, "model_create: null output");
@@ -900,15 +953,7 @@ int model_create(b200_ctx *ctx, const float *xyz, int n, int stride, const float
   B200_TRY(m->desc.alloc(ctx, (size_t)std::max(K, 1) * 352));
   B200_TRY(dev_shot(ctx, cloud.get(), normals.p, m->kp.p, K, p->descr_radius, m->desc.p, nullptr, false));
   B200_TRY(match_prepare_model(ctx, m.get()));
-  if (h) {
-    if (!ctx->rand_seeded) board_rand_seed(ctx, 1u);
-    B200_TRY(m->rf.alloc(ctx, (size_t)std::max(K, 1) * 9));
-    B200_TRY(m->votes.alloc(ctx, (size_t)std::max(K, 1) * 3));
-    B200_TRY(dev_board_lrf(ctx, cloud.get(), normals.p, m->kp.p, K, h->rf_radius, &h->board, m->rf.p));
-    B200_TRY(dev_hough_model_votes(ctx, m->kp.p, m->rf.p, K, m->votes.p));
-    memcpy(m->rand_state, ctx->rand_state, sizeof(m->rand_state));
-    m->has_frames = true;
-  }
+  if (h) B200_TRY(model_frames(ctx, m.get(), cloud.get(), normals.p, h));
   B200_CUDA(ctx, ctx->sync());
   *out = m.release();
   return B200_OK;
@@ -1012,8 +1057,8 @@ int register_scene(b200_ctx *ctx, const b200_model *model, const float *scene_xy
   B200_TRY(scene_pipeline(ctx, model, scene.get(), dkp.p, Ks, p, r.out(), r.corrs.p, r.n_corrs.p, nullptr, h, drf.p,
                           dstatus.p));
   tr.tick("e2e pipeline issue");
-  B200_TRY(download_result(ctx, r, dstatus.p, rf_out, drf.p, (size_t)Ks * 9, transforms, inst_offsets,
-                           inst_corrs, corr_cap, n_inst, corrs_out, n_corrs));
+  B200_TRY(download_result(ctx, r, dstatus.p, {{rf_out, drf.p, (size_t)Ks * 9}}, transforms, inst_offsets, inst_corrs,
+                           corr_cap, n_inst, corrs_out, n_corrs));
   tr.tick("e2e download");
   return B200_OK;
 }
@@ -1075,13 +1120,17 @@ int fpfh_side(b200_ctx *ctx, b200_cloud *cloud, const b200_shot_params *p, DevBu
   B200_TRY(dev_normals(ctx, cloud, cloud->raw.p, cloud->n, true, p->normal_k, p->normal_radius, nullptr, normals.p));
   return dev_fpfh(ctx, cloud, normals.p, cloud->raw.p, cloud->n, true, p->descr_radius, desc.p);
 }
-}  // namespace
 
-int b200_model_create_fpfh(b200_ctx *ctx, const float *kp, int K, int kstride, const b200_shot_params *p,
-                           b200_model **out) {
-  API_ENTER(ctx);
+// b200_model_create_fpfh (h == nullptr) / b200_model_create_fpfh_hough: with h, also the BOARD frames of the
+// keypoints over the dense cloud `surface` and the Hough votes (model_frames)
+int model_create_fpfh(b200_ctx *ctx, const float *kp, int K, int kstride, const b200_shot_params *p,
+                      const DenseSurface *surface, const b200_hough_params *h, b200_model **out) {
   if (!out) return ctx->fail(B200_ERR_INVALID, "model_create_fpfh: null output");
   B200_TRY(check_params(ctx, p));
+  if (h) {
+    B200_TRY(check_hough_params(ctx, h));
+    B200_TRY(surface->check(ctx));
+  }
   std::unique_ptr<b200_cloud> cloud;
   B200_TRY(cloud_upload(ctx, kp, K, kstride, false, cloud));
   std::unique_ptr<b200_model> m(new (std::nothrow) b200_model());
@@ -1095,20 +1144,32 @@ int b200_model_create_fpfh(b200_ctx *ctx, const float *kp, int K, int kstride, c
     B200_CUDA(ctx, cudaMemcpyAsync(m->kp.p, cloud->raw.p, (size_t)K * sizeof(float4), cudaMemcpyDeviceToDevice,
                                    ctx->stream));
   B200_TRY(match_prepare_model(ctx, m.get()));
+  if (h) {
+    std::unique_ptr<b200_cloud> dense;
+    DevBuf<float> normals;
+    B200_TRY(surface->upload(ctx, dense, normals));
+    B200_TRY(model_frames(ctx, m.get(), dense.get(), normals.p, h));
+  }
   B200_CUDA(ctx, ctx->sync());
   *out = m.release();
   return B200_OK;
 }
 
-int b200_model_descriptor_length(const b200_model *m) { return m ? m->D : 0; }
-
-int b200_register_scene_fpfh(b200_ctx *ctx, const b200_model *model, const float *scene_kp, int Ks, int kstride,
-                             const b200_shot_params *p, float *transforms, int *inst_offsets, b200_corr *inst_corrs,
-                             int corr_cap, int *n_inst, b200_corr *corrs_out, int *n_corrs, float *desc_out) {
-  API_ENTER(ctx);
+// b200_register_scene_fpfh (h == nullptr: GC grouping) / b200_register_scene_fpfh_hough (the Hough branch over the
+// dense scene cloud `surface`; rf_out nullable)
+int register_scene_fpfh(b200_ctx *ctx, const b200_model *model, const float *scene_kp, int Ks, int kstride,
+                        const b200_shot_params *p, const DenseSurface *surface, const b200_hough_params *h,
+                        float *transforms, int *inst_offsets, b200_corr *inst_corrs, int corr_cap, int *n_inst,
+                        b200_corr *corrs_out, int *n_corrs, float *desc_out, float *rf_out) {
   if (!model || model->D != 33 || !n_inst || Ks < 0)
     return ctx->fail(B200_ERR_INVALID, "register_scene_fpfh: bad arguments (the model must come from b200_model_create_fpfh)");
   B200_TRY(check_params(ctx, p));
+  if (h) {
+    B200_TRY(check_hough_params(ctx, h));
+    if (!model->has_frames)
+      return ctx->fail(B200_ERR_INVALID, "register_scene_fpfh_hough: the model has no frames (b200_model_create_fpfh_hough)");
+    B200_TRY(surface->check(ctx));
+  }
   *n_inst = 0;
   if (n_corrs) *n_corrs = 0;
   std::unique_ptr<b200_cloud> scene;
@@ -1119,9 +1180,58 @@ int b200_register_scene_fpfh(b200_ctx *ctx, const b200_model *model, const float
   B200_TRY(r.alloc(ctx, std::max(Ks, 1), p->max_instances));
   B200_TRY(dev_match(ctx, model->desc.p, model->K, desc.p, Ks, 33, p->match_mode, p->match_thr, r.corrs.p, r.n_corrs.p,
                      &model->tc));
-  B200_TRY(dev_gc(ctx, model->kp.p, scene->raw.p, r.corrs.p, r.n_corrs.p, Ks, p->gc_size, p->gc_threshold, r.out()));
-  return download_result(ctx, r, nullptr, desc_out, desc.p, (size_t)Ks * 33, transforms, inst_offsets, inst_corrs,
-                         corr_cap, n_inst, corrs_out, n_corrs);
+  std::unique_ptr<b200_cloud> dense;
+  DevBuf<float> normals, rf;
+  DevBuf<int> status;
+  if (!h) {
+    B200_TRY(dev_gc(ctx, model->kp.p, scene->raw.p, r.corrs.p, r.n_corrs.p, Ks, p->gc_size, p->gc_threshold, r.out()));
+  } else {
+    B200_TRY(surface->upload(ctx, dense, normals));
+    B200_TRY(rf.alloc(ctx, (size_t)std::max(Ks, 1) * 9));
+    B200_TRY(status.alloc(ctx, 1));
+    B200_TRY(hough_branch(ctx, model, dense.get(), normals.p, scene->raw.p, Ks, h, r.corrs.p, r.n_corrs.p, r.out(),
+                          rf.p, status.p));
+  }
+  return download_result(ctx, r, status.p, {{desc_out, desc.p, (size_t)Ks * 33}, {rf_out, rf.p, (size_t)Ks * 9}},
+                         transforms, inst_offsets, inst_corrs, corr_cap, n_inst, corrs_out, n_corrs);
+}
+}  // namespace
+
+int b200_model_create_fpfh(b200_ctx *ctx, const float *kp, int K, int kstride, const b200_shot_params *p,
+                           b200_model **out) {
+  API_ENTER(ctx);
+  return model_create_fpfh(ctx, kp, K, kstride, p, nullptr, nullptr, out);
+}
+
+int b200_model_create_fpfh_hough(b200_ctx *ctx, const float *xyz, int n, int stride, const float *kp, int K,
+                                 int kstride, const b200_shot_params *p, int surface_normal_k,
+                                 double surface_normal_radius, const b200_hough_params *h, b200_model **out) {
+  API_ENTER(ctx);
+  if (!h) return ctx->fail(B200_ERR_INVALID, "null Hough params");
+  const DenseSurface surface = {xyz, n, stride, surface_normal_k, surface_normal_radius};
+  return model_create_fpfh(ctx, kp, K, kstride, p, &surface, h, out);
+}
+
+int b200_model_descriptor_length(const b200_model *m) { return m ? m->D : 0; }
+
+int b200_register_scene_fpfh(b200_ctx *ctx, const b200_model *model, const float *scene_kp, int Ks, int kstride,
+                             const b200_shot_params *p, float *transforms, int *inst_offsets, b200_corr *inst_corrs,
+                             int corr_cap, int *n_inst, b200_corr *corrs_out, int *n_corrs, float *desc_out) {
+  API_ENTER(ctx);
+  return register_scene_fpfh(ctx, model, scene_kp, Ks, kstride, p, nullptr, nullptr, transforms, inst_offsets,
+                             inst_corrs, corr_cap, n_inst, corrs_out, n_corrs, desc_out, nullptr);
+}
+
+int b200_register_scene_fpfh_hough(b200_ctx *ctx, const b200_model *model, const float *scene_xyz, int n, int stride,
+                                   const float *scene_kp, int Ks, int kstride, const b200_shot_params *p,
+                                   int surface_normal_k, double surface_normal_radius, const b200_hough_params *h,
+                                   float *transforms, int *inst_offsets, b200_corr *inst_corrs, int corr_cap,
+                                   int *n_inst, b200_corr *corrs_out, int *n_corrs, float *desc_out, float *rf_out) {
+  API_ENTER(ctx);
+  if (!h) return ctx->fail(B200_ERR_INVALID, "null Hough params");
+  const DenseSurface surface = {scene_xyz, n, stride, surface_normal_k, surface_normal_radius};
+  return register_scene_fpfh(ctx, model, scene_kp, Ks, kstride, p, &surface, h, transforms, inst_offsets, inst_corrs,
+                             corr_cap, n_inst, corrs_out, n_corrs, desc_out, rf_out);
 }
 
 /* ------------------------------------------------------------------ multi-GPU (comm.cu) */
@@ -1169,6 +1279,8 @@ int b200_register_scene_shot_sharded(b200_ctx *ctx, const b200_model *model, int
   API_ENTER(ctx);
   const int G = ctx->comm_world, r = ctx->comm_rank;
   if (!model || root < 0 || root >= G) return ctx->fail(B200_ERR_INVALID, "register_scene_sharded: bad arguments");
+  if (model->D != 352)
+    return ctx->fail(B200_ERR_INVALID, "register_scene_sharded: the model is not a SHOT352 model (b200_model_create_shot)");
   B200_TRY(check_params(ctx, p));
   const bool is_root = r == root;
   if (is_root && (!n_inst || Ks < 0 || n < 0)) return ctx->fail(B200_ERR_INVALID, "register_scene_sharded: bad arguments");
@@ -1219,8 +1331,8 @@ int b200_register_scene_shot_sharded(b200_ctx *ctx, const b200_model *model, int
   B200_TRY(res.alloc(ctx, std::max(Ks, 1), p->max_instances));
   B200_TRY(dev_concat_lists(ctx, dall.p, dcounts.p, G, cap, res.corrs.p, res.cap, res.n_corrs.p));
   B200_TRY(dev_gc(ctx, model->kp.p, dkp.p, res.corrs.p, res.n_corrs.p, Ks, p->gc_size, p->gc_threshold, res.out()));
-  return download_result(ctx, res, nullptr, nullptr, nullptr, 0, transforms, inst_offsets, inst_corrs, corr_cap, n_inst,
-                         corrs_out, n_corrs);
+  return download_result(ctx, res, nullptr, {}, transforms, inst_offsets, inst_corrs, corr_cap, n_inst, corrs_out,
+                         n_corrs);
 }
 
 /* ------------------------------------------------------------------ lanes */

@@ -1,11 +1,17 @@
 // fpfh_recognition.cpp — the FPFH variant of the reference's recognition callback
-// (FPFH_demo.cpp:405-538) through the PCL-style adapters: normals on the keypoint clouds by radius
+// (FPFH_demo.cpp:405-585) through the PCL-style adapters: normals on the keypoint clouds by radius
 // (FPFH_demo.cpp:416-420, 486-492), FPFHEstimation with input = surface = keypoints
 // (FPFH_demo.cpp:422-428, 505-510), KdTreeFLANN<FPFHSignature33> k = 2 with the ratio test
-// (FPFH_demo.cpp:516-538), then GeometricConsistencyGrouping (the north-star grouping; the reference's
-// default there is Hough3D, which is a "next" row of SURVEY.md §8(f)).
+// (FPFH_demo.cpp:516-538), then grouping.  By default GeometricConsistencyGrouping (the north-star grouping, which
+// FPFH_demo itself does not have); with --hough the reference's own grouping block (FPFH_demo.cpp:548-585):
+// NormalEstimationOMP with k = 50 on the two dense clouds (FPFH_demo.cpp:405-409), BOARD frames of the keypoints over
+// the dense clouds and their normals (FPFH_demo.cpp:556-568: find_holes, rf_rad_ 0.02; the model's frames, then the
+// scene's, from one rand() stream), Hough3DGrouping with bin cg_size and threshold cg_thresh (0.02 / 2).
 //
-// usage: fpfh_recognition <model_kp.f32> <scene_kp.f32> <out_prefix> [radius=0.05] [cg_size=0.02] [cg_thresh=2]
+// usage: fpfh_recognition [--hough <model.f32> <scene.f32>] <model_kp.f32> <scene_kp.f32> <out_prefix> [radius=0.05]
+//                         [cg_size=0.02] [cg_thresh=2]
+// writes <out_prefix>.desc (scene FPFH33), .normals (scene keypoint normals), .corr (b200_corr records), .T (instances
+//        x 16 float); with --hough also .rf (model then scene BOARD frames, 9 float each)
 #include <pcl_b200/pcl_b200.h>
 
 #include <cmath>
@@ -33,13 +39,21 @@ static bool load_cloud(const char *path, pcl::PointCloud<PointType> &cloud) {
 }
 
 int main(int argc, char **argv) {
+  const bool use_hough = argc > 3 && std::string(argv[1]) == "--hough";
+  const char *model_path = use_hough ? argv[2] : nullptr, *scene_path = use_hough ? argv[3] : nullptr;
+  if (use_hough) {  // the dense clouds come first; the remaining arguments are those of the GC invocation
+    argc -= 3;
+    argv += 3;
+  }
   if (argc < 4) {
-    std::cerr << "usage: " << argv[0] << " model_kp.f32 scene_kp.f32 out_prefix [radius cg_size cg_thresh]" << std::endl;
+    std::cerr << "usage: fpfh_recognition [--hough model.f32 scene.f32] model_kp.f32 scene_kp.f32 out_prefix "
+              << "[radius cg_size cg_thresh]" << std::endl;
     return 2;
   }
   const double radius = argc > 4 ? atof(argv[4]) : 0.05;
   const float cg_size_ = argc > 5 ? (float)atof(argv[5]) : 0.02f;
   const float cg_thresh_ = argc > 6 ? (float)atof(argv[6]) : 2.0f;
+  const float rf_rad_ = 0.02f;
   pcl::PointCloud<PointType>::Ptr model_keypoints(new pcl::PointCloud<PointType>()),
       scene_keypoints(new pcl::PointCloud<PointType>());
   pcl::PointCloud<NormalType>::Ptr model_normals(new pcl::PointCloud<NormalType>()),
@@ -47,6 +61,19 @@ int main(int argc, char **argv) {
   pcl::PointCloud<DescriptorType>::Ptr model_descriptors(new pcl::PointCloud<DescriptorType>()),
       scene_descriptors(new pcl::PointCloud<DescriptorType>());
   if (!load_cloud(argv[1], *model_keypoints) || !load_cloud(argv[2], *scene_keypoints)) return 1;
+  pcl::PointCloud<PointType>::Ptr model(new pcl::PointCloud<PointType>()), scene(new pcl::PointCloud<PointType>());
+  pcl::PointCloud<NormalType>::Ptr model_cloud_normals(new pcl::PointCloud<NormalType>()),
+      scene_cloud_normals(new pcl::PointCloud<NormalType>());
+  if (use_hough) {
+    if (!load_cloud(model_path, *model) || !load_cloud(scene_path, *scene)) return 1;
+    // FPFH_demo.cpp:405-409: normals of the dense clouds, k = 50
+    pcl::NormalEstimationOMP<PointType, NormalType> cloud_norm_est;
+    cloud_norm_est.setKSearch(50);
+    cloud_norm_est.setInputCloud(scene);
+    cloud_norm_est.compute(*scene_cloud_normals);
+    cloud_norm_est.setInputCloud(model);
+    cloud_norm_est.compute(*model_cloud_normals);
+  }
 
   pcl::search::KdTree<PointType>::Ptr kdtree(new pcl::search::KdTree<PointType>());
   pcl::NormalEstimationOMP<PointType, NormalType> norm_est;
@@ -83,16 +110,56 @@ int main(int argc, char **argv) {
 
   std::vector<pcl::Matrix4f> rototranslations;
   std::vector<pcl::Correspondences> clustered_corrs;
-  pcl::GeometricConsistencyGrouping<PointType, PointType> gc_clusterer;
-  gc_clusterer.setGCSize(cg_size_);
-  gc_clusterer.setGCThreshold(cg_thresh_);
-  gc_clusterer.setInputCloud(model_keypoints);
-  gc_clusterer.setSceneCloud(scene_keypoints);
-  gc_clusterer.setModelSceneCorrespondences(model_scene_corrs);
-  gc_clusterer.recognize(rototranslations, clustered_corrs);
+  const std::string prefix = argv[3];
+  if (use_hough) {
+    // FPFH_demo.cpp:548-585
+    pcl::PointCloud<pcl::ReferenceFrame>::Ptr model_rf(new pcl::PointCloud<pcl::ReferenceFrame>()),
+        scene_rf(new pcl::PointCloud<pcl::ReferenceFrame>());
+    pcl::BOARDLocalReferenceFrameEstimation<PointType, NormalType, pcl::ReferenceFrame> rf_est;
+    rf_est.setFindHoles(true);
+    rf_est.setRadiusSearch(rf_rad_);
+
+    rf_est.setInputCloud(model_keypoints);
+    rf_est.setInputNormals(model_cloud_normals);
+    rf_est.setSearchSurface(model);
+    rf_est.compute(*model_rf);
+
+    rf_est.setInputCloud(scene_keypoints);
+    rf_est.setInputNormals(scene_cloud_normals);
+    rf_est.setSearchSurface(scene);
+    rf_est.compute(*scene_rf);
+
+    pcl::Hough3DGrouping<PointType, PointType, pcl::ReferenceFrame, pcl::ReferenceFrame> clusterer;
+    clusterer.setHoughBinSize(cg_size_);
+    clusterer.setHoughThreshold(cg_thresh_);
+    clusterer.setUseInterpolation(false);
+    clusterer.setUseDistanceWeight(true);
+    clusterer.setInputCloud(model_keypoints);
+    clusterer.setInputRf(model_rf);
+    clusterer.setSceneCloud(scene_keypoints);
+    clusterer.setSceneRf(scene_rf);
+    clusterer.setModelSceneCorrespondences(model_scene_corrs);
+    clusterer.recognize(rototranslations, clustered_corrs);
+
+    FILE *frf = fopen((prefix + ".rf").c_str(), "wb");
+    for (int side = 0; side < 2; ++side)
+      for (const pcl::ReferenceFrame &r : (side ? *scene_rf : *model_rf).points) {
+        fwrite(r.x_axis, sizeof(float), 3, frf);
+        fwrite(r.y_axis, sizeof(float), 3, frf);
+        fwrite(r.z_axis, sizeof(float), 3, frf);
+      }
+    fclose(frf);
+  } else {
+    pcl::GeometricConsistencyGrouping<PointType, PointType> gc_clusterer;
+    gc_clusterer.setGCSize(cg_size_);
+    gc_clusterer.setGCThreshold(cg_thresh_);
+    gc_clusterer.setInputCloud(model_keypoints);
+    gc_clusterer.setSceneCloud(scene_keypoints);
+    gc_clusterer.setModelSceneCorrespondences(model_scene_corrs);
+    gc_clusterer.recognize(rototranslations, clustered_corrs);
+  }
   std::cout << "Model instances found: " << rototranslations.size() << std::endl;
 
-  const std::string prefix = argv[3];
   FILE *f = fopen((prefix + ".desc").c_str(), "wb");
   for (size_t i = 0; i < scene_descriptors->size(); ++i) fwrite(scene_descriptors->at(i).histogram, sizeof(float), 33, f);
   fclose(f);

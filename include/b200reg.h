@@ -282,7 +282,9 @@ B200_API int b200_register_scene_fpfh(b200_ctx *ctx, const b200_model *model, co
 
 /* Scene side of SHOT.cpp:305-483 in one call (host buffers in, host results out): normals →
  * SHOT352 at the keypoints → correspondence search against the resident model → GC grouping.
- * corrs_out (capacity Ks) / n_corrs receive the model-scene correspondences; may be NULL. */
+ * corrs_out (capacity Ks) / n_corrs receive the model-scene correspondences; may be NULL.  This call, its device,
+ * Hough, batch and sharded forms return B200_ERR_INVALID, before any work, for a model whose descriptors are not
+ * SHOT352 (an FPFH model). */
 B200_API int b200_register_scene_shot(b200_ctx *ctx, const b200_model *model, const float *scene_xyz, int n, int stride,
                              const float *scene_kp, int Ks, int kstride, const b200_shot_params *p,
                              float *transforms, int *inst_offsets, b200_corr *inst_corrs, int corr_cap,
@@ -373,6 +375,38 @@ B200_API int b200_register_scene_batch_shot_hough(int device, const b200_model *
                                                   float *const *transforms, int *const *inst_offsets,
                                                   b200_corr *const *inst_corrs, const int *corr_cap, int *n_inst,
                                                   b200_corr *const *corrs_out, int *n_corrs, int *status);
+
+/* The FPFH pipeline's Hough branch, which is the only grouping FPFH_demo has (FPFH_demo.cpp:548-585, `if (use_hough_)`
+ * with no else).  The descriptor side is that of b200_model_create_fpfh / b200_register_scene_fpfh: p->normal_k /
+ * p->normal_radius are the normals estimated ON the keypoint cloud (FPFH_demo.cpp:416-420, 486-492), descr_radius is
+ * the FPFH radius with input = surface = keypoints (:422-428, :505-510), match_mode / match_thr the k = 2 ratio test
+ * (:516-538); p->gc_size / p->gc_threshold are not read.  The model's descriptors are those of
+ * b200_model_create_fpfh(kp), the scene's correspondences those of b200_register_scene_fpfh, byte for byte.
+ * BOARD frames (FPFH_demo.cpp:556-568: setInputCloud(keypoints), setInputNormals(cloud normals),
+ * setSearchSurface(cloud)): the search surface is the dense cloud xyz / scene_xyz, and its normals are estimated on
+ * it with surface_normal_k or surface_normal_radius (exactly one positive, the other 0, else B200_ERR_INVALID; the reference's
+ * scene uses k = 50, FPFH_demo.cpp:405-409); radius h->rf_radius, parameters h->board.  A caller who reads the
+ * reference as "surface = the keypoint cloud" passes the keypoints as xyz with the keypoint normal setting.
+ * The rand() stream is handled as in b200_model_create_shot_hough: the model's frames draw from ctx's stream, the
+ * model records the state after them, and every scene draws from that recorded state.  The model works with
+ * b200_model_download_frames and with b200_register_scene_fpfh (GC), which gives the same result as for a plain FPFH
+ * model. */
+B200_API int b200_model_create_fpfh_hough(b200_ctx *ctx, const float *xyz, int n, int stride, const float *kp, int K,
+                                          int kstride, const b200_shot_params *p, int surface_normal_k,
+                                          double surface_normal_radius, const b200_hough_params *h, b200_model **out);
+/* Scene side: normals + FPFH33 of the scene keypoint cloud -> correspondence search -> BOARD frames of the scene
+ * keypoints over scene_xyz and its normals -> Hough3DGrouping -> RANSAC poses.  Outputs as
+ * b200_register_scene_shot_hough; desc_out (Ks x 33) and rf_out (Ks x 9) may each be NULL.  B200_ERR_CAPACITY when the
+ * Hough space would exceed 2^27 bins (no instance; the correspondences are still returned) or there are more than
+ * p->max_instances instances (the first ones are kept).  B200_ERR_INVALID for a model that is not an FPFH model with
+ * frames (b200_model_create_fpfh_hough). */
+B200_API int b200_register_scene_fpfh_hough(b200_ctx *ctx, const b200_model *model, const float *scene_xyz, int n,
+                                            int stride, const float *scene_kp, int Ks, int kstride,
+                                            const b200_shot_params *p, int surface_normal_k,
+                                            double surface_normal_radius, const b200_hough_params *h,
+                                            float *transforms, int *inst_offsets, b200_corr *inst_corrs, int corr_cap,
+                                            int *n_inst, b200_corr *corrs_out, int *n_corrs, float *desc_out,
+                                            float *rf_out);
 
 /* ---------------------------------------------------------------- multi-view library ----- */
 /* The reference recognises against a set of rendered partial views of the CAD models: CAD_desc.cpp:231-370
